@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the recommendation scoring hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--rows R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--rows R] [--dump-outputs DIR]
 
 Workload (BASELINE.json `metric`): single-query cosine top-10 with a 133-row seen-movie exclusion over a
 10M x 1536 bf16 synthetic catalog.  One step = one query through the whole hot path.
@@ -20,6 +20,9 @@ Workload (BASELINE.json `metric`): single-query cosine top-10 with a 133-row see
            route, lib.py:43-55) and the int8-prefilter variant of the headline.  Secondary: never instead of the headline.
 `--impl reference` times the reference's own CPU path (oracle/, pandas + scikit-learn, float64, all host threads) on
 a bounded row sample of the same workload and scales to the full catalog.
+`--dump-outputs DIR` writes what the last timed step returned as float64 .npy files, so that two builds can be compared
+           output for output on the same seeded inputs: rows.npy / scores.npy of the device-resident step (`value`) and
+           e2e_rows.npy / e2e_scores.npy of the host-buffer request (`e2e`); row ids are exact in float64.
 """
 from __future__ import annotations
 
@@ -420,6 +423,7 @@ def run_b200(args):
 
     from robot_ebert_b200 import CatalogStore, RowFilter, synth
     from robot_ebert_b200 import _native as nat
+    from robot_ebert_b200.catalog import unpack_result
     from robot_ebert_b200.sharding import ShardedCatalog
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -484,10 +488,11 @@ def run_b200(args):
         t0.record()
         for i in range(steps):
             kev[i][0].record()
-            step()
+            packed = step()
             kev[i][1].record()
         t1.record()
         barrier()
+    outputs = dict(zip(("rows", "scores"), unpack_result(packed.cpu().numpy(), K)[:2]))
     elapsed_ms = t0.elapsed_time(t1)
     kernel_ms = sum(a.elapsed_time(b) for a, b in kev) / steps
     if world > 1:
@@ -497,7 +502,9 @@ def run_b200(args):
     value = steps / (elapsed_ms * 1e-3)
 
     # ---- e2e: host buffers in, host buffers out, through the public API
-    e2e_s = time_wall(lambda: api.recommend(query=q, exclude_rows=excl, k=K), steps, warmup, barrier, world, dist, dev)
+    def e2e_step():
+        outputs["e2e_rows"], outputs["e2e_scores"] = api.recommend(query=q, exclude_rows=excl, k=K)
+    e2e_s = time_wall(e2e_step, steps, warmup, barrier, world, dist, dev)
     e2e = 1.0 / e2e_s
     h2d, d2h = int(store.last_h2d_bytes), int(store.last_d2h_bytes)
 
@@ -749,6 +756,10 @@ def run_b200(args):
         if world == 1 and not args.no_cpu_baseline:
             qps, desc, _, cores = cpu_reference_leg(rows, 5, 1, args.cpu_sample_rows, budget_s=20.0)
             line["cpu_baseline"] = {"value": qps, "unit": "queries/s", "cores": cores, "cpu_model": cpu_model(), "kind": "port", "sample": desc}
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), np.asarray(a, dtype=np.float64))
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -767,7 +778,12 @@ def main():
     ap.add_argument("--no-prefilter", action="store_true", help="skip the int8-prefilter measurement")
     ap.add_argument("--no-batched", action="store_true", help="skip the batched (tcgen05) measurements")
     ap.add_argument("--no-configs", action="store_true", help="skip the single-GPU BASELINE configs C1-C3 and the production shape")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:
