@@ -719,6 +719,12 @@ class CatalogStore:
         whole 128-byte k-blocks (tcgen05 kind::i8, K = 32 per instruction, 128-byte swizzled tiles)."""
         return self._c8 is not None and self._c8.ld % 128 == 0
 
+    @property
+    def batch_gemm_ok(self) -> bool:
+        """True when the batched path can run on bf16 operands: a bf16 catalog whose rows are whole 64-element (128-byte)
+        k-blocks.  bf16 rows of d <= 32 are stored 16 or 32 elements wide, which the tcgen05 GEMM does not take."""
+        return self.dtype == "bf16" and self.ld % 64 == 0
+
     def quantize_queries(self, qn32: torch.Tensor):
         """Unit queries / profiles [b, ld] fp32 -> (q8 int8 [b, ld8], qscale fp32 [b], qeps fp64 [b]) for the int8 batched path."""
         lib = nat.load()
@@ -781,13 +787,14 @@ class CatalogStore:
             if prefilter and not self.batch_shadow_ok:
                 raise ValueError("prefilter=True needs enable_prefilter() and rows of whole 128-byte int8 k-blocks")
             use_shadow = self.batch_shadow_ok and prefilter is not False
-            try:
-                plan = self.gemm_plan(b, k, shadow=use_shadow)
-            except nat.NativeError as e:
-                if e.code != nat.ERR_UNSUPPORTED:
-                    raise
-                plan = None          # catalog too small for the sampled-threshold scheme: one fused GEMV per user instead
-            if plan is None or (self.dtype != "bf16" and not use_shadow):
+            plan = None
+            if use_shadow or self.batch_gemm_ok:
+                try:
+                    plan = self.gemm_plan(b, k, shadow=use_shadow)
+                except nat.NativeError as e:
+                    if e.code != nat.ERR_UNSUPPORTED:
+                        raise    # ERR_UNSUPPORTED: catalog too small for the sampled-threshold scheme, plan stays None
+            if plan is None:        # too small, or neither operand type fits the GEMM: one fused GEMV per user instead
                 return self._recommend_batch_loop(qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter)
             ep = ec = None
             if excl_ptr is not None:
@@ -823,7 +830,8 @@ class CatalogStore:
         return rows, scores, counts
 
     def _recommend_batch_loop(self, qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter=None):
-        """Small or fp32 catalogs: the batch is served by the single-query kernel, one launch per prepared query."""
+        """Small catalogs, and catalogs neither GEMM operand type takes: the batch is served by the single-query kernel, one
+        launch per prepared query."""
         lib = nat.load()
         b = qn32.shape[0]
         kc = lib.rebert_candidates_for_k(k)

@@ -516,6 +516,9 @@ class ShardedCatalog:
         dev = store.device
         b = qbf.shape[0]
         shadow = store.quantize_queries(qn32) if (qn32 is not None and store.batch_shadow_ok) else None
+        if shadow is None and not store.batch_gemm_ok:
+            raise nat.NativeError(nat.ERR_UNSUPPORTED, f"batch_context: the tcgen05 GEMM takes neither this {store.dtype} shard "
+                                                       f"(ld={store.ld}) nor an int8 shadow of it")
         plan = store.gemm_plan(b, k, shadow=shadow is not None)
         ep = ec = None
         if excl_ptr is not None:
@@ -589,7 +592,8 @@ class ShardedCatalog:
             except nat.NativeError as e:
                 if e.code != nat.ERR_UNSUPPORTED:
                     raise
-                ctx = None           # shard too small for the tensor-core scheme (same verdict on every rank: equal shard sizes)
+                ctx = None           # shard too small for the tensor-core scheme, or of a dtype / width it does not take (same
+                                     # verdict on every rank: equal shard sizes, one dtype and width)
             if ctx is None:
                 return self._recommend_batch_loop(queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter,
                                                   return_info)

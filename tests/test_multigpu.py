@@ -405,3 +405,38 @@ def test_sharded_diverged_request_order_is_refused():
         pytest.skip("needs >= 2 GPUs")
     for rank, refused, recovered in _spawn("_diverge_worker", world, 50_000, 128):
         assert refused and recovered, rank
+
+
+def _routing_batch_worker(rank, world, port, n, d, dtype, b, k, out_q):
+    dist = _init(rank, world, port)
+    from robot_ebert_b200 import synth
+    from robot_ebert_b200.sharding import ShardedCatalog
+    try:
+        sc = ShardedCatalog.synthetic(0, n, d, dtype, scale_rows=True, device=torch.device("cuda", rank))
+        lp, lc, ep, ec = _csr_users(n, b)
+        rq = sc.recommend_batch(queries=synth.catalog_rows_f32(11, 0, b, d), excl_ptr=ep, excl_col=ec, k=k)
+        rp = sc.recommend_batch(liked_ptr=lp, liked_col=lc, excl_ptr=ep, excl_col=ec, k=k)
+        out_q.put((rank, [x.tolist() for x in rq], [x.tolist() for x in rp]))
+        dist.barrier()
+    finally:
+        dist.destroy_process_group()
+
+
+@pytest.mark.parametrize("dtype,d", [("fp32", 64), ("bf16", 32)])
+def test_sharded_batch_on_shards_the_gemm_cannot_take(dtype, d):
+    """fp32 shards, and bf16 shards of 32-element rows, each above gemm_plan's minimum size: the tcgen05 GEMM takes
+    neither, so recommend_batch must serve them through the sharded single-query path, with the single-GPU answer."""
+    world = min(torch.cuda.device_count(), 8)
+    if world < 2:
+        pytest.skip("needs >= 2 GPUs")
+    from robot_ebert_b200 import CatalogStore, synth
+    n, b, k = 20_000 * world, 12, 10
+    results = _spawn("_routing_batch_worker", world, n, d, dtype, b, k)
+    store = CatalogStore.synthetic(0, n, d, dtype, scale_rows=True, device="cuda:0")
+    lp, lc, ep, ec = _csr_users(n, b)
+    wq = store.recommend_batch(queries=synth.catalog_rows_f32(11, 0, b, d), excl_ptr=ep, excl_col=ec, k=k)
+    wp = store.recommend_batch(liked_ptr=lp, liked_col=lc, excl_ptr=ep, excl_col=ec, k=k)
+    for rank, rq, rp in results:
+        for got, want in ((rq, wq), (rp, wp)):
+            assert got[0] == want[0].tolist() and got[2] == want[2].tolist(), rank
+            np.testing.assert_allclose(got[1], want[1], rtol=1e-12)

@@ -5,12 +5,14 @@ import numpy as np
 import pytest
 
 
-def _quantize_rows(x):
+def _quantize_rows(x, nrm=None):
+    """x: fp32 rows [n, d]; nrm: fp64 row norms (zero -> 1), recomputed here when not given."""
     mx = np.abs(x).max(axis=1).astype(np.float32)
     scale = np.where(mx > 0, mx / np.float32(127), np.float32(1)).astype(np.float32)
     q8 = np.clip(np.rint(x / scale[:, None]), -127, 127).astype(np.int32)
-    nrm = np.linalg.norm(x.astype(np.float64), axis=1)
-    nrm[nrm == 0] = 1.0
+    if nrm is None:
+        nrm = np.linalg.norm(x.astype(np.float64), axis=1)
+        nrm[nrm == 0] = 1.0
     err = np.linalg.norm(x.astype(np.float64) - q8 * scale[:, None].astype(np.float64), axis=1) / nrm
     factor = (scale.astype(np.float64) / nrm).astype(np.float32)
     return q8, factor, err.max()
