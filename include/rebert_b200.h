@@ -278,11 +278,15 @@ REBERT_API int rebert_scores_dense(const rebert_catalog_t* cat, const float* q32
 typedef struct {
     int32_t b;            /* queries */
     int32_t k;            /* results per query */
-    int32_t kc;           /* exact-pass candidates per query (from rebert_candidates_for_k) */
+    int32_t kc;           /* exact-pass candidates per query */
     int32_t sample_rows;  /* catalog rows in the threshold sample (multiple of 256) */
     int32_t sample_rank;  /* order statistic of the sample used as the threshold */
     int32_t cand_cap;     /* per-query capacity of the filtered candidate buffer */
 } rebert_gemm_plan_t;
+/* Plan for b queries of top-k over an n-row catalog (shard).  k <= 240: kc = round32(max(k + 16, 1.25 k)), sample rank 16,
+ * ~max(8 kc, 1024) survivors.  241 <= k <= 2048 (long lists, their own selection and exact-pass kernels): the same kc (up
+ * to 2560), sample rank 64, max(3 kc, 3200) survivors, so the sample is <= 2 % of the GEMM.  k > 2048: REBERT_ERR_UNSUPPORTED.
+ * A catalog with fewer than 64 x survivors rows is REBERT_ERR_UNSUPPORTED ("too small"): serve it one query at a time. */
 REBERT_API int    rebert_gemm_plan(int64_t n, int32_t b, int32_t k, rebert_gemm_plan_t* plan);
 REBERT_API size_t rebert_gemm_workspace_bytes(const rebert_catalog_t* cat, const rebert_gemm_plan_t* plan);
 /* Whole batched path: sample -> per-query threshold -> full GEMM with fused scale + threshold filter -> per-query
@@ -305,6 +309,7 @@ REBERT_API int rebert_gemm_topk(const rebert_catalog_t* cat, const void* qbf16, 
  * rebert_gemm_topk, and a query whose proof margin does not clear its bound gets out_status != 0 and is re-run by the
  * caller on the single-query path, whose bound is rigorous.
  *   rebert_gemm_plan_i8       as rebert_gemm_plan, with the wider candidate list the larger filter error needs
+ *                             (kc = round32(k + max(k, 64)), up to 4096 at k = 2048)
  *   rebert_query_quantize_i8  qn32 [b, ld] unit queries / profiles -> q8 [b, ld8] int8, qscale [b] (dequantisation step),
  *                             qeps [b] = the margin a result of that query must clear: 6 sigma of the score error under the
  *                             random-direction model, sigma = sqrt(row_err^2 + rho_q^2) / sqrt(d) with row_err the shadow's

@@ -436,12 +436,22 @@ class CatalogStore:
         """k > 240: see large_k_search — count-only sweeps for the bisection, then collect + fp64 re-score."""
         if liked_rows is not None and len(liked_rows) == 0:
             raise ValueError("Found array with 0 sample(s): user has no liked movies in the catalog")
-        if k > self.SWEEP_CAP // 2:
-            raise ValueError(f"k={k} is too large (limit {self.SWEEP_CAP // 2})")
+        self._check_large_k(k)
         with torch.cuda.device(self.device):
             excl_ptr, ne = self.stage_inputs(query, liked_rows, weights, exclude_rows, 1, 32)
-            return large_k_search(lambda thr: self.count_above(thr, excl_ptr, ne, row_filter),
-                                  lambda thr: self.sweep_above(thr, excl_ptr, ne, row_filter), k, self.fast_eps)
+            return self.topk_prepared_large_k(k, excl_ptr, ne, row_filter)
+
+    def _check_large_k(self, k: int):
+        if k > self.SWEEP_CAP // 2:
+            raise ValueError(f"k={k} is too large (limit {self.SWEEP_CAP // 2})")
+
+    def topk_prepared_large_k(self, k: int, excl_ptr=None, n_excl: int = 0, row_filter: Optional[RowFilter] = None):
+        """Exact top-k for k > 240 (up to SWEEP_CAP / 2) for the query / profile already in this thread's scratch (qn32, qn64):
+        large_k_search over count_above / sweep_above.  About 10-20 count-only passes over the catalog plus a sweep per
+        call, so the batched path sends only the queries its own passes could not prove."""
+        self._check_large_k(k)
+        return large_k_search(lambda thr: self.count_above(thr, excl_ptr, n_excl, row_filter),
+                              lambda thr: self.sweep_above(thr, excl_ptr, n_excl, row_filter), k, self.fast_eps)
 
     def count_above(self, threshold: float, excl_ptr=None, n_excl: int = 0, row_filter: Optional[RowFilter] = None) -> int:
         """Number of allowed rows of this shard whose fast score >= threshold (count-only sweep; query / profile from this
@@ -774,6 +784,9 @@ class CatalogStore:
         if (queries is None) == (liked_ptr is None):
             raise ValueError("pass exactly one of queries / liked CSR")
         lib = nat.load()
+        long_list = k > 0 and lib.rebert_candidates_for_k(k) == 0       # k > 240: beyond the single-query kernel
+        if long_list:
+            self._check_large_k(k)
         dev = self.device
         with torch.cuda.device(dev):
             if queries is not None:
@@ -803,16 +816,10 @@ class CatalogStore:
                     raise ValueError("exclusion CSR must have one segment per query")
                 ep = torch.from_numpy(excl_ptr).to(dev)
                 ec = torch.from_numpy(excl_col).to(dev)
-            ws = torch.empty(lib.rebert_gemm_workspace_bytes(C.byref(self._c), C.byref(plan)), dtype=torch.uint8, device=dev)
-            out_rows = torch.empty((b, k), dtype=torch.int64, device=dev)
-            out_scores = torch.empty((b, k), dtype=torch.float64, device=dev)
-            out_count = torch.empty(b, dtype=torch.int32, device=dev)
-            out_status = torch.empty(b, dtype=torch.int32, device=dev)
-            self.enqueue_batch(plan, qbf, qn64, ep, ec, ws, out_rows, out_scores, out_count, out_status, row_filter,
-                               shadow=self.quantize_queries(qn32) if use_shadow else None)
-            rows, scores = out_rows.cpu().numpy(), out_scores.cpu().numpy()
-            counts, status = out_count.cpu().numpy(), out_status.cpu().numpy()
+            rows, scores, counts, status = self._run_batch(plan, qbf, qn64, qn32, ep, ec, row_filter, use_shadow)
             redo = np.nonzero(status)[0]
+            if len(redo) and long_list:
+                redo = self._widened_retry(redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts)
             if len(redo):
                 s = self._scratch()
                 ecp = None if excl_ptr is None else np.asarray(excl_ptr, dtype=np.int64)
@@ -822,21 +829,72 @@ class CatalogStore:
                     ptr, ne = None, 0
                     if ecp is not None and ecp[u + 1] > ecp[u]:
                         ptr, ne = ec.data_ptr() + 4 * int(ecp[u]), int(ecp[u + 1] - ecp[u])
-                    r, sc = self.topk_prepared(k, ptr, ne, row_filter)
+                    if long_list:
+                        r, sc = self.topk_prepared_large_k(k, ptr, ne, row_filter)
+                    else:
+                        r, sc = self.topk_prepared(k, ptr, ne, row_filter)
                     rows[u, :], scores[u, :] = -1, -np.inf
                     rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
         if return_info:
-            return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}, "int8_operands": use_shadow}
+            return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}, "int8_operands": use_shadow,
+                                          "per_query": len(redo)}
         return rows, scores, counts
 
+    # Largest k of the tensor-core path (rebert_gemm_plan); also the cap of the widened retry of long lists.
+    BATCH_MAX_K = 2048
+
+    def _run_batch(self, plan, qbf, qn64, qn32, ep, ec, row_filter, use_shadow):
+        """One batched pass with freshly allocated workspace and outputs; returns host (rows, scores, counts, status)."""
+        lib = nat.load()
+        dev = self.device
+        b, k = plan.b, plan.k
+        ws = torch.empty(lib.rebert_gemm_workspace_bytes(C.byref(self._c), C.byref(plan)), dtype=torch.uint8, device=dev)
+        out_rows = torch.empty((b, k), dtype=torch.int64, device=dev)
+        out_scores = torch.empty((b, k), dtype=torch.float64, device=dev)
+        out_count = torch.empty(b, dtype=torch.int32, device=dev)
+        out_status = torch.empty(b, dtype=torch.int32, device=dev)
+        self.enqueue_batch(plan, qbf, qn64, ep, ec, ws, out_rows, out_scores, out_count, out_status, row_filter,
+                           shadow=self.quantize_queries(qn32) if use_shadow else None)
+        return out_rows.cpu().numpy(), out_scores.cpu().numpy(), out_count.cpu().numpy(), out_status.cpu().numpy()
+
+    def _widened_retry(self, redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts):
+        """Long lists: the queries the batched pass could not prove run once more, as a sub-batch at k' = min(2k, 2048) with
+        its longer candidate list, and keep the first k results (a proven top-k' starts with the proven top-k).  Much cheaper
+        than the per-query route when it works.  Fills rows / scores / counts in place; returns the queries still unproven."""
+        k2 = min(2 * k, self.BATCH_MAX_K)
+        if k2 <= k:
+            return redo
+        try:
+            plan = self.gemm_plan(len(redo), k2, shadow=use_shadow)
+        except nat.NativeError as e:
+            if e.code != nat.ERR_UNSUPPORTED:
+                raise
+            return redo                          # catalog too small for the plan at k'
+        dev = self.device
+        idx = torch.from_numpy(redo).to(dev)
+        ep = ec = None
+        if excl_ptr is not None:                 # excl_ptr / excl_col: the sorted CSR of the whole batch
+            segs = [np.asarray(excl_col[excl_ptr[u]:excl_ptr[u + 1]], dtype=np.int32) for u in redo]
+            sub_ptr = np.zeros(len(redo) + 1, dtype=np.int64)
+            np.cumsum([len(x) for x in segs], out=sub_ptr[1:])
+            ep = torch.from_numpy(sub_ptr).to(dev)
+            ec = torch.from_numpy(np.concatenate(segs) if sub_ptr[-1] else np.zeros(1, dtype=np.int32)).to(dev)
+        r2, s2, c2, st2 = self._run_batch(plan, qbf[idx].contiguous(), qn64[idx].contiguous(), qn32[idx].contiguous(), ep, ec,
+                                          row_filter, use_shadow)
+        ok = st2 == 0
+        for i in np.nonzero(ok)[0]:
+            u = redo[i]
+            rows[u], scores[u], counts[u] = r2[i, :k], s2[i, :k], min(int(c2[i]), k)
+        return redo[~ok]
+
     def _recommend_batch_loop(self, qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter=None):
-        """Small catalogs, and catalogs neither GEMM operand type takes: the batch is served by the single-query kernel, one
-        launch per prepared query."""
+        """Small catalogs, catalogs neither GEMM operand type takes, and k > 2048: the batch is served one prepared query at
+        a time, by the single-query kernel for k <= 240 and by topk_prepared_large_k above."""
         lib = nat.load()
         b = qn32.shape[0]
         kc = lib.rebert_candidates_for_k(k)
         if kc == 0:
-            raise ValueError(f"k={k} is outside the supported range (1..240)")
+            self._check_large_k(k)
         rows = np.full((b, k), -1, dtype=np.int64)
         scores = np.full((b, k), -np.inf, dtype=np.float64)
         counts = np.zeros(b, dtype=np.int32)
@@ -851,10 +909,10 @@ class CatalogStore:
             ptr, ne = None, 0
             if ecp is not None and ecp[u + 1] > ecp[u]:
                 ptr, ne = ec.data_ptr() + 4 * int(ecp[u]), int(ecp[u + 1] - ecp[u])
-            r, sc = self.topk_prepared(k, ptr, ne, row_filter)
+            r, sc = self.topk_prepared(k, ptr, ne, row_filter) if kc else self.topk_prepared_large_k(k, ptr, ne, row_filter)
             rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
         if return_info:
-            return rows, scores, counts, {"status": np.zeros(b, dtype=np.int32), "plan": None}
+            return rows, scores, counts, {"status": np.zeros(b, dtype=np.int32), "plan": None, "per_query": b}
         return rows, scores, counts
 
     # ------------------------------------------------------------------ diagnostics -------------

@@ -66,6 +66,104 @@ finalize_topk_kernel(const T* __restrict__ rows, const double* __restrict__ norm
                           out_scores + (size_t)u * k, out_count + u, out_margin ? out_margin + u : nullptr, s_tmp, &s_kth, err_mult);
 }
 
+// Long lists of the batched path (k > 240, kc <= 4096).  The re-score is finalize_topk_kernel's (exact_score_row<T, false>:
+// the same bits); the ranking is a bitonic sort of (orderable fp64 score, local row) pairs in shared memory — kc log^2 kc
+// steps instead of rank_candidates' kc x kc count, which at kc = 4096 would be 16 M compares per query.  Results, margin and
+// the 4-ulp near-tie rule are those of rank_candidates<true>: in sorted order two distinct scores within 4 ulp of each other
+// are adjacent, and the pair counts when the higher score's first position is at or above place k, i.e. ord[k] <= ord[i].
+// Dynamic shared memory: [ld] query planes, [p2] keys, [p2] rows (p2 = the power of two >= kc).
+__device__ __forceinline__ bool pair_before(unsigned long long ka, uint32_t ra, unsigned long long kb, uint32_t rb) {
+    return ka > kb || (ka == kb && ra < rb);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kFinalThreads, 2)
+finalize_large_kernel(const T* __restrict__ rows, const double* __restrict__ norm64, int64_t row_base, int64_t n, int ld,
+                      const double* __restrict__ q64, const uint64_t* __restrict__ cand_keys, int kc, int p2, int k,
+                      int64_t* __restrict__ out_rows, double* __restrict__ out_scores, int32_t* __restrict__ out_count,
+                      double* __restrict__ out_margin, double err_mult) {
+    constexpr int EPC = ChunkDot<T>::EPC;
+    extern __shared__ __align__(16) double s_q[];
+    unsigned long long* s_ord = (unsigned long long*)(s_q + ld);
+    uint32_t* s_lr = (uint32_t*)(s_ord + p2);
+    __shared__ unsigned long long s_maxerr;
+    __shared__ int s_valid, s_near;
+    const int u = blockIdx.x;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+    pdl_trigger();
+    pdl_wait();                                      // the candidates come from the kernel launched just before
+    const uint64_t* keys = cand_keys + (size_t)u * kc;
+    stage_query_planes(q64 + (size_t)u * ld, ld, EPC, s_q);
+    if (threadIdx.x == 0) { s_maxerr = 0ull; s_valid = 0; s_near = 0; }
+    for (int c = kc + threadIdx.x; c < p2; c += blockDim.x) { s_ord[c] = 0ull; s_lr[c] = 0xFFFFFFFFu; }
+    __syncthreads();
+    const QueryPlanes qsrc{s_q, ld / EPC};
+    for (int c = warp; c < kc; c += nwarps) {
+        const uint64_t key = keys[c];
+        unsigned long long ord = 0ull;
+        uint32_t lr = 0xFFFFFFFFu;
+        if (key != 0) {
+            lr = key_row(key);
+            REBERT_ASSERT((int64_t)lr < n);
+            const double sc = exact_score_row<T, false>(rows, ld, norm64, lr, qsrc, lane);
+            ord = f64_orderable(sc);
+            if (lane == 0) atomicMax(&s_maxerr, (unsigned long long)__double_as_longlong(fabs(sc - (double)key_score(key))));
+        }
+        if (lane == 0) {
+            REBERT_ASSERT(c < p2);
+            s_ord[c] = ord;
+            s_lr[c] = lr;
+        }
+    }
+    __syncthreads();
+    for (int w = 2; w <= p2; w <<= 1) {
+        for (int j = w >> 1; j > 0; j >>= 1) {
+            for (int i = threadIdx.x; i < p2; i += blockDim.x) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const unsigned long long x = s_ord[i], y = s_ord[ixj];
+                    const uint32_t rx = s_lr[i], ry = s_lr[ixj];
+                    const bool desc = (i & w) == 0;
+                    if (desc ? pair_before(y, ry, x, rx) : pair_before(x, rx, y, ry)) {
+                        s_ord[i] = y; s_ord[ixj] = x;
+                        s_lr[i] = ry; s_lr[ixj] = rx;
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    const unsigned long long ord_k = s_ord[k];       // k < kc <= p2; 0 when fewer than k + 1 candidates are valid
+    for (int i = threadIdx.x; i < p2; i += blockDim.x) {
+        const unsigned long long a = s_ord[i];
+        if (a == 0ull) continue;
+        const unsigned long long nb = i + 1 < p2 ? s_ord[i + 1] : 0ull;
+        if (nb == 0ull) s_valid = i + 1;             // the last valid entry: exactly one thread
+        else if (a != nb && a - nb <= 4ull && ord_k <= a) s_near = 1;
+    }
+    __syncthreads();
+    const int valid = s_valid;
+    const int nout = valid < k ? valid : k;
+    int64_t* o_rows = out_rows + (size_t)u * k;
+    double* o_scores = out_scores + (size_t)u * k;
+    for (int i = threadIdx.x; i < k; i += blockDim.x) {
+        REBERT_ASSERT(i < p2);
+        o_rows[i] = i < nout ? row_base + s_lr[i] : -1;
+        o_scores[i] = i < nout ? f64_from_orderable(s_ord[i]) : -INFINITY;
+    }
+    if (threadIdx.x == 0) {
+        out_count[u] = nout;
+        if (out_margin) {
+            const uint64_t last = keys[kc - 1];
+            double mg = (last != 0 && valid >= k) ? f64_from_orderable(s_ord[k - 1]) - (double)key_score(last) -
+                                                        err_mult * __longlong_as_double((long long)s_maxerr)
+                                                  : INFINITY;
+            if (s_near) mg = -INFINITY;
+            out_margin[u] = mg;
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // Request path, second (and last) launch: a CLUSTER of 8 CTAs placed behind the streaming kernel by programmatic dependent
 // launch.  The streaming kernel's CTAs have published their pruned candidate keys (gemv_topk.cu); here
@@ -408,6 +506,28 @@ int finalize_launch(const rebert_catalog_t* cat, const double* q64, const uint64
                            : finalize_launch_t<float, false>(cat, q64, cand_keys, b, kc, k, out_rows, out_scores, out_count, out_margin, st, err_mult);
     return exact_order ? finalize_launch_t<__nv_bfloat16, true>(cat, q64, cand_keys, b, kc, k, out_rows, out_scores, out_count, out_margin, st, err_mult)
                        : finalize_launch_t<__nv_bfloat16, false>(cat, q64, cand_keys, b, kc, k, out_rows, out_scores, out_count, out_margin, st, err_mult);
+}
+
+// Exact pass of the batched path's long lists (finalize_large_kernel): divide-after formula, near-ties flagged via the margin.
+int finalize_large_launch(const rebert_catalog_t* cat, const double* q64, const uint64_t* cand_keys, int b, int kc, int k,
+                          int64_t* out_rows, double* out_scores, int32_t* out_count, double* out_margin, cudaStream_t st, double err_mult) {
+    REBERT_REQUIRE(kc > 0 && k > 0 && k < kc, "finalize_large: k=%d kc=%d", k, kc);
+    int p2 = 2;
+    while (p2 < kc) p2 <<= 1;
+    const size_t smem = (size_t)cat->ld * sizeof(double) + (size_t)p2 * (sizeof(unsigned long long) + sizeof(uint32_t));
+    if (cat->dtype == REBERT_F32) {
+        auto kern = finalize_large_kernel<float>;
+        { int rc = raise_smem_limit(kern); if (rc != REBERT_OK) return rc; }
+        REBERT_CUDA(launch_pdl(kern, dim3(b), dim3(kFinalThreads), smem, st, (const float*)cat->rows, cat->norm64, cat->row_base, cat->n,
+                               cat->ld, q64, cand_keys, kc, p2, k, out_rows, out_scores, out_count, out_margin, err_mult));
+    } else {
+        auto kern = finalize_large_kernel<__nv_bfloat16>;
+        { int rc = raise_smem_limit(kern); if (rc != REBERT_OK) return rc; }
+        REBERT_CUDA(launch_pdl(kern, dim3(b), dim3(kFinalThreads), smem, st, (const __nv_bfloat16*)cat->rows, cat->norm64, cat->row_base,
+                               cat->n, cat->ld, q64, cand_keys, kc, p2, k, out_rows, out_scores, out_count, out_margin, err_mult));
+    }
+    REBERT_CUDA(cudaGetLastError());
+    return REBERT_OK;
 }
 
 }  // namespace rebert

@@ -13,6 +13,8 @@
 //      and appends (score,row) keys to cand[q] with one atomicAdd per thread per tile
 //   4. select_candidates: per query, drop excluded rows, bucket-select + small bitonic sort -> best kc keys
 //   5. finalize_topk (csrc/finalize.cu): fp64 re-score, (score desc, row asc), best k, proof margin
+//   Long lists (241 <= k <= 2048, kc up to 4096) use sample rank 64 with ~3 kc survivors, and their own stages 4 and 5:
+//   select_candidates_large (histogram over the global buffer, gather + sort) and finalize_large (bitonic ranking).
 //   status[q] != 0 tells the caller to re-run that query through the single-query kernel (threshold too optimistic,
 //   staging / buffer overflow, margin below eps or a sub-4-ulp gap) — exactness never depends on the sample being lucky.
 //
@@ -38,6 +40,8 @@ namespace rebert {
 int finalize_launch(const rebert_catalog_t* cat, const double* q64, const uint64_t* cand_keys, int b, int kc, int k,
                     int64_t* out_rows, double* out_scores, int32_t* out_count, double* out_margin, cudaStream_t st,
                     bool exact_order, double err_mult = 4.0);
+int finalize_large_launch(const rebert_catalog_t* cat, const double* q64, const uint64_t* cand_keys, int b, int kc, int k,
+                          int64_t* out_rows, double* out_scores, int32_t* out_count, double* out_margin, cudaStream_t st, double err_mult);
 
 constexpr int BM = 128, BN = 256, BK = 64, UK = 16;
 constexpr int GEMM_STAGES = 4;
@@ -48,6 +52,8 @@ constexpr int SMEM_STAGING = STAGE_SLOTS * 128 * 8;
 constexpr int SMEM_INV = 2 * BN * 4;
 constexpr int GEMM_SMEM = GEMM_STAGES * STAGE_BYTES + SMEM_STAGING + SMEM_INV + 256 + 1024;   // + alignment slack
 constexpr uint32_t TMEM_COLS = 512;
+// k above kLargeK0 (the single-query kernel's limit) takes the long-list stages; kLargeKMax bounds kc at 4096 (int8 plans)
+constexpr int kLargeK0 = 240, kLargeKMax = 2048, kLargeRank = 64, kLargeKcMax = 4096;
 
 enum { MODE_STORE = 0, MODE_FILTER = 1 };
 
@@ -745,6 +751,122 @@ __global__ void __launch_bounds__(512) select_candidates_kernel(const uint64_t* 
     }
 }
 
+// Long lists (k > 240, kc up to 4096): the survivors (~3 kc, up to cand_cap = 64 Ki keys) stay in global memory.  Per query:
+//   pass 1  drop excluded rows (zeroed in place, so later passes skip the search) and find the score range [lo, hi];
+//   pass 2  only when more than gather_cap keys are valid: histogram of the scores over 2048 linear buckets of [lo, hi], and
+//           the bucket b* that holds the kc-th best (suffix sums: one lane per 64 buckets, then one lane walks its 64);
+//   pass 3  gather every key from bucket b* upwards (kc plus part of one bucket) into shared memory, bitonic sort, write the
+//           best kc.
+// gather_cap = the power of two >= 2 kc.  A gathered set larger than that (mass ties inside one bucket) sets status bit 16 and
+// writes no keys: the caller re-runs the query, nothing is dropped silently.  Bits 2 and 4 as in select_candidates_kernel.
+constexpr int kSelLargeThreads = 512, kSelLargeBuckets = 2048;
+
+__device__ __forceinline__ int large_bucket(uint64_t key, unsigned lo, unsigned long long range) {
+    return (int)(((unsigned long long)((unsigned)(key >> 32) - lo) * (unsigned long long)kSelLargeBuckets) / range);
+}
+
+__global__ void __launch_bounds__(kSelLargeThreads) select_candidates_large_kernel(uint64_t* __restrict__ cand, const unsigned* __restrict__ cand_count,
+                                                                              int cand_cap, int kc, int gather_cap, int64_t row_base,
+                                                                              const int64_t* __restrict__ excl_ptr,
+                                                                              const int32_t* __restrict__ excl_col,
+                                                                              const float* __restrict__ tau, uint64_t* __restrict__ out_keys,
+                                                                              int* __restrict__ status) {
+    extern __shared__ __align__(16) uint64_t top[];        // [gather_cap]
+    __shared__ unsigned hist[kSelLargeBuckets];
+    __shared__ int s_valid, s_m, s_bstar, s_n;
+    __shared__ unsigned s_lo, s_hi;
+    const int q = blockIdx.x;
+    const unsigned cnt_raw = cand_count[q];
+    const int cnt = cnt_raw < (unsigned)cand_cap ? (int)cnt_raw : cand_cap;
+    uint64_t* src = cand + (size_t)q * cand_cap;
+    const int32_t* ex = nullptr;
+    int nex = 0;
+    if (excl_ptr) { ex = excl_col + excl_ptr[q]; nex = (int)(excl_ptr[q + 1] - excl_ptr[q]); }
+    if (threadIdx.x == 0) { s_valid = 0; s_n = 0; s_lo = 0xFFFFFFFFu; s_hi = 0; s_bstar = 0; }
+    for (int i = threadIdx.x; i < kSelLargeBuckets; i += blockDim.x) hist[i] = 0;
+    __syncthreads();
+    int mine = 0;
+    unsigned lo = 0xFFFFFFFFu, hi = 0;
+    for (int i = threadIdx.x; i < cnt; i += blockDim.x) {
+        const uint64_t key = src[i];
+        if (!key) continue;
+        if (nex && sorted_contains(ex, nex, (int32_t)(row_base + key_row(key)))) { src[i] = 0; continue; }
+        ++mine;
+        lo = min(lo, (unsigned)(key >> 32));
+        hi = max(hi, (unsigned)(key >> 32));
+    }
+    if (mine) { atomicAdd(&s_valid, mine); atomicMin(&s_lo, lo); atomicMax(&s_hi, hi); }
+    __syncthreads();
+    const int valid = s_valid;
+    const unsigned blo = s_lo;
+    const unsigned long long range = (unsigned long long)(s_hi - blo) + 1ull;   // only used when valid > 0
+    int m = valid, bstar = 0;                                // few enough valid keys: gather them all
+    if (valid > gather_cap && s_hi > blo) {
+        for (int i = threadIdx.x; i < cnt; i += blockDim.x) {
+            const uint64_t key = src[i];
+            if (key) atomicAdd(&hist[large_bucket(key, blo, range)], 1u);
+        }
+        __syncthreads();
+        if (threadIdx.x < 32) {
+            constexpr int PER = kSelLargeBuckets / 32;
+            const int lane = threadIdx.x;
+            const int top_b = kSelLargeBuckets - lane * PER;  // lane 0 owns the best buckets [B - 64, B)
+            unsigned sum = 0;
+            for (int j = 1; j <= PER; ++j) sum += hist[top_b - j];
+            unsigned incl = sum;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += v;
+            }
+            const unsigned ballot = __ballot_sync(0xffffffffu, incl >= (unsigned)kc);   // != 0: valid > gather_cap > kc
+            if (lane == __ffs(ballot) - 1) {
+                unsigned cum = incl - sum;
+                int bb = top_b - 1;
+                for (; bb > top_b - PER; --bb) {
+                    cum += hist[bb];
+                    if (cum >= (unsigned)kc) break;
+                }
+                if (cum < (unsigned)kc) cum += hist[bb];      // the walk ended on the lane's lowest bucket
+                s_bstar = bb;
+                s_m = (int)cum;
+            }
+        }
+        __syncthreads();
+        m = s_m;
+        bstar = s_bstar;
+    } else if (valid > gather_cap) {
+        m = valid;                                           // every valid key has the same score: cannot split
+    }
+    const bool fits = m <= gather_cap;
+    if (fits) {
+        for (int i = threadIdx.x; i < cnt; i += blockDim.x) {
+            const uint64_t key = src[i];
+            if (key && large_bucket(key, blo, range) >= bstar) {
+                const int idx = atomicAdd(&s_n, 1);
+                REBERT_ASSERT(idx >= 0 && idx < gather_cap);
+                top[idx] = key;
+            }
+        }
+        int t2 = 2;
+        while (t2 < m || t2 < kc) t2 <<= 1;
+        for (int i = m + threadIdx.x; i < t2; i += blockDim.x) top[i] = 0;
+        __syncthreads();
+        block_bitonic_sort_desc(top, t2);
+    }
+    for (int i = threadIdx.x; i < kc; i += blockDim.x) {
+        REBERT_ASSERT(i < gather_cap);
+        out_keys[(size_t)q * kc + i] = fits ? top[i] : 0ull;
+    }
+    if (threadIdx.x == 0) {
+        int st = status[q];
+        if (cnt_raw > (unsigned)cand_cap) st |= 2;                         // buffer overflow: some survivors were dropped
+        if (valid < kc && tau[q] != -INFINITY) st |= 4;                    // threshold too optimistic: not enough candidates
+        if (!fits) st |= 16;                                               // mass ties: the kc best could not be isolated
+        status[q] = st;
+    }
+}
+
 __global__ void margin_status_kernel(const double* __restrict__ margin, double eps, int b, int* __restrict__ status) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q < b && !(margin[q] > eps)) status[q] |= 8;
@@ -934,10 +1056,37 @@ static int gemm_plan_impl(int64_t n, int32_t b, int32_t k, bool shadow, rebert_g
     // int8 operands (shadow): the score error is ~10x larger (sigma ~ 0.009 / sqrt(d) per unit of row and query error), and
     // the margin has to clear 6 sigma plus twice the largest error seen on the candidates — ~0.16 standard deviations of the
     // score distribution, i.e. ~0.7 k more rows at the densities of a 1M..10M catalog (k z rows per unit z): the list doubles.
-    if (rebert_candidates_for_k(k) == 0) { set_error("gemm_plan: k=%d unsupported", k); return REBERT_ERR_UNSUPPORTED; }
+    if (k > kLargeKMax || (k <= kLargeK0 && rebert_candidates_for_k(k) == 0)) {
+        set_error("gemm_plan: k=%d unsupported", k);
+        return REBERT_ERR_UNSUPPORTED;
+    }
     int need = k + 16 > k + (k + 3) / 4 ? k + 16 : k + (k + 3) / 4;
     if (shadow) need = k + (k > 64 ? k : 64);
     const int kc = (need + 31) / 32 * 32;
+    if (k > kLargeK0) {
+        // Long lists (k > 240, served by select_candidates_large_kernel + finalize_large_kernel).  The sample rank is 64 and
+        // the survivor target E = max(3 kc, 50 x 64): P(Gamma(64) < 64 / 3) = 7e-14 that fewer than kc rows pass, and the
+        // sample is rank / E <= 2 % of the rows (sample tiles round down, which only raises E).  E <= n / 64 as below.
+        const int rank = kLargeRank;
+        double e = 3.0 * kc;
+        if (e < 50.0 * rank) e = 50.0 * rank;
+        if (e > (double)n / 64.0) {
+            set_error("gemm_plan: catalog of %lld rows is too small for the batched path at k=%d (needs >= %lld rows); "
+                      "use the single-query path", (long long)n, k, (long long)(64.0 * e));
+            return REBERT_ERR_UNSUPPORTED;
+        }
+        int64_t st = (int64_t)((double)n * rank / e / BN);
+        if (st < 1) st = 1;
+        plan->b = b;
+        plan->k = k;
+        plan->kc = kc;
+        plan->sample_rows = (int32_t)(st * BN);
+        plan->sample_rank = rank;
+        int cap = 2 * kc;
+        while (cap < 4.0 * e) cap <<= 1;
+        plan->cand_cap = cap;
+        return REBERT_OK;
+    }
     // Expected survivors per query E = rank * n / sample_rows.  Want E >= 8 kc (the kc best are then inside with
     // overwhelming probability: the survivor count is Gamma(rank)-distributed around E) plus headroom for excluded
     // rows, which tend to score high; and E <= n / 64 so a thread stages ~4 keys per tile on average (24 slots).
@@ -1020,6 +1169,9 @@ static int gemm_topk_impl(const rebert_catalog_t* cat, const rebert_catalog_t* o
     REBERT_REQUIRE(!shadow || (qscale && qeps && op->n == cat->n && op->d == cat->d && op->row_base == cat->row_base),
                    "gemm_topk: int8 operands need query scales / bounds and a shadow of the same shape as the catalog");
     REBERT_REQUIRE((excl_row_ptr == nullptr) == (excl_col == nullptr), "gemm_topk: exclusion CSR needs both arrays");
+    const bool large = plan->k > kLargeK0;                   // long lists: their own selection and exact-pass kernels
+    REBERT_REQUIRE(!large || (plan->k < plan->kc && plan->kc <= kLargeKcMax && plan->cand_cap > 0),
+                   "gemm_topk: plan k=%d kc=%d is not a long-list plan", plan->k, plan->kc);
     GemmWorkspace w = carve(workspace, plan);
     if (workspace_bytes < w.bytes) { set_error("gemm_topk: workspace %zu < %zu", workspace_bytes, w.bytes); return REBERT_ERR_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
@@ -1070,16 +1222,29 @@ static int gemm_topk_impl(const rebert_catalog_t* cat, const rebert_catalog_t* o
     rc = launch_gemm<MODE_FILTER>(op, qbf16, p, st);
     if (rc != REBERT_OK) return rc;
     // 4. per-query candidate selection
-    int p2 = 2;
-    while (p2 < plan->cand_cap) p2 <<= 1;
-    const size_t csmem = (size_t)(p2 + 1024) * 8;        // survivors + the bucket-selected top set
-    { int rc__ = raise_smem_limit(select_candidates_kernel); if (rc__ != REBERT_OK) return rc__; }
-    select_candidates_kernel<<<b, 512, csmem, st>>>(w.cand, w.cand_count, plan->cand_cap, plan->kc, cat->row_base, excl_row_ptr,
-                                                    excl_col, w.tau, w.cand_keys, out_status);
+    if (large) {
+        int gcap = 2;
+        while (gcap < 2 * plan->kc) gcap <<= 1;
+        { int rc__ = raise_smem_limit(select_candidates_large_kernel); if (rc__ != REBERT_OK) return rc__; }
+        select_candidates_large_kernel<<<b, kSelLargeThreads, (size_t)gcap * 8, st>>>(w.cand, w.cand_count, plan->cand_cap, plan->kc, gcap,
+                                                                                      cat->row_base, excl_row_ptr, excl_col, w.tau,
+                                                                                      w.cand_keys, out_status);
+    } else {
+        int p2 = 2;
+        while (p2 < plan->cand_cap) p2 <<= 1;
+        const size_t csmem = (size_t)(p2 + 1024) * 8;        // survivors + the bucket-selected top set
+        { int rc__ = raise_smem_limit(select_candidates_kernel); if (rc__ != REBERT_OK) return rc__; }
+        select_candidates_kernel<<<b, 512, csmem, st>>>(w.cand, w.cand_count, plan->cand_cap, plan->kc, cat->row_base, excl_row_ptr,
+                                                        excl_col, w.tau, w.cand_keys, out_status);
+    }
     REBERT_CUDA(cudaGetLastError());
-    // 5. exact pass
-    rc = finalize_launch(cat, q64, w.cand_keys, b, plan->kc, plan->k, out_rows, out_scores, out_count, w.margin, st,
-                         /*exact_order=*/false, shadow ? 2.0 : 4.0);   // near-ties come back as margin = -inf and are re-run by the caller
+    // 5. exact pass; near-ties come back as margin = -inf and are re-run by the caller
+    if (large)
+        rc = finalize_large_launch(cat, q64, w.cand_keys, b, plan->kc, plan->k, out_rows, out_scores, out_count, w.margin, st,
+                                   shadow ? 2.0 : 4.0);
+    else
+        rc = finalize_launch(cat, q64, w.cand_keys, b, plan->kc, plan->k, out_rows, out_scores, out_count, w.margin, st,
+                             /*exact_order=*/false, shadow ? 2.0 : 4.0);
     if (rc != REBERT_OK) return rc;
     if (shadow) {
         // int8 operands: the margin (exact k-th - fast score of the worst kept candidate - 2 x the largest |fast - exact| seen on

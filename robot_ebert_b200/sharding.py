@@ -573,7 +573,9 @@ class ShardedCatalog:
     def recommend_batch(self, *, queries=None, liked_ptr=None, liked_col=None, liked_w=None, excl_ptr=None, excl_col=None,
                         k: int = 10, row_filter=None, return_info: bool = False):
         """Sharded form of CatalogStore.recommend_batch: every rank runs the tcgen05 pass over its rows, the per-rank
-        [b, k] results are all-gathered in ONE packed buffer and merged on every rank.  CUDA backend only."""
+        [b, k] results are all-gathered in ONE packed buffer and merged on every rank.  CUDA backend only.
+        k up to 2048 runs on the tensor cores when every shard is above the plan minimum (rebert_gemm_plan); the packed buffer
+        is 2 b k + b words per rank (128 MiB at b = 4096, k = 2048).  Larger k, and smaller shards, take the per-query loop."""
         store: CatalogStore = self.backend.store
         dev = store.device
         if (queries is None) == (liked_ptr is None):
@@ -616,7 +618,8 @@ class ShardedCatalog:
             rows[u, :], scores[u, :] = -1, -np.inf
             rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
         if return_info:
-            return rows, scores, counts, {"status": status}
+            plan = ctx["plan"]
+            return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}}
         return rows, scores, counts
 
     def _recommend_batch_loop(self, queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, return_info):
