@@ -163,6 +163,65 @@ def unpack_result(words: np.ndarray, k: int):
     return words[:cnt].copy(), words[k:k + cnt].view(np.float64).copy(), margin
 
 
+# same failure the reference hits: sklearn's check_array on an empty frame (SURVEY.md §3.2)
+EMPTY_PROFILE = "Found array with 0 sample(s): user has no liked movies in the catalog"
+
+
+def validated_table(ids, matrix, sort_ids: bool):
+    """Host catalog as fp32 [N, D] and its id table (str) checked against it; with sort_ids, both in ascending id order."""
+    matrix = np.asarray(matrix, dtype=np.float32)
+    if matrix.ndim != 2:
+        raise ValueError("matrix must be [N, D]")
+    n = matrix.shape[0]
+    if ids is not None:
+        if len(ids) != n:
+            raise ValueError("len(ids) != rows")
+        ids = [str(i) for i in ids]
+        if len(set(ids)) != n:
+            raise ValueError("duplicate ids")
+        if sort_ids:
+            order = sorted(range(n), key=ids.__getitem__)
+            if order != list(range(n)):
+                matrix = matrix[np.asarray(order)]
+                ids = [ids[i] for i in order]
+    return ids, matrix
+
+
+def topk_order(rows: np.ndarray, scores: np.ndarray, k: int):
+    """The first k of (rows, scores) in result order: score desc, row asc."""
+    order = np.lexsort((rows, -scores))[:k]
+    return rows[order], scores[order]
+
+
+def widen_until_proven(attempt, kc: int, eps: float):
+    """attempt(kc) -> (rows, scores, margin) with 4x more candidates each time, until the margin clears eps or kc reaches
+    256.  Returns (rows, scores, margin, kc) of the last attempt; the caller checks margin > eps."""
+    while True:
+        rows, scores, margin = attempt(kc)
+        if margin > eps or kc >= 256:
+            return rows, scores, margin, kc
+        kc = min(256, kc * 4)
+
+
+def close_proof(rows, scores, k: int, eps: float, margin: float, count, sweep):
+    """Fail closed: the exact top-k of a request whose candidate list (rows, scores) did not prove itself (margin <= eps),
+    or RuntimeError.  count / sweep as in large_k_search, over the staged request.
+
+    Mass ties: more rows than any candidate list holds sit within fp32 noise of the k-th score.  The sweep collects every
+    allowed row that could still belong to the top-k (fast score >= k-th exact score - 2 eps) and orders them by fp64
+    score: provably exact.  If it overflows (or fewer than k rows are allowed), the bisection route of large_k_search
+    handles any tie mass it can hold."""
+    if len(rows) == k:
+        res = sweep(float(scores[k - 1]) - 2.0 * eps)
+        if res is not None and len(res[0]) >= k:
+            return topk_order(res[0], res[1], k)
+    try:
+        return large_k_search(count, sweep, k, eps)
+    except RuntimeError as e:
+        raise RuntimeError(f"top-{k}: the result cannot be proven exact (margin {margin:.3e} <= {eps:.3e}) and the "
+                           f"exhaustive route failed: {e}") from e
+
+
 def large_k_search(count, sweep, k: int, eps: float):
     """Exact top-k for k beyond the register-list kernel (k > 240), on one shard or across shards.
 
@@ -189,11 +248,10 @@ def large_k_search(count, sweep, k: int, eps: float):
         res = sweep(thr)
         if res is None:
             raise RuntimeError("large-k sweep overflow: more than SWEEP_CAP rows within the threshold band")
-        rr, sc = res
-        order = np.lexsort((rr, -sc))[:k]
-        if len(rr) >= total or len(order) < k or sc[order[-1]] - 2.0 * eps > thr:
-            return rr[order], sc[order]
-        thr = float(sc[order[-1]]) - 4.0 * eps - 1e-6     # k-th exact score too close to the cut: widen
+        rr, sc = topk_order(res[0], res[1], k)
+        if len(res[0]) >= total or len(rr) < k or sc[-1] - 2.0 * eps > thr:
+            return rr, sc
+        thr = float(sc[-1]) - 4.0 * eps - 1e-6            # k-th exact score too close to the cut: widen
 
 
 class CatalogStore:
@@ -260,21 +318,8 @@ class CatalogStore:
         """Upload an [N, D] host matrix (what Chroma's collection.get returns, constants.py:55) and build the store."""
         dev = cls._require_cuda(device)
         lib = nat.load()
-        matrix = np.asarray(matrix, dtype=np.float32)
-        if matrix.ndim != 2:
-            raise ValueError("matrix must be [N, D]")
+        ids, matrix = validated_table(ids, matrix, sort_ids)
         n, d = matrix.shape
-        if ids is not None:
-            if len(ids) != n:
-                raise ValueError("len(ids) != rows")
-            ids = [str(i) for i in ids]
-            if sort_ids:
-                order = sorted(range(n), key=ids.__getitem__)
-                if order != list(range(n)):
-                    matrix = matrix[np.asarray(order)]
-                    ids = [ids[i] for i in order]
-            if len(set(ids)) != n:
-                raise ValueError("duplicate ids")
         ld, rows, inv_norm, norm64 = cls._alloc(n, d, dtype, dev)
         with torch.cuda.device(dev):
             st = torch.cuda.current_stream().cuda_stream
@@ -380,78 +425,60 @@ class CatalogStore:
             kc = self._kc_for_k[k] = lib.rebert_candidates_for_k(k)
         if kc == 0:
             # k beyond the register-list kernel (k > 240): threshold bisection + sweep, still exact (rare, slower path)
-            rows, scores = self._recommend_large_k(lib, query, liked_rows, weights, exclude_rows, k, row_filter)
+            rows, scores = self._recommend_large_k(query, liked_rows, weights, exclude_rows, k, row_filter)
             if return_info:
                 return rows, scores, {"kc": 0, "margin": float("inf"), "proven_exact": True, "exact_sweep": True}
             return rows, scores
         if prefilter and self._c8 is None:
             raise ValueError("prefilter=True needs enable_prefilter()")
-        shadow_max_k = 0
-        if self._c8 is not None and prefilter is not False:
-            shadow_max_k = 240 if prefilter else self.PREFILTER_MAX_K
-        rows, scores, info = self._recommend_host(query, liked_rows, weights, exclude_rows, k, kc, row_filter, shadow_max_k)
-        rows, scores, info = self._close_proof(lib, rows, scores, info, query, liked_rows, weights, exclude_rows, k, row_filter)
+        rows, scores, info = self._recommend_host(query, liked_rows, weights, exclude_rows, k, kc, row_filter,
+                                                  self.shadow_max_k(self._c8 is not None, prefilter))
+        if not info["proven_exact"]:
+            # fail closed: the margin proved nothing, so the exhaustive routes answer (close_proof) or the call raises
+            with torch.cuda.device(self.device):
+                excl_ptr, ne = self.stage_inputs(query, liked_rows, weights, exclude_rows, k, kc)   # the sweeps read qn32 / qn64
+                rows, scores = close_proof(rows, scores, k, self.fast_eps, info["margin"], *self._sweeps(excl_ptr, ne, row_filter))
+            info = dict(info, proven_exact=True, exact_sweep=True)
         if return_info:
             return rows, scores, info
         return rows, scores
-
-    def _close_proof(self, lib, rows, scores, info, query, liked_rows, weights, exclude_rows, k, row_filter):
-        """Fail closed: a result whose margin proved nothing goes through the exhaustive routes or raises."""
-        if info["proven_exact"]:
-            return rows, scores, info
-        res = None
-        if len(rows) == k:
-            # Mass ties: more rows than any candidate list holds sit within fp32 noise of the k-th score.  Sweep for every
-            # allowed row that could still belong to the top-k, re-score those in fp64, order them: provably exact.
-            res = self._exact_sweep(lib, query, liked_rows, weights, exclude_rows, k, row_filter, float(scores[k - 1]))
-        if res is None:
-            try:                                   # sweep buffer overflow: the bisection route handles any tie mass it can hold
-                res = self._recommend_large_k(lib, query, liked_rows, weights, exclude_rows, k, row_filter)
-            except RuntimeError as e:
-                raise RuntimeError(f"top-{k}: the result cannot be proven exact (margin {info['margin']:.3e} <= "
-                                   f"{self.fast_eps:.3e}) and the exhaustive route failed: {e}") from e
-        info = dict(info, proven_exact=True, exact_sweep=True)
-        return res[0], res[1], info
 
     # 256 candidates absorb the shadow's proven error bound (~0.009 for gaussian rows) only while the k-th and the 256-th
     # best scores are far enough apart; beyond k ~ 16 the proof usually fails and the attempt would be wasted work.
     PREFILTER_MAX_K = 16
 
+    @classmethod
+    def shadow_max_k(cls, has_shadow: bool, prefilter: Optional[bool]) -> int:
+        """Largest k for which a single request tries the int8 shadow first (0 = never); see recommend()'s `prefilter`."""
+        if not has_shadow or prefilter is False:
+            return 0
+        return 240 if prefilter else cls.PREFILTER_MAX_K
+
     SWEEP_CAP = 1 << 16
 
-    def _exact_sweep(self, lib, query, liked_rows, weights, exclude_rows, k, row_filter, kth_score):
-        """Fallback for results no candidate list can prove: collect every allowed row with fast score >= k-th exact
-        score - 2 eps (a superset of the true top-k), fp64 re-score them, order by (score desc, row asc)."""
-        with torch.cuda.device(self.device):
-            kc = lib.rebert_candidates_for_k(k)
-            excl_ptr, ne = self.stage_inputs(query, liked_rows, weights, exclude_rows, k, kc)   # refreshes qn32 / qn64
-            res = self.sweep_above(kth_score - 2.0 * self.fast_eps, excl_ptr, ne, row_filter)
-        if res is None or len(res[0]) < k:
-            return None
-        rr, sc = res
-        order = np.lexsort((rr, -sc))[:k]            # bookkeeping on the handful of survivors
-        return rr[order], sc[order]
-
-    def _recommend_large_k(self, lib, query, liked_rows, weights, exclude_rows, k, row_filter):
+    def _recommend_large_k(self, query, liked_rows, weights, exclude_rows, k, row_filter):
         """k > 240: see large_k_search — count-only sweeps for the bisection, then collect + fp64 re-score."""
-        if liked_rows is not None and len(liked_rows) == 0:
-            raise ValueError("Found array with 0 sample(s): user has no liked movies in the catalog")
         self._check_large_k(k)
         with torch.cuda.device(self.device):
             excl_ptr, ne = self.stage_inputs(query, liked_rows, weights, exclude_rows, 1, 32)
             return self.topk_prepared_large_k(k, excl_ptr, ne, row_filter)
 
-    def _check_large_k(self, k: int):
-        if k > self.SWEEP_CAP // 2:
-            raise ValueError(f"k={k} is too large (limit {self.SWEEP_CAP // 2})")
+    @classmethod
+    def _check_large_k(cls, k: int):
+        if k > cls.SWEEP_CAP // 2:
+            raise ValueError(f"k={k} is too large (limit {cls.SWEEP_CAP // 2})")
 
     def topk_prepared_large_k(self, k: int, excl_ptr=None, n_excl: int = 0, row_filter: Optional[RowFilter] = None):
         """Exact top-k for k > 240 (up to SWEEP_CAP / 2) for the query / profile already in this thread's scratch (qn32, qn64):
         large_k_search over count_above / sweep_above.  About 10-20 count-only passes over the catalog plus a sweep per
         call, so the batched path sends only the queries its own passes could not prove."""
         self._check_large_k(k)
-        return large_k_search(lambda thr: self.count_above(thr, excl_ptr, n_excl, row_filter),
-                              lambda thr: self.sweep_above(thr, excl_ptr, n_excl, row_filter), k, self.fast_eps)
+        return large_k_search(*self._sweeps(excl_ptr, n_excl, row_filter), k, self.fast_eps)
+
+    def _sweeps(self, excl_ptr, n_excl: int, row_filter: Optional[RowFilter]):
+        """(count, sweep) of large_k_search / close_proof over this shard, for the request staged in this thread's scratch."""
+        return (lambda thr: self.count_above(thr, excl_ptr, n_excl, row_filter),
+                lambda thr: self.sweep_above(thr, excl_ptr, n_excl, row_filter))
 
     def count_above(self, threshold: float, excl_ptr=None, n_excl: int = 0, row_filter: Optional[RowFilter] = None) -> int:
         """Number of allowed rows of this shard whose fast score >= threshold (count-only sweep; query / profile from this
@@ -587,8 +614,7 @@ class CatalogStore:
             liked = np.asarray(liked_rows, dtype=np.int32)
             nl = int(liked.shape[0])
             if nl == 0:
-                # same failure the reference hits: sklearn's check_array on an empty frame (SURVEY.md §3.2)
-                raise ValueError("Found array with 0 sample(s): user has no liked movies in the catalog")
+                raise ValueError(EMPTY_PROFILE)
         off_rp = _align(4 * d)
         off_e = off_rp + 16
         off_c = off_e + _align(4 * ne)
@@ -670,25 +696,21 @@ class CatalogStore:
 
     def topk_prepared(self, k: int, excl_ptr=None, n_excl: int = 0, row_filter: Optional[RowFilter] = None):
         """PROVEN top-k for the query / profile already in this thread's scratch (qn32, qn64): the fused launch with
-        4x more candidates until the margin clears the fp32 bound, then the exhaustive sweep; raises if neither proves
-        the ids.  Used for the queries a batched pass hands back."""
+        4x more candidates until the margin clears the fp32 bound, then the exhaustive routes of close_proof; raises if
+        none proves the ids.  Used for the queries a batched pass hands back."""
         lib = nat.load()
         s = self._scratch()
         kc = lib.rebert_candidates_for_k(k)
         if kc == 0:
             raise ValueError(f"k={k} is outside the supported range (1..240)")
-        while True:
+
+        def attempt(kc):
             self.enqueue_fused(k, kc, excl_ptr, n_excl, row_filter)
-            r, sc, margin = unpack_result(s.d_out.cpu().numpy(), k)
-            if margin > self.fast_eps or kc >= 256:
-                break
-            kc = min(256, kc * 4)
+            return unpack_result(s.d_out.cpu().numpy(), k)
+
+        r, sc, margin, _ = widen_until_proven(attempt, kc, self.fast_eps)
         if not margin > self.fast_eps:
-            res = self.sweep_above(float(sc[k - 1]) - 2.0 * self.fast_eps, excl_ptr, n_excl, row_filter) if len(r) == k else None
-            if res is None or len(res[0]) < k:
-                raise RuntimeError(f"top-{k}: the result cannot be proven exact (margin {margin:.3e} <= {self.fast_eps:.3e})")
-            order = np.lexsort((res[0], -res[1]))[:k]
-            r, sc = res[0][order], res[1][order]
+            r, sc = close_proof(r, sc, k, self.fast_eps, margin, *self._sweeps(excl_ptr, n_excl, row_filter))
         return r, sc
 
     # ------------------------------------------------------------------ batched (tensor cores) --
@@ -706,6 +728,18 @@ class CatalogStore:
             nat.check(lib.rebert_query_normalize(q.data_ptr(), b, self.d, self.ld, qn32.data_ptr(), qn64.data_ptr(),
                                                  qbf.data_ptr(), torch.cuda.current_stream().cuda_stream))
         return qn32, qn64, qbf
+
+    def prepare_batch(self, queries, liked_ptr, liked_col, liked_w, reduce_fn=None):
+        """Device (qn32, qn64, qnbf16) [b, ld] for a batch given as queries [b, d] OR a ragged CSR of liked rows (+ optional
+        weights): prepare_queries or build_profiles (reduce_fn as there)."""
+        if (queries is None) == (liked_ptr is None):
+            raise ValueError("pass exactly one of queries / liked CSR")
+        if queries is not None:
+            return self.prepare_queries(queries)
+        lp = np.asarray(liked_ptr, dtype=np.int64)
+        if np.any(np.diff(lp) == 0):
+            raise ValueError(EMPTY_PROFILE)
+        return self.build_profiles(lp, liked_col, liked_w, reduce_fn)
 
     def gemm_scores(self, qbf16: torch.Tensor, row0: int, nrows: int) -> torch.Tensor:
         """fp32 scores [b, nrows] of rows [row0, row0+nrows) on the tensor cores (bf16 catalogs; multiples of 256)."""
@@ -781,21 +815,13 @@ class CatalogStore:
         Returns rows int64 [b, k] (-1 padded), scores float64 [b, k], counts int32 [b].  Queries the batched pass could
         not prove exact (status != 0) are transparently re-run through the single-query kernel.
         """
-        if (queries is None) == (liked_ptr is None):
-            raise ValueError("pass exactly one of queries / liked CSR")
         lib = nat.load()
         long_list = k > 0 and lib.rebert_candidates_for_k(k) == 0       # k > 240: beyond the single-query kernel
         if long_list:
             self._check_large_k(k)
         dev = self.device
         with torch.cuda.device(dev):
-            if queries is not None:
-                qn32, qn64, qbf = self.prepare_queries(queries)
-            else:
-                lp = np.asarray(liked_ptr, dtype=np.int64)
-                if np.any(np.diff(lp) == 0):
-                    raise ValueError("Found array with 0 sample(s): a user has no liked movies in the catalog")
-                qn32, qn64, qbf = self.build_profiles(lp, liked_col, liked_w)
+            qn32, qn64, qbf = self.prepare_batch(queries, liked_ptr, liked_col, liked_w)
             b = qbf.shape[0]
             if prefilter and not self.batch_shadow_ok:
                 raise ValueError("prefilter=True needs enable_prefilter() and rows of whole 128-byte int8 k-blocks")
@@ -820,21 +846,8 @@ class CatalogStore:
             redo = np.nonzero(status)[0]
             if len(redo) and long_list:
                 redo = self._widened_retry(redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts)
-            if len(redo):
-                s = self._scratch()
-                ecp = None if excl_ptr is None else np.asarray(excl_ptr, dtype=np.int64)
-                for u in redo:                                   # proven single-query route for the ones the batch could not prove
-                    s.qn32.copy_(qn32[u])
-                    s.qn64.copy_(qn64[u])
-                    ptr, ne = None, 0
-                    if ecp is not None and ecp[u + 1] > ecp[u]:
-                        ptr, ne = ec.data_ptr() + 4 * int(ecp[u]), int(ecp[u + 1] - ecp[u])
-                    if long_list:
-                        r, sc = self.topk_prepared_large_k(k, ptr, ne, row_filter)
-                    else:
-                        r, sc = self.topk_prepared(k, ptr, ne, row_filter)
-                    rows[u, :], scores[u, :] = -1, -np.inf
-                    rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
+            # proven single-query route for the ones the batch could not prove
+            self._rerun_prepared(redo, qn32, qn64, excl_ptr, ec, k, row_filter, rows, scores, counts)
         if return_info:
             return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}, "int8_operands": use_shadow,
                                           "per_query": len(redo)}
@@ -890,30 +903,34 @@ class CatalogStore:
     def _recommend_batch_loop(self, qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter=None):
         """Small catalogs, catalogs neither GEMM operand type takes, and k > 2048: the batch is served one prepared query at
         a time, by the single-query kernel for k <= 240 and by topk_prepared_large_k above."""
-        lib = nat.load()
         b = qn32.shape[0]
-        kc = lib.rebert_candidates_for_k(k)
-        if kc == 0:
-            self._check_large_k(k)
         rows = np.full((b, k), -1, dtype=np.int64)
         scores = np.full((b, k), -np.inf, dtype=np.float64)
         counts = np.zeros(b, dtype=np.int32)
-        s = self._scratch()
         ecp = ec = None
         if excl_ptr is not None:
             ecp, ecol = sorted_csr(excl_ptr, excl_col)
             ec = torch.from_numpy(ecol).to(self.device)
-        for u in range(b):
-            s.qn32.copy_(qn32[u])
-            s.qn64.copy_(qn64[u])
-            ptr, ne = None, 0
-            if ecp is not None and ecp[u + 1] > ecp[u]:
-                ptr, ne = ec.data_ptr() + 4 * int(ecp[u]), int(ecp[u + 1] - ecp[u])
-            r, sc = self.topk_prepared(k, ptr, ne, row_filter) if kc else self.topk_prepared_large_k(k, ptr, ne, row_filter)
-            rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
+        self._rerun_prepared(range(b), qn32, qn64, ecp, ec, k, row_filter, rows, scores, counts)
         if return_info:
             return rows, scores, counts, {"status": np.zeros(b, dtype=np.int32), "plan": None, "per_query": b}
         return rows, scores, counts
+
+    def _rerun_prepared(self, users, qn32, qn64, excl_ptr, excl_col_dev, k, row_filter, rows, scores, counts):
+        """Proven single-query route for `users` of a prepared batch (qn32 / qn64 [b, ld]): topk_prepared, or
+        topk_prepared_large_k for k > 240, over the user's segment of the sorted exclusion CSR (host excl_ptr, device
+        excl_col_dev).  Overwrites those users' rows / scores / counts."""
+        large = nat.load().rebert_candidates_for_k(k) == 0
+        s = self._scratch()
+        for u in users:
+            s.qn32.copy_(qn32[u])
+            s.qn64.copy_(qn64[u])
+            ptr, ne = None, 0
+            if excl_ptr is not None and excl_ptr[u + 1] > excl_ptr[u]:
+                ptr, ne = excl_col_dev.data_ptr() + 4 * int(excl_ptr[u]), int(excl_ptr[u + 1] - excl_ptr[u])
+            r, sc = (self.topk_prepared_large_k if large else self.topk_prepared)(k, ptr, ne, row_filter)
+            rows[u, :], scores[u, :] = -1, -np.inf
+            rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
 
     # ------------------------------------------------------------------ diagnostics -------------
     def scores_dense(self, q32: torch.Tensor) -> torch.Tensor:

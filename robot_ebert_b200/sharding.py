@@ -21,7 +21,8 @@ import torch
 import torch.distributed as dist
 
 from . import _native as nat
-from .catalog import CatalogStore, RowFilter, large_k_search, sorted_csr, unpack_result
+from .catalog import (EMPTY_PROFILE, CatalogStore, RowFilter, close_proof, large_k_search, sorted_csr, unpack_result,
+                      validated_table, widen_until_proven)
 
 log = logging.getLogger("robot_ebert_b200")
 
@@ -277,21 +278,8 @@ class ShardedCatalog:
                   sort_ids: bool = True) -> "ShardedCatalog":
         """Every rank passes the SAME [N, D] host matrix (what Chroma's collection.get returns, constants.py:55) and keeps
         only its contiguous slice of the id-sorted rows in HBM; the id table stays whole on every rank."""
-        matrix = np.asarray(matrix, dtype=np.float32)
-        if matrix.ndim != 2:
-            raise ValueError("matrix must be [N, D]")
+        ids, matrix = validated_table(ids, matrix, sort_ids)
         n = matrix.shape[0]
-        if ids is not None:
-            if len(ids) != n:
-                raise ValueError("len(ids) != rows")
-            ids = [str(i) for i in ids]
-            if len(set(ids)) != n:
-                raise ValueError("duplicate ids")
-            if sort_ids:
-                order = sorted(range(n), key=ids.__getitem__)
-                if order != list(range(n)):
-                    matrix = matrix[np.asarray(order)]
-                    ids = [ids[i] for i in order]
         plan = ShardPlan(n, dist.get_world_size(group))
         row0, cnt = plan.range(dist.get_rank(group))
         store = CatalogStore.from_host(None, matrix[row0:row0 + cnt], dtype, device=device, row_base=row0)
@@ -384,7 +372,7 @@ class ShardedCatalog:
         if k <= 0:
             raise ValueError("k must be positive")
         if liked_rows is not None and len(liked_rows) == 0:
-            raise ValueError("Found array with 0 sample(s): user has no liked movies in the catalog")
+            raise ValueError(EMPTY_PROFILE)
         p2p = getattr(self.backend, "exchange", "nccl") == "p2p"
         if not 0 <= channel < len(self._locks):
             raise ValueError(f"channel must be in [0, {len(self._locks)})")
@@ -409,60 +397,44 @@ class ShardedCatalog:
         if p2p:
             # the whole request is ONE C call per rank (no torch ops, no NCCL): staging, profile exchange, fused scoring
             # launch with the result exchange in its tail, proof loop
-            shadow_max_k = 0
-            if self.q8_eps is not None and prefilter is not False:
-                shadow_max_k = 240 if prefilter else CatalogStore.PREFILTER_MAX_K
             rows, scores, info = self.backend.recommend_host(query, liked_rows, weights, exclude_rows, k, kc, row_filter, channel,
-                                                             shadow_max_k, self.q8_eps)
+                                                             CatalogStore.shadow_max_k(self.q8_eps is not None, prefilter),
+                                                             self.q8_eps)
             margin, proven, kc = info["margin"], info["proven_exact"], info["kc"]
         else:
-            while True:
-                partial = self.backend.stage(query, liked_rows, weights, exclude_rows, k, kc)
-                if partial is not None:
-                    dist.all_reduce(partial, op=dist.ReduceOp.SUM, group=self.group)
-                    self.backend.set_profile(partial)
-                packed = self.enqueue(k, kc, row_filter)
-                rows, scores, margin = self.backend.fetch(packed, k)
-                if margin > eps or kc >= 256:
-                    break
-                kc = min(256, kc * 4)
+            def attempt(kc):
+                self._stage(query, liked_rows, weights, exclude_rows, k, kc)
+                return self.backend.fetch(self.enqueue(k, kc, row_filter), k)
+
+            rows, scores, margin, kc = widen_until_proven(attempt, kc, eps)
             proven = margin > eps
             info = {"kc": kc, "margin": margin, "proven_exact": proven, "exact_sweep": False}
         if not proven:
-            # Fail closed (see CatalogStore._close_proof).  The margin is the same on every rank, so all ranks take this
-            # branch together and the collectives below stay aligned.
-            res = None
-            if hasattr(self.backend, "sweep_local"):
-                partial = self.backend.stage(query, liked_rows, weights, exclude_rows, k, kc)    # the sweeps read torch scratch
-                if partial is not None:
-                    dist.all_reduce(partial, op=dist.ReduceOp.SUM, group=self.group)
-                    self.backend.set_profile(partial)
-                if len(rows) == k:
-                    res = self._exact_sweep(float(scores[k - 1]) - 2.0 * eps, k, row_filter)
-                if res is None:
-                    try:
-                        res = self._recommend_large_k(query, liked_rows, weights, exclude_rows, k, row_filter, eps)
-                    except RuntimeError:
-                        res = None
-            if res is None:
-                raise RuntimeError(f"top-{k}: the sharded result cannot be proven exact (margin {margin:.3e} <= {eps:.3e})")
-            rows, scores = res
+            # Fail closed (close_proof).  The margin is the same on every rank, so all ranks take this branch together, and
+            # every branch inside it depends on all-reduced counts and all-gathered sweeps: the collectives stay aligned.
+            self._stage(query, liked_rows, weights, exclude_rows, k, kc)         # the sweeps read torch scratch
+            rows, scores = close_proof(rows, scores, k, eps, margin, *self._sweeps(row_filter))
             info = dict(info, proven_exact=True, exact_sweep=True)
         if return_info:
             return rows, scores, info
         return rows, scores
 
-    def _recommend_large_k(self, query, liked_rows, weights, exclude_rows, k, row_filter, eps):
-        """Sharded form of CatalogStore._recommend_large_k.  The bisection runs on the all-reduced count, so every rank
-        takes the same branches and the collectives stay aligned; the survivors are all-gathered and ordered alike."""
-        if liked_rows is not None and len(liked_rows) == 0:
-            raise ValueError("Found array with 0 sample(s): user has no liked movies in the catalog")
-        if k > CatalogStore.SWEEP_CAP // 2:
-            raise ValueError(f"k={k} is too large (limit {CatalogStore.SWEEP_CAP // 2})")
-        partial = self.backend.stage(query, liked_rows, weights, exclude_rows, 1, 32)
+    def _stage(self, query, liked_rows, weights, exclude_rows, k, kc):
+        """Collective: stage the request on every rank; a liked-rows profile is completed by an all-reduce of the partials."""
+        partial = self.backend.stage(query, liked_rows, weights, exclude_rows, k, kc)
         if partial is not None:
             dist.all_reduce(partial, op=dist.ReduceOp.SUM, group=self.group)
             self.backend.set_profile(partial)
+
+    def _recommend_large_k(self, query, liked_rows, weights, exclude_rows, k, row_filter, eps):
+        """Sharded form of CatalogStore._recommend_large_k: large_k_search over the whole catalog (see _sweeps)."""
+        CatalogStore._check_large_k(k)
+        self._stage(query, liked_rows, weights, exclude_rows, 1, 32)
+        return large_k_search(*self._sweeps(row_filter), k, eps)
+
+    def _sweeps(self, row_filter):
+        """(count, sweep) of large_k_search / close_proof over every shard, for the staged request: the count is all-reduced
+        and the survivors all-gathered, so every rank sees the same values, takes the same branches and orders alike."""
         dev = self.backend.device
 
         def count(thr):
@@ -470,16 +442,7 @@ class ShardedCatalog:
             dist.all_reduce(c, op=dist.ReduceOp.SUM, group=self.group)
             return int(c.item())
 
-        return large_k_search(count, lambda thr: self._sweep_gather(thr, row_filter), k, eps)
-
-    def _exact_sweep(self, threshold: float, k: int, row_filter):
-        """Sharded form of the exact fallback: local sweeps, one all-gather of the (padded) survivors, same order on every rank."""
-        res = self._sweep_gather(threshold, row_filter)
-        if res is None or len(res[0]) < k:
-            return None
-        rr, sc = res
-        order = np.lexsort((rr, -sc))[:k]
-        return rr[order], sc[order]
+        return count, lambda thr: self._sweep_gather(thr, row_filter)
 
     def _sweep_gather(self, threshold: float, row_filter):
         """(global rows, exact fp64 scores) of every allowed row of ANY shard whose fast score >= threshold, identical on
@@ -553,22 +516,40 @@ class ShardedCatalog:
                                         ctx["m_rows"].data_ptr(), ctx["m_scores"].data_ptr(), ctx["m_count"].data_ptr(),
                                         torch.cuda.current_stream().cuda_stream))
 
-    def batch_collect(self, ctx, queries, excl_ptr=None, excl_col=None):
+    def batch_collect(self, ctx, queries, excl_ptr=None, excl_col=None, *, liked_ptr=None, liked_col=None, liked_w=None,
+                      prefilter: Optional[bool] = False):
         """Second half of a batched step: read the merged results and the per-query status back, and re-run every query some
-        rank could not prove through the sharded single-query route (identical decisions on every rank).
+        rank could not prove through the sharded single-query route (identical decisions on every rank), with `prefilter`.
+        The batch is queries [b, d] or, with queries None, the liked CSR (+ optional weights) its profiles were built from.
         Returns (rows [b, k], scores [b, k], counts [b], status [b])."""
         b, k, hb = ctx["b"], ctx["k"], ctx["hb"]
         status = ctx["gathered"][:, 2 * b * k + hb:].contiguous().view(torch.int32)[:, :b].max(dim=0).values   # any rank unsure
         rows, scores = ctx["m_rows"].cpu().numpy(), ctx["m_scores"].cpu().numpy()
         counts, status = ctx["m_count"].cpu().numpy(), status.cpu().numpy()
+        self._rerun(np.nonzero(status)[0], queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, ctx.get("row_filter"),
+                    prefilter, rows, scores, counts)
+        return rows, scores, counts, status
+
+    def _rerun(self, users, queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, prefilter,
+               rows, scores, counts):
+        """Sharded single-query route (recommend) for `users` of a batch of queries or of a liked CSR with optional weights,
+        each with its segment of the exclusion CSR.  `users` must be the same on every rank (the collectives stay aligned).
+        Overwrites those users' rows / scores / counts."""
         ecp = None if excl_ptr is None else np.asarray(excl_ptr, dtype=np.int64)
         eca = None if excl_col is None else np.asarray(excl_col)
-        for u in np.nonzero(status)[0]:
+        if queries is None:
+            lpn, lcol = np.asarray(liked_ptr, dtype=np.int64), np.asarray(liked_col)
+            lw = None if liked_w is None else np.asarray(liked_w)
+        for u in users:
             ex = None if ecp is None else eca[ecp[u]:ecp[u + 1]]
-            r, sc = self.recommend(query=np.asarray(queries[u]), exclude_rows=ex, k=k, row_filter=ctx.get("row_filter"), prefilter=False)
+            if queries is not None:
+                r, sc = self.recommend(query=np.asarray(queries[u]), exclude_rows=ex, k=k, row_filter=row_filter, prefilter=prefilter)
+            else:
+                seg = slice(lpn[u], lpn[u + 1])
+                r, sc = self.recommend(liked_rows=lcol[seg], weights=None if lw is None else lw[seg], exclude_rows=ex, k=k,
+                                       row_filter=row_filter, prefilter=prefilter)
             rows[u, :], scores[u, :] = -1, -np.inf
             rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
-        return rows, scores, counts, status
 
     def recommend_batch(self, *, queries=None, liked_ptr=None, liked_col=None, liked_w=None, excl_ptr=None, excl_col=None,
                         k: int = 10, row_filter=None, return_info: bool = False):
@@ -577,18 +558,9 @@ class ShardedCatalog:
         k up to 2048 runs on the tensor cores when every shard is above the plan minimum (rebert_gemm_plan); the packed buffer
         is 2 b k + b words per rank (128 MiB at b = 4096, k = 2048).  Larger k, and smaller shards, take the per-query loop."""
         store: CatalogStore = self.backend.store
-        dev = store.device
-        if (queries is None) == (liked_ptr is None):
-            raise ValueError("pass exactly one of queries / liked CSR")
-        with torch.cuda.device(dev):
-            if queries is not None:
-                qn32, qn64, qbf = store.prepare_queries(queries)
-            else:
-                lp = np.asarray(liked_ptr, dtype=np.int64)
-                if np.any(np.diff(lp) == 0):
-                    raise ValueError("Found array with 0 sample(s): a user has no liked movies in the catalog")
-                qn32, qn64, qbf = store.build_profiles(
-                    lp, liked_col, liked_w, reduce_fn=lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group))
+        with torch.cuda.device(store.device):
+            qn32, qn64, qbf = store.prepare_batch(queries, liked_ptr, liked_col, liked_w,
+                                                  reduce_fn=lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group))
             try:
                 ctx = self.batch_context(qbf, qn64, k, excl_ptr, excl_col, row_filter, qn32=qn32)
             except nat.NativeError as e:
@@ -600,23 +572,8 @@ class ShardedCatalog:
                 return self._recommend_batch_loop(queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter,
                                                   return_info)
             self.batch_step(ctx)
-            b, hb = ctx["b"], ctx["hb"]
-            status = ctx["gathered"][:, 2 * b * k + hb:].contiguous().view(torch.int32)[:, :b].max(dim=0).values   # any rank unsure
-            rows, scores = ctx["m_rows"].cpu().numpy(), ctx["m_scores"].cpu().numpy()
-            counts, status = ctx["m_count"].cpu().numpy(), status.cpu().numpy()
-        ecp = None if excl_ptr is None else np.asarray(excl_ptr, dtype=np.int64)
-        eca = None if excl_col is None else np.asarray(excl_col)
-        for u in np.nonzero(status)[0]:                                  # identical on every rank -> collectives stay aligned
-            ex = None if ecp is None else eca[ecp[u]:ecp[u + 1]]
-            if queries is not None:
-                r, sc = self.recommend(query=np.asarray(queries[u]), exclude_rows=ex, k=k, row_filter=row_filter)
-            else:
-                lpn = np.asarray(liked_ptr, dtype=np.int64)
-                lw = None if liked_w is None else np.asarray(liked_w)[lpn[u]:lpn[u + 1]]
-                r, sc = self.recommend(liked_rows=np.asarray(liked_col)[lpn[u]:lpn[u + 1]], weights=lw, exclude_rows=ex, k=k,
-                                       row_filter=row_filter)
-            rows[u, :], scores[u, :] = -1, -np.inf
-            rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
+            rows, scores, counts, status = self.batch_collect(ctx, queries, excl_ptr, excl_col, liked_ptr=liked_ptr,
+                                                              liked_col=liked_col, liked_w=liked_w, prefilter=None)
         if return_info:
             plan = ctx["plan"]
             return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}}
@@ -628,18 +585,7 @@ class ShardedCatalog:
         rows = np.full((b, k), -1, dtype=np.int64)
         scores = np.full((b, k), -np.inf, dtype=np.float64)
         counts = np.zeros(b, dtype=np.int32)
-        ecp = None if excl_ptr is None else np.asarray(excl_ptr, dtype=np.int64)
-        eca = None if excl_col is None else np.asarray(excl_col)
-        lpn = None if liked_ptr is None else np.asarray(liked_ptr, dtype=np.int64)
-        for u in range(b):
-            ex = None if ecp is None else eca[ecp[u]:ecp[u + 1]]
-            if queries is not None:
-                r, sc = self.recommend(query=np.asarray(queries[u]), exclude_rows=ex, k=k, row_filter=row_filter)
-            else:
-                lw = None if liked_w is None else np.asarray(liked_w)[lpn[u]:lpn[u + 1]]
-                r, sc = self.recommend(liked_rows=np.asarray(liked_col)[lpn[u]:lpn[u + 1]], weights=lw, exclude_rows=ex, k=k,
-                                       row_filter=row_filter)
-            rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
+        self._rerun(range(b), queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, None, rows, scores, counts)
         if return_info:
             return rows, scores, counts, {"status": np.zeros(b, dtype=np.int32), "plan": None}
         return rows, scores, counts

@@ -469,12 +469,12 @@ def test_tiny_catalogs_vs_oracle(dtype, n, d):
         np.testing.assert_allclose(scores, want_scores, rtol=SCORE_RTOL, atol=1e-300)
 
 
-def test_unprovable_result_raises_instead_of_returning(monkeypatch):
-    """Fail closed: when neither a candidate list nor the exhaustive routes can prove the ids, recommend() raises."""
+def test_unprovable_result_raises_when_every_sweep_overflows(monkeypatch):
+    """Fail closed: when neither a candidate list nor the exhaustive routes can prove the ids, recommend() raises.  Every
+    sweep reports an overflow, so the mass-tie sweep and the bisection route both fail for real."""
     n = 3000
     m = synth.catalog_rows_f32(0, 0, n, 1, scale_rows=True)      # d = 1: every cosine is +-1, thousands of exact ties
     store = CatalogStore.from_host(None, np.repeat(m, 64, axis=1), "fp32")        # 3000 x 64, every cosine exactly +-1
-    monkeypatch.setattr(CatalogStore, "_exact_sweep", lambda self, *a, **k: None)
-    monkeypatch.setattr(CatalogStore, "_recommend_large_k", lambda self, *a, **k: (_ for _ in ()).throw(RuntimeError("sweep overflow")))
+    monkeypatch.setattr(CatalogStore, "sweep_above", lambda self, *a, **k: None)   # every sweep overflows: both exhaustive routes fail
     with pytest.raises(RuntimeError, match="cannot be proven exact"):
         store.recommend(query=np.ones(64, dtype=np.float32), k=10)
