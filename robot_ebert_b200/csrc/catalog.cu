@@ -6,8 +6,6 @@
 #include <mutex>
 #include <unordered_set>
 
-#include <stdlib.h>
-
 #include "exchange.cuh"
 #include "request.cuh"
 
@@ -48,10 +46,6 @@ int raise_smem_limit_impl(const void* kern) {
     REBERT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, max_optin_smem() - (int)a.sharedSizeBytes));
     done.insert(kern);
     return REBERT_OK;
-}
-bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("REBERT_PDL"); return !(e && e[0] == '0'); }();
-    return on;
 }
 int num_sms() {
     static int cached = 0;

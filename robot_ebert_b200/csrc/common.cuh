@@ -32,10 +32,9 @@ int max_optin_smem();
 // memory), once per kernel.  Always the same constant, so concurrent callers cannot race each other's launches.
 int raise_smem_limit_impl(const void* kern);
 template <typename K> static inline int raise_smem_limit(K kern) { return raise_smem_limit_impl((const void*)kern); }
-bool pdl_enabled();
 // host_api.cu -> catalog.cu / finalize.cu (internal launchers)
 int stage_query_launch(const float* q_host, int d, int ld, float* qn32, double* qn64, const int32_t* excl_host, int n_excl,
-                       int32_t* excl_dev, cudaStream_t st);   // REBERT_PDL=0 switches programmatic dependent launch off (read once)
+                       int32_t* excl_dev, cudaStream_t st);   // launched with programmatic dependent launch, like every kernel of a request
 
 // ---------------------------------------------------------------- layout --------------------
 // A stored row is LANES * CPL chunks of 16 bytes: LANES lanes of a warp each own CPL chunks.
@@ -254,7 +253,7 @@ static inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 blo
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 #endif

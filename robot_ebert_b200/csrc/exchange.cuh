@@ -186,7 +186,6 @@ struct GemvFused {
 struct Published {
     PublishedKeys keys;
     unsigned* ctl;             // 32 control words (ticket, hint, tile claims, compaction cursors): the cluster kernel leaves them zero
-    unsigned long long* trace; // tuning only
 };
 int finalize_published_launch(const Published& pub, const GemvFused& f, int64_t row_base, cudaStream_t st);
 int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_filter_t* filter, int32_t kc, void* workspace,

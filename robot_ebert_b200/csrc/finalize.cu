@@ -189,7 +189,6 @@ struct FinalizeParams {
     int64_t row_base, x_n;
     int k, cap;
     int stage_words;           // words from fk on that are free until the winners are known: max(3 kc, heads of every list)
-    int split_select;          // 0: every CTA selects on its own; 1 / 2: selection spread over the cluster (24 / 4 key loads in flight)
     unsigned long long* out_packed;
     uint32_t tag;
     uint32_t* done_flag;       // pinned host word the host polls instead of synchronising the stream (or nullptr)
@@ -197,19 +196,10 @@ struct FinalizeParams {
     Exchange xchg;
 };
 
-__device__ __forceinline__ unsigned long long ftimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define FIN_TRACE(slot) do { if (p.pub.trace && threadIdx.x == 0 && crank == 0) p.pub.trace[(slot)] = ftimer_ns(); } while (0)
-
-// SPLIT: winner selection spread over the cluster (long candidate lists); XCHG: row shard, NVLink exchange + merge at the end.
+// SPLIT: winner selection spread over the cluster (kc >= 128, long candidate lists); XCHG: row shard, NVLink exchange + merge at the end.
 // Eight instantiations (with the element type) instead of run-time branches: this kernel runs once per request with a cold instruction cache, and
 // every variant it does not need (each one thousands of unrolled instructions) would sit between the ones it does.
 // T: element type of the catalog of record — the exact pass carries one row function instead of both.
-// SPLIT: 0 = every CTA selects on its own, 1 = cluster-wide with 24 key loads in flight per thread (kc >= 128), 2 = cluster-wide
-// with 4 in flight (kc <= 64: a CTA's two regions hold <= 5 keys per thread; a sixth of the unrolled code).
 template <int SPLIT, bool XCHG, typename T>
 __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_kernel(const FinalizeParams p) {
     extern __shared__ __align__(16) unsigned char fsm[];
@@ -228,7 +218,6 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
     cg::cluster_group cluster = cg::this_cluster();
     const int crank = (int)cluster.block_rank();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = kFinalClusterThreads / 32;
-    FIN_TRACE(0);
     // Programmatic dependent launch lets the NEXT kernel of the stream place its CTAs early.  A kernel that will wait for
     // a PEER must not do that before the wait is over: the next request's streaming CTAs would sit resident on every SM,
     // blocked behind this kernel, while the peer — in the mirrored state on another channel — needs exactly those SMs to
@@ -242,7 +231,6 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
     pdl_wait();                                      // the keys come from the streaming kernel launched just before
     // (Waiting on the CTAs' publish counter instead would start 1-3 us earlier, but a cluster placed early by programmatic
     // launch could then mistake the PREVIOUS request's count for its own; stream order is the simple, safe hand-off.)
-    FIN_TRACE(1);
     constexpr int epc = ChunkDot<T>::EPC;
     // the fp64 query: its loads are issued here, ahead of the ones select_winners issues, and consumed only afterwards —
     // one L2 round trip for everything this kernel reads before the candidate rows
@@ -253,13 +241,10 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
         const int i = threadIdx.x + j * kFinalClusterThreads;
         qv[j] = i < p.x_ld ? __ldg(p.q64 + i) : 0.0;
     }
-    if (SPLIT == 2)
-        select_winners_cluster<4, kFinalCluster, kFinalClusterThreads>(cluster, p.pub.keys, p.cap, buf, fk, p.stage_words, fk, &s_total,
-                                                                       (p.pub.trace && crank == 0) ? p.pub.trace + 8 : nullptr);
-    else if (SPLIT == 1)     // fk | s_score | s_row = 3 kc words that are free until the winners are known
-        select_winners_cluster<24, kFinalCluster, kFinalClusterThreads>(cluster, p.pub.keys, p.cap, buf, fk, p.stage_words, fk, &s_total, (p.pub.trace && crank == 0) ? p.pub.trace + 8 : nullptr);
+    if (SPLIT)     // fk | s_score | s_row = 3 kc words that are free until the winners are known
+        select_winners_cluster<kFinalCluster, kFinalClusterThreads>(cluster, p.pub.keys, p.cap, buf, fk, p.stage_words, fk, &s_total);
     else
-        select_winners<24, kFinalClusterThreads>(p.pub.keys, p.cap, buf, fk, (p.pub.trace && crank == 0) ? p.pub.trace + 8 : nullptr);
+        select_winners<24, kFinalClusterThreads>(p.pub.keys, p.cap, buf, fk);
     {
         const int chunks = p.x_ld / epc;
 #pragma unroll
@@ -276,7 +261,6 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
         }
     }
     __syncthreads();
-    FIN_TRACE(2);
     double* r_score = cluster.map_shared_rank(s_score, 0);
     int64_t* r_row = cluster.map_shared_rank(s_row, 0);
     unsigned long long* r_werr = cluster.map_shared_rank(s_werr, 0);
@@ -296,10 +280,8 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
         if (lane == 0) { r_score[c] = sc; r_row[c] = gr; }
     }
     if (lane == 0) r_werr[crank * nwarps + warp] = (unsigned long long)__double_as_longlong(werr);
-    FIN_TRACE(7);
     cluster.sync();                                  // all scores have landed in CTA 0
     if (crank != 0) return;
-    FIN_TRACE(3);
     unsigned long long me = 0;                       // bits of non-negative doubles: integer order == numeric order
     for (int i = lane; i < kFinalCluster * nwarps; i += 32) me = s_werr[i] > me ? s_werr[i] : me;
 #pragma unroll
@@ -309,7 +291,6 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
     rank_candidates<false>(s_score, s_row, kc, k, last != 0, last ? (double)key_score(last) : 0.0, __longlong_as_double((long long)me),
                            (int64_t*)blk, (double*)(blk + k), (int32_t*)(blk + 2 * k), (double*)(blk + 2 * k + 1), s_tmp, &s_kth);
     if (threadIdx.x == 0) ((uint32_t*)(blk + 2 * k))[1] = p.tag;
-    FIN_TRACE(4);
     if (exchange) {
         __syncthreads();
         exchange_results(p.xchg, k, s_block, p.out_packed, s_all);
@@ -323,7 +304,13 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
             *(volatile uint32_t*)p.done_flag = p.done_token;
         }
     }
-    FIN_TRACE(5);
+}
+
+using PublishedKernel = void (*)(const FinalizeParams);
+template <typename T>
+static PublishedKernel published_kernel(bool split, bool xchg) {
+    return split ? (xchg ? finalize_published_kernel<1, true, T> : finalize_published_kernel<1, false, T>)
+                 : (xchg ? finalize_published_kernel<0, true, T> : finalize_published_kernel<0, false, T>);
 }
 
 int finalize_published_launch(const Published& pub, const GemvFused& f, int64_t row_base, cudaStream_t st) {
@@ -344,14 +331,8 @@ int finalize_published_launch(const Published& pub, const GemvFused& f, int64_t 
     p.cap = cap;
     // Long candidate lists (kc >= 128: k > 16, the int8 shadow, a widened retry) publish tens of thousands of keys: the cluster
     // shares the scan and the ordering (merge.cuh).  Short lists fit one round of loads per CTA and skip the two extra
-    // cluster barriers.  REBERT_FIN_SPLIT=0/1 forces either way (tools).
-    {
-        static const int forced = [] { const char* e = getenv("REBERT_FIN_SPLIT"); return e ? (e[0] == '0' ? 0 : 1) : -1; }();
-        static const bool tuning = getenv("REBERT_GEMV_TUNE") != nullptr;      // read once: getenv is a linear scan, this is the request path
-        int want = forced;
-        if (tuning) { const char* e = getenv("REBERT_FIN_SPLIT"); want = e ? (e[0] == '0' ? 0 : 1) : -1; }
-        p.split_select = (want < 0 ? pub.keys.kc >= 128 : want == 1) ? (pub.keys.kc >= 128 ? 1 : 2) : 0;
-    }
+    // cluster barriers.
+    const bool split = pub.keys.kc >= 128;
     p.stage_words = 3 * pub.keys.kc > pub.keys.kc + pub.keys.lists ? 3 * pub.keys.kc : pub.keys.kc + pub.keys.lists;
     p.out_packed = f.out_packed;
     p.tag = f.tag;
@@ -361,14 +342,8 @@ int finalize_published_launch(const Published& pub, const GemvFused& f, int64_t 
     const size_t smem = (size_t)p.x_ld * 8 + (size_t)cap * 8 + (size_t)p.stage_words * 8 + (size_t)kFinalCluster * (kFinalClusterThreads / 32) * 8 +
                         (size_t)(2 * f.k + 2) * 8 * (1 + (f.xchg ? f.xchg->world : 0));
     const bool xchg = p.xchg.world > 1;
-    void (*kern)(const FinalizeParams) = nullptr;
-#define REBERT_FIN_PICK(TT)                                                                                                         \
-    kern = p.split_select == 2 ? (xchg ? finalize_published_kernel<2, true, TT> : finalize_published_kernel<2, false, TT>)           \
-         : p.split_select == 1 ? (xchg ? finalize_published_kernel<1, true, TT> : finalize_published_kernel<1, false, TT>)           \
-                               : (xchg ? finalize_published_kernel<0, true, TT> : finalize_published_kernel<0, false, TT>)
-    if (p.x_dtype == REBERT_F32) REBERT_FIN_PICK(float);
-    else REBERT_FIN_PICK(__nv_bfloat16);
-#undef REBERT_FIN_PICK
+    const PublishedKernel kern =
+        p.x_dtype == REBERT_F32 ? published_kernel<float>(split, xchg) : published_kernel<__nv_bfloat16>(split, xchg);
     { int rc = raise_smem_limit(kern); if (rc != REBERT_OK) return rc; }
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
@@ -384,7 +359,7 @@ int finalize_published_launch(const Published& pub, const GemvFused& f, int64_t 
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    cfg.numAttrs = 2;
     REBERT_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
     REBERT_CUDA(cudaGetLastError());
     return REBERT_OK;

@@ -31,7 +31,6 @@
 //   once) and Q (12.6 MB at B = 4096) stays L2-resident (evict_last).
 //   Measured (profiles/r01_gemm2_filter_1M_ncu_summary.md): tensor pipe 97 % active, 1607 TFLOP/s.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -929,7 +928,7 @@ static void set_pred(GemmParams& p, const rebert_catalog_t* cat, const rebert_fi
 // [b, ld8] and p.qscale holds the queries' dequantisation steps).
 template <int MODE, bool I8>
 static int launch_gemm_t(const rebert_catalog_t* cat, const void* qmat, GemmParams& p, cudaStream_t st) {
-    const bool pair = p.b > BM && getenv("REBERT_GEMM_1CTA") == nullptr;   // cta_group::2 needs >= 2 query tiles to pay off
+    const bool pair = p.b > BM;   // cta_group::2 needs >= 2 query tiles to pay off
     CUtensorMap map_q, map_rows;
     int rc = make_tmap(&map_q, qmat, p.b, cat->ld, BM, I8);
     if (rc != REBERT_OK) return rc;

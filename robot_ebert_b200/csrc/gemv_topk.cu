@@ -23,8 +23,6 @@
 //   * launched with programmatic stream serialization: no access to memory an earlier kernel of the stream writes before
 //     griddepcontrol.wait.  The catalog is immutable, so the producer starts streaming the first tiles BEFORE that wait:
 //     the first TMA round trip overlaps the previous kernel's tail (query staging / the previous request's merge).
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "exchange.cuh"
@@ -34,7 +32,8 @@ namespace rebert {
 constexpr int kConsumerWarps = 8;
 constexpr int kThreads = (kConsumerWarps + 1) * 32;
 constexpr int kStageBytes = 48 * 1024;
-constexpr int kMaxStages = 8;
+constexpr int kStages = 4;           // pipeline depth (lowered when shared memory is short); 48 KB x 4 is within 0.3 % of the best
+constexpr int kDynTailPct = 12;      // share of the tiles claimed dynamically at the end (balances SMs of unequal speed)
 constexpr int kMaxExclSmem = 4096;   // exclusion rows staged in shared memory (larger lists are searched in global memory)
 
 struct GemvParams {
@@ -49,7 +48,6 @@ struct GemvParams {
     int          tile_rows;
     int          stages;
     int          kc;
-    int          l2_policy; // 0 = evict_first (default), 1 = evict_normal, 2 = evict_last  (tuning knob)
     DevFilter    filter;
     uint64_t*    pub_keys;  // [kPubRegions][region_cap] kept keys of all CTAs: CTA b compacts into region b % kPubRegions
     uint64_t*    pub_heads; // [grid, pub_P] the pub_P = ceil(kc / grid) best keys of every CTA (zero padded)
@@ -61,10 +59,6 @@ struct GemvParams {
     unsigned*    ghint;     // grid-wide threshold hint, orderable fp32 bits (zero before launch; reset with the counter)
     unsigned*    tile_ctr;  // tail tiles claimed so far (zero before launch; reset with the counter)
     int64_t      static_rounds;  // every CTA takes tiles blockIdx.x + i * grid for i < static_rounds, the rest are claimed
-    unsigned long long* trace;  // tuning only (REBERT_GEMV_TRACE): [grid + 1][8] %globaltimer stamps, or nullptr
-    int          cta_hint;  // 1 = CTA-level quantile hint from the warps' (kc/8)-th best keys (default; 0 is a tuning knob)
-    int          merge_prune; // 1 = the CTA merge drops keys below the threshold hints (default; 0 is a tuning knob)
-    int          early_tma; // 1 = first tiles are requested before griddepcontrol.wait (default; 0 is a tuning knob)
     int          merge_cap; // keys the final merge may hold in shared memory (power of two)
     int          publish_only;  // request path: no ticket, no merge here — the cluster kernel behind this launch takes over
 };
@@ -143,10 +137,9 @@ struct WarpTopK {
 //   * the CTA-wide quantile bound: min over the 8 warps of their (kc/8)-th best score (kc rows of this CTA reach it).
 // s_wq entries only grow, so a stale read only yields a smaller, still valid bound.
 template <int QLANE>
-__device__ __forceinline__ void publish_hints(uint64_t key0, float thr, int warp, int lane, int cta_hint, unsigned* s_hint,
-                                              unsigned* s_wq) {
+__device__ __forceinline__ void publish_hints(uint64_t key0, float thr, int warp, int lane, unsigned* s_hint, unsigned* s_wq) {
     if (lane == 0 && thr > -INFINITY) atomicMax(s_hint, f32_orderable(thr));
-    if (cta_hint && lane == QLANE && key0 != 0) {
+    if (lane == QLANE && key0 != 0) {
         const unsigned mine = (unsigned)(key0 >> 32);
         ((volatile unsigned*)s_wq)[warp] = mine;
         unsigned mn = mine;
@@ -155,13 +148,6 @@ __device__ __forceinline__ void publish_hints(uint64_t key0, float thr, int warp
         if (mn) atomicMax(s_hint, mn);
     }
 }
-
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define REBERT_TRACE(slot) do { if (p.trace && threadIdx.x == 0) p.trace[(size_t)blockIdx.x * 8 + (slot)] = globaltimer_ns(); } while (0)
 
 template <typename T, int CPL, int LANES, int M>
 __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams p) {
@@ -180,16 +166,15 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     const int stage_stride = tile_bytes + ((inv_bytes + 127) & ~127);
     unsigned char* stage_base = smem;
     uint64_t* full_bar = (uint64_t*)(smem + (size_t)p.stages * stage_stride);
-    uint64_t* empty_bar = full_bar + kMaxStages;
-    float* q_smem = (float*)(empty_bar + kMaxStages);            // generic kernel only: [ld]
+    uint64_t* empty_bar = full_bar + kStages;
+    float* q_smem = (float*)(empty_bar + kStages);               // generic kernel only: [ld]
     int32_t* excl_smem = (int32_t*)(q_smem + (kRegQ ? 0 : p.ld));
     const bool excl_staged = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem;
     const int32_t* excl_s = excl_staged ? excl_smem : nullptr;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    REBERT_TRACE(0);                                   // kernel entry
 
-    __shared__ int s_tile[kMaxStages];          // tile held by each stage, written by the producer before it arms the barrier
+    __shared__ int s_tile[kStages];             // tile held by each stage, written by the producer before it arms the barrier
     if (threadIdx.x == 0) {
         for (int s = 0; s < p.stages; ++s) {
             mbar_init(&full_bar[s], 1);
@@ -219,8 +204,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         bulk_g2s(dst, (const unsigned char*)p.rows + row0 * row_bytes_e, bytes, &full_bar[s], policy);
         if (ibytes) bulk_g2s(dst + tile_bytes, p.inv_norm + row0, ibytes, &full_bar[s], policy);
     };
-    if (warp == kConsumerWarps && lane == 0 && p.early_tma) {
-        const uint64_t policy = p.l2_policy == 0 ? l2_policy_evict_first() : (p.l2_policy == 2 ? l2_policy_evict_last() : l2_policy_evict_normal());
+    if (warp == kConsumerWarps && lane == 0) {
+        const uint64_t policy = l2_policy_evict_first();
         for (; early < p.stages && early < p.static_rounds; ++early) {
             const int64_t t = blockIdx.x + early * (int64_t)gridDim.x;
             if (t >= p.num_tiles) break;
@@ -257,12 +242,11 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     if (threadIdx.x == 0) s_hint = 0u;
     if (threadIdx.x < kConsumerWarps) s_wq[threadIdx.x] = 0u;
     __syncthreads();
-    REBERT_TRACE(1);                                   // prologue done
 
     if (warp == kConsumerWarps) {
         // ===================== producer warp: one elected lane issues the bulk copies =====================
         if (lane == 0) {
-            const uint64_t policy = p.l2_policy == 0 ? l2_policy_evict_first() : (p.l2_policy == 2 ? l2_policy_evict_last() : l2_policy_evict_normal());
+            const uint64_t policy = l2_policy_evict_first();
             // SMs do not stream at the same speed (measured: equal shares finish up to 10 % apart), so only the first
             // `static_rounds` rounds are dealt out statically (tile = blockIdx.x + i * grid); the tail tiles are claimed
             // one by one from a grid-wide counter.  Four claims are kept in flight — the first four issued right here —
@@ -362,7 +346,6 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
             const float hint = hb ? orderable_f32(hb) : -INFINITY;
 
             mbar_wait(&full_bar[s], round & 1u);
-            if (it == 0) REBERT_TRACE(2);              // first tile landed
             const int64_t t = s_tile[s];               // which tile the producer put into this stage (-1: none left)
             if (t < 0) break;
             const int64_t row0 = t * p.tile_rows;
@@ -412,7 +395,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                             const uint32_t lr = (uint32_t)(row0 + base + u * kConsumerWarps * RPW + src / LANES);
                             if (sc > top.thr && row_allowed(p.filter, lr, excl_s)) {
                                 top.insert(make_key(sc, lr), lane);
-                                publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, p.cta_hint, &s_hint, s_wq);
+                                publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
                             }
                         }
                     }
@@ -474,7 +457,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                     REBERT_ASSERT((int64_t)lr < p.n);
                     if (sc > top.thr && row_allowed(p.filter, lr, excl_s)) {
                         top.insert(make_key(sc, lr), lane);
-                        publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, p.cta_hint, &s_hint, s_wq);
+                        publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
                     }
                 }
                 unsigned mb = __ballot_sync(0xffffffffu, vB && cl == 0 && sb > top.thr && sb >= hint);
@@ -485,7 +468,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                     const uint32_t lr = (uint32_t)(row0 + base + kConsumerWarps * RPW + src / LANES);
                     if (sc > top.thr && row_allowed(p.filter, lr, excl_s)) {
                         top.insert(make_key(sc, lr), lane);
-                        publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, p.cta_hint, &s_hint, s_wq);
+                        publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
                     }
                 }
             }
@@ -495,9 +478,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     }
 
     // ===================== CTA merge: 8 sorted warp lists -> one sorted list of kc keys =====================
-    if (warp == 0) REBERT_TRACE(3);                    // warp 0 finished its last tile
     __syncthreads();   // every stage has been consumed; the pipeline memory is free to reuse
-    REBERT_TRACE(4);                                   // all warps finished
     uint64_t* lists = (uint64_t*)smem;           // [kConsumerWarps][kc]
     const int kc = p.kc;
     __shared__ int s_kept[kConsumerWarps];       // entries of each warp list that can still matter
@@ -505,7 +486,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         // Keys scoring below the best lower bound of the global kc-th best (CTA hint, or the grid-wide word) cannot be in
         // the result: drop them here, so only ~kc of the CTA's 8 kc keys go through the rank merge and reach the final
         // merge.  The lists are sorted, so the dropped keys are a tail and the zero-terminated-list convention holds.
-        const unsigned hb = p.merge_prune ? max(*(volatile unsigned*)&s_hint, __ldcg(p.ghint)) : 0u;
+        const unsigned hb = max(*(volatile unsigned*)&s_hint, __ldcg(p.ghint));
         int kept = 0;
 #pragma unroll
         for (int m = 0; m < M; ++m) {
@@ -549,7 +530,6 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         for (int j = threadIdx.x; j < p.pub_P; j += blockDim.x) p.pub_heads[(size_t)blockIdx.x * p.pub_P + j] = j < kc ? merged[j] : 0;
         if (threadIdx.x == 0) p.pub_tails[blockIdx.x] = nkeep == kc ? merged[kc - 1] : 0;
     }
-    REBERT_TRACE(5);                                   // CTA keys published
     if (p.publish_only) return;                        // request path: the cluster kernel behind this launch merges
 
     // ===================== rebert_gemv_topk: the last CTA to finish merges what all CTAs kept (no second launch) =========
@@ -567,55 +547,22 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         select_winners<16>(pub, p.merge_cap, (uint64_t*)smem, p.cand_keys);
         __syncthreads();
     }
-    if (p.trace && threadIdx.x == 0) { p.trace[(size_t)gridDim.x * 8] = globaltimer_ns(); p.trace[(size_t)gridDim.x * 8 + 1] = blockIdx.x; }
     if (threadIdx.x < 32) p.counter[threadIdx.x] = 0u;       // ticket, hint, tile-claim counter, compaction cursors
 }
 
 // ---------------------------------------------------------------- host side ----------------------------------
-// Tuning knobs (tools/tune_gemv.py, tools/probe_knobs.py, tools/trace_gemv.py).  The environment is read ONCE, at the
-// first launch — getenv is a linear scan and this sits on the per-request path — unless REBERT_GEMV_TUNE is set at that
-// moment, in which case every launch re-reads it (what the tools do to sweep values inside one process).
-struct GemvKnobs {
-    int stage_bytes = kStageBytes;
-    int stages = 4;
-    int l2_policy = 0;
-    int cta_hint = 1;
-    int dyn_pct = 12;          // share of the tiles claimed dynamically at the end; 0 = all static
-    int merge_prune = 1;       // CTA merge drops keys below the threshold hints
-    int early_tma = 1;         // first tiles requested before griddepcontrol.wait
-    unsigned long long* trace = nullptr;
-    unsigned long long* fin_trace = nullptr;   // phase stamps of the request path's cluster kernel
-};
-static GemvKnobs read_knobs() {
-    GemvKnobs k;
-    if (const char* e = getenv("REBERT_GEMV_STAGE_BYTES")) { int v = atoi(e); if (v >= 4096 && v <= 96 * 1024) k.stage_bytes = v; }
-    if (const char* e = getenv("REBERT_GEMV_STAGES")) { int v = atoi(e); if (v >= 1 && v <= kMaxStages) k.stages = v; }
-    if (const char* e = getenv("REBERT_GEMV_L2_POLICY")) k.l2_policy = atoi(e);
-    if (const char* e = getenv("REBERT_GEMV_CTA_HINT")) k.cta_hint = atoi(e) != 0;
-    if (const char* e = getenv("REBERT_GEMV_DYN_PCT")) { int v = atoi(e); if (v >= 0 && v <= 100) k.dyn_pct = v; }
-    if (const char* e = getenv("REBERT_GEMV_MERGE_PRUNE")) k.merge_prune = atoi(e) != 0;
-    if (const char* e = getenv("REBERT_GEMV_EARLY_TMA")) k.early_tma = atoi(e) != 0;
-    if (const char* e = getenv("REBERT_FIN_TRACE")) k.fin_trace = (unsigned long long*)strtoull(e, nullptr, 0);
-    if (const char* e = getenv("REBERT_GEMV_TRACE")) k.trace = (unsigned long long*)strtoull(e, nullptr, 0);
-    return k;
-}
-static GemvKnobs gemv_knobs() {
-    static const bool tuning = getenv("REBERT_GEMV_TUNE") != nullptr;
-    static const GemvKnobs cached = read_knobs();
-    return tuning ? read_knobs() : cached;
-}
-
+// The pipeline shape, the L2 policy, the dynamic tail share, the CTA-wide hint, merge pruning and the early TMA issue are
+// fixed: each is the setting measured fastest on the B200 (DESIGN.md §4.1, "Tuning record").
 struct GemvLaunch {
     int grid, stages, tile_rows, merge_cap;
     size_t smem;
 };
 
-static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, bool generic, int n_exclude, const GemvKnobs& knobs) {
+static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, bool generic, int n_exclude) {
     GemvLaunch g;
     const int row_bytes = L.ld * L.esize;
     const int rpw = 32 / L.lanes;
-    const int stage_bytes = knobs.stage_bytes;
-    int tr = stage_bytes / row_bytes;
+    int tr = kStageBytes / row_bytes;
     const int unit = kConsumerWarps * rpw;           // rows one step of all warps covers
     if (tr >= 2 * unit) tr = (tr / (2 * unit)) * (2 * unit);
     else if (tr >= unit) tr = unit;
@@ -628,8 +575,8 @@ static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, bool generic,
     const int tile_bytes = tr * row_bytes;
     const int stage_stride = tile_bytes + ((tr * 4 + 127) & ~127);
     const size_t excl_bytes = (n_exclude > 0 && n_exclude <= kMaxExclSmem) ? (size_t)n_exclude * 4 : 0;
-    const size_t fixed = 2 * kMaxStages * sizeof(uint64_t) + (generic ? (size_t)L.ld * 4 : 0) + excl_bytes + 128;
-    int stages = knobs.stages;
+    const size_t fixed = 2 * kStages * sizeof(uint64_t) + (generic ? (size_t)L.ld * 4 : 0) + excl_bytes + 128;
+    int stages = kStages;
     while (stages > 1 && (size_t)stages * stage_stride + fixed > 220 * 1024) --stages;
     g.stages = stages;
     g.smem = (size_t)stages * stage_stride + fixed;
@@ -801,8 +748,7 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
     }
     const bool generic = use_generic(L);
     const int n_excl = (filter && filter->exclude_rows && filter->n_exclude > 0) ? filter->n_exclude : 0;
-    const GemvKnobs knobs = gemv_knobs();
-    GemvLaunch g = plan_gemv(L, cat->n, kc, generic, n_excl, knobs);
+    GemvLaunch g = plan_gemv(L, cat->n, kc, generic, n_excl);
     GemvParams p;
     memset(&p, 0, sizeof(p));
     p.rows = cat->rows;
@@ -816,7 +762,6 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
     p.num_tiles = (cat->n + g.tile_rows - 1) / g.tile_rows;
     p.stages = g.stages;
     p.kc = kc;
-    p.l2_policy = knobs.l2_policy;
     p.filter = make_filter(filter, cat->row_base);
     unsigned char* ws = (unsigned char*)(((uintptr_t)workspace + 127) & ~(uintptr_t)127);
     p.counter = (unsigned*)ws;
@@ -829,21 +774,15 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
     p.pub_heads = p.pub_keys + (size_t)kPubRegions * p.region_cap;
     p.pub_P = (kc + g.grid - 1) / g.grid;
     {
-        // share of the tiles claimed dynamically at the end (balances SMs of unequal speed); 0 = all static
-        const int dyn_pct = knobs.dyn_pct;
         const int64_t rounds = (p.num_tiles + g.grid - 1) / g.grid;       // static schedule would need this many
-        int64_t sr = rounds - (rounds * dyn_pct + 99) / 100;
+        int64_t sr = rounds - (rounds * kDynTailPct + 99) / 100;
         // Each CTA keeps four claims in flight from its first instruction on, so a dynamic tail shorter than a few rounds is
         // swallowed by the CTAs that start first (2264 x 1536: 34 CTAs took all 136 tail tiles and finished 5 us after the
         // rest).  Short launches are dealt out statically.
-        if (dyn_pct == 0 || rounds - sr < 8) sr = rounds;
+        if (rounds - sr < 8) sr = rounds;
         if (sr < 1) sr = 1;                                               // the first tile is always blockIdx.x
         p.static_rounds = sr;
     }
-    p.trace = knobs.trace;
-    p.cta_hint = knobs.cta_hint;
-    p.merge_prune = knobs.merge_prune;
-    p.early_tma = knobs.early_tma;
     p.cand_keys = cand_keys;
     p.merge_cap = g.merge_cap;
     p.publish_only = fused ? 1 : 0;
@@ -864,7 +803,6 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
     pub.keys.kc = kc;
     pub.keys.region_cap = p.region_cap;
     pub.ctl = p.counter;
-    pub.trace = knobs.fin_trace;
     return finalize_published_launch(pub, *fused, cat->row_base, st);
 }
 

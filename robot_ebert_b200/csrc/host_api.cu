@@ -7,8 +7,6 @@
 // shadow first when the caller has one, then the plain fast pass with 4x more candidates until the margin proves the ids.
 // Scratch (pinned host + device) is provided by the caller, so the library still allocates nothing and concurrent
 // callers only need their own scratch + stream (+ their own exchange channel on a row shard).
-#include <stdlib.h>
-
 #include <algorithm>
 #include <chrono>
 
@@ -17,15 +15,9 @@
 namespace rebert {
 
 // The result block lives in pinned host memory and the exact-pass kernel stores a completion token behind it, so the host
-// can wait by polling that word instead of synchronising the stream (saves the driver's completion path, a few us per
-// request).  REBERT_HOST_POLL=0 switches back to cudaStreamSynchronize.  Read once.
-static bool host_poll_enabled() {
-    static const bool on = [] { const char* e = getenv("REBERT_HOST_POLL"); return !(e && e[0] == '0'); }();
-    return on;
-}
-
-// true when *flag == token arrived; false after ~20 s (a faulted kernel or a dead peer: the caller then synchronises the
-// stream, which reports the error)
+// waits by polling that word instead of synchronising the stream (saves the driver's completion path, a few us per
+// request).  true when *flag == token arrived; false after ~20 s (a faulted kernel or a dead peer: the caller then
+// synchronises the stream, which reports the error)
 static bool poll_done(const volatile uint32_t* flag, uint32_t token) {
     for (int spin = 0; spin < 4096; ++spin) {
         if (*flag == token) return true;
@@ -238,17 +230,12 @@ REBERT_API int rebert_recommend_host(const rebert_catalog_t* cat, const float* q
         gf.out_packed = res;
         gf.tag = tag;
         gf.xchg = nullptr;
-        gf.done_flag = nullptr;
-        gf.done_token = 0;
-        const bool poll = host_poll_enabled();
-        if (poll) {
-            uint32_t token = *token_ctr + 1u;
-            if (token == 0u) token = 1u;
-            *token_ctr = token;
-            *done_flag = 0u;
-            gf.done_flag = (uint32_t*)done_flag;
-            gf.done_token = token;
-        }
+        uint32_t token = *token_ctr + 1u;
+        if (token == 0u) token = 1u;
+        *token_ctr = token;
+        *done_flag = 0u;
+        gf.done_flag = (uint32_t*)done_flag;
+        gf.done_token = token;
         if (sharded) {
             x.seq = seq ? seq : 1u;
             gf.xchg = &x;
@@ -258,7 +245,7 @@ REBERT_API int rebert_recommend_host(const rebert_catalog_t* cat, const float* q
         if (rc != REBERT_OK) return rc;
         const double t_enq = now_us();
         inf.host_enqueue_us += t_enq - t_mark;
-        if (!poll || !poll_done(done_flag, gf.done_token)) REBERT_CUDA(cudaStreamSynchronize(st));
+        if (!poll_done(done_flag, token)) REBERT_CUDA(cudaStreamSynchronize(st));
         t_mark = now_us();
         inf.host_wait_us += t_mark - t_enq;
         ++inf.attempts;

@@ -48,12 +48,6 @@ struct PublishedKeys {
 //   T1 = kc-th largest key among the first P keys of every list
 // and the few survivors are ordered by rank counting (one pass, no barriers) or, beyond 512 of them, a bitonic sort.
 // buf: `cap` keys of scratch (power of two >= max(2 kc, kc + lists)); all threads call.
-__device__ __forceinline__ unsigned long long merge_timer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define MERGE_TRACE(slot) do { if (tr && threadIdx.x == 0) tr[(slot)] = merge_timer_ns(); } while (0)
 
 // Mass ties (more keys within the threshold than any buffer holds): merge everything that was published, region by region,
 // into the running best kc.  Correct for any input, slow.  rtot: keys per region (shared memory); all threads call.
@@ -97,7 +91,7 @@ static __device__ void sort_survivors(uint64_t* buf, int cnt, int kc, uint64_t* 
 // THREADS: the block size when the caller knows it at compile time (the slot arithmetic below then folds into shifts and masks —
 // a third of this function's instructions otherwise), 0 = read blockDim.x.
 template <int INFLIGHT, int THREADS = 0>
-__device__ inline void select_winners(const PublishedKeys& pub, int cap, uint64_t* buf, uint64_t* out, unsigned long long* tr = nullptr) {
+__device__ inline void select_winners(const PublishedKeys& pub, int cap, uint64_t* buf, uint64_t* out) {
     __shared__ unsigned long long s_t0, s_t1;
     __shared__ int s_cnt;
     __shared__ unsigned s_rtot[kPubRegions];
@@ -132,7 +126,6 @@ __device__ inline void select_winners(const PublishedKeys& pub, int cap, uint64_
     }
     if ((threadIdx.x & 31) == 0 && t0) atomicMax(&s_t0, t0);
     __syncthreads();
-    MERGE_TRACE(0);                                 // heads / tails landed
     for (int e = threadIdx.x; e < S; e += blockDim.x) {
         const uint64_t key = buf[e];
         if (key == 0) continue;
@@ -148,7 +141,6 @@ __device__ inline void select_winners(const PublishedKeys& pub, int cap, uint64_
     if ((int)max_tot > pub.region_cap) max_tot = (unsigned)pub.region_cap;
     const int slots = (((int)max_tot + 31) / 32) * 32 * kPubRegions;   // flattened slots that can hold a key
     __syncthreads();                                // everybody is past the T1 count: buf may now be reused for the survivors
-    MERGE_TRACE(1);                                 // threshold known
     for (int base = 0; base < slots; base += per_round) {
         if (base > 0) {
 #pragma unroll
@@ -178,7 +170,6 @@ __device__ inline void select_winners(const PublishedKeys& pub, int cap, uint64_
         }
     }
     __syncthreads();
-    MERGE_TRACE(2);                                 // survivors gathered
     const int cnt = s_cnt;
     if (cnt > cap) {                               // mass ties: correct but slow path over everything that was published
         merge_all_regions(pub, s_rtot, cap, buf, out);
@@ -212,11 +203,12 @@ __device__ inline void select_winners(const PublishedKeys& pub, int cap, uint64_
 // stage: stage_cap >= max(3 kc, kc + lists) keys of scratch that nothing else uses until the winners are known (heads first, then
 // the local survivors); `out` may be its first kc entries.  s_total: one int per CTA, zero before a cluster barrier that precedes this call.
 // Falls back to merge_all_regions (every CTA, redundantly) when the survivors overflow `buf` or a CTA's stage.
-template <int INFLIGHT, int CSIZE, int THREADS, typename Cluster>
+template <int CSIZE, int THREADS, typename Cluster>
 __device__ inline void select_winners_cluster(Cluster& cluster, const PublishedKeys& pub, int cap, uint64_t* buf, uint64_t* stage, int stage_cap,
-                                              uint64_t* out, int* s_total, unsigned long long* tr = nullptr) {
+                                              uint64_t* out, int* s_total) {
     static_assert(kPubRegions % CSIZE == 0, "regions must divide over the cluster");
     constexpr int RPC = kPubRegions / CSIZE;        // regions scanned by one CTA
+    constexpr int INFLIGHT = 24;                    // key loads in flight per thread
     __shared__ unsigned long long s_t0, s_t1;
     __shared__ int s_cnt;
     __shared__ unsigned s_rtot[kPubRegions];
@@ -250,7 +242,6 @@ __device__ inline void select_winners_cluster(Cluster& cluster, const PublishedK
     }
     if ((threadIdx.x & 31) == 0 && t0) atomicMax(&s_t0, t0);
     __syncthreads();
-    MERGE_TRACE(0);                                 // heads / tails landed
     for (int e = threadIdx.x; e < S; e += blockDim.x) {
         const uint64_t key = stage[e];
         if (key == 0) continue;
@@ -266,7 +257,6 @@ __device__ inline void select_winners_cluster(Cluster& cluster, const PublishedK
     if ((int)max_tot > pub.region_cap) max_tot = (unsigned)pub.region_cap;
     const int slots = (((int)max_tot + 31) / 32) * 32 * RPC;
     __syncthreads();                                // the heads are dead: `stage` now collects this CTA's survivors
-    MERGE_TRACE(1);                                 // threshold known
     for (int base = 0; base < slots; base += per_round) {
         if (base > 0) {
 #pragma unroll
@@ -307,7 +297,6 @@ __device__ inline void select_winners_cluster(Cluster& cluster, const PublishedK
         }
     }
     cluster.sync();                                 // every CTA's survivors are in every CTA's buf (and every stage is dead)
-    MERGE_TRACE(2);                                 // survivors gathered
     const int total = *s_total;
     if (total > cap) {
         merge_all_regions(pub, s_rtot, cap, buf, out);
