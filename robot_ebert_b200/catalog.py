@@ -357,7 +357,9 @@ class CatalogStore:
         re-scores them from the catalog of record as always.  Returns the proven bound on |shadow score - true score|:
         max_r ||x_r - dequant(q8_r)|| / ||x_r|| (Cauchy-Schwarz, any unit query) plus the worst-case error of the two
         int8 query planes.  A request whose proof margin does not clear that bound silently takes the standard path, so
-        results never depend on the shadow."""
+        results never depend on the shadow.  The streaming kernel has no int8 variant for rows of 5 or 7-11 chunks per lane
+        (d = 2049-2560 and 3073-5632, d = 4096 among them): there single requests always take the standard path, and the
+        shadow serves only the batched int8 GEMM."""
         lib = nat.load()
         ld8, _ = self.layout(self.n, self.d, "i8")
         with torch.cuda.device(self.device):

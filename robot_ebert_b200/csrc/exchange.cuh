@@ -190,6 +190,8 @@ struct Published {
 int finalize_published_launch(const Published& pub, const GemvFused& f, int64_t row_base, cudaStream_t st);
 int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_filter_t* filter, int32_t kc, void* workspace,
                 size_t workspace_bytes, uint64_t* cand_keys, const GemvFused* fused, cudaStream_t st);
+// false for an int8 shadow whose rows no streaming kernel takes (gemv_launch would return REBERT_ERR_UNSUPPORTED)
+bool gemv_streams(const rebert_catalog_t* cat);
 int stage_profile_launch(const rebert_catalog_t* cat, const int32_t* liked_host, const float* w_host, int n_liked, const int32_t* excl_host,
                          int n_excl, int32_t* excl_dev, double* sum64, double* wsum, float* qn32, double* qn64, const Exchange* x,
                          cudaStream_t st);

@@ -674,6 +674,12 @@ static bool use_generic(const RowLayout& L) {
     return true;
 }
 
+// The int8 shadow has register-query kernels only (launch_gemv_i8): rows of 5 or 7-11 chunks per lane (d = 2049-2560,
+// 3073-5632) have none, and such a shadow serves only the batched int8 GEMM.
+bool gemv_streams(const rebert_catalog_t* cat) {
+    return cat->dtype != REBERT_I8 || !use_generic(row_layout(cat->d, cat->dtype));
+}
+
 }  // namespace rebert
 
 using namespace rebert;

@@ -219,7 +219,8 @@ REBERT_API int rebert_recommend_host(const rebert_catalog_t* cat, const float* q
                                  : 0u;
 
     // ---- proof loop: each attempt is the streaming launch + its cluster kernel + one synchronisation
-    const bool try_shadow = proof && proof->shadow && k <= proof->shadow_max_k && proof->shadow_eps > 0.0;
+    // a shadow without a streaming kernel for its rows cannot help: the plain pass answers, as when its bound proves nothing
+    const bool try_shadow = proof && proof->shadow && k <= proof->shadow_max_k && proof->shadow_eps > 0.0 && gemv_streams(proof->shadow);
     int cur_kc = kc;
     bool shadow_turn = try_shadow;
     while (true) {

@@ -8,28 +8,6 @@ namespace rebert {
 
 __device__ __forceinline__ uint64_t ldcg_u64(const uint64_t* p) { return __ldcg((const unsigned long long*)p); }
 
-// `total` unordered keys (zeros allowed) -> the kc best, sorted, in `out`; buf holds `cap` keys.  Correct for any input,
-// slow: used only when mass ties overflow the pruned paths.
-__device__ inline void chunked_merge(const uint64_t* __restrict__ in, int total, int kc, int cap, uint64_t* buf, uint64_t* out) {
-    int done = 0, carried = 0;
-    while (true) {
-        int take = total - done;
-        if (take > cap - carried) take = cap - carried;
-        for (int i = threadIdx.x; i < take; i += blockDim.x) buf[carried + i] = ldcg_u64(in + done + i);
-        const int filled = carried + take;
-        int p2 = 2;
-        while (p2 < filled) p2 <<= 1;
-        for (int i = filled + threadIdx.x; i < p2; i += blockDim.x) buf[i] = 0;
-        __syncthreads();
-        block_bitonic_sort_desc(buf, p2);
-        done += take;
-        carried = kc;
-        if (done >= total) break;
-    }
-    for (int i = threadIdx.x; i < kc; i += blockDim.x) out[i] = buf[i];
-    __syncthreads();
-}
-
 constexpr int kPubRegions = 16;             // compaction regions (CTA b publishes into region b % 16: 16x less contention on a cursor)
 
 // What the CTAs of the streaming kernel publish (all pointers into the launch workspace).
