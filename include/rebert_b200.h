@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define REBERT_ABI_VERSION 3
+#define REBERT_ABI_VERSION 4
 
 #if defined(__GNUC__)
 #define REBERT_API __attribute__((visibility("default")))
@@ -87,6 +87,19 @@ typedef struct {
     uint16_t        year_lo, year_hi;/* keep year_lo <= year <= year_hi */
     uint32_t        reserved;
 } rebert_filter_t;
+
+/* Per-QUERY genre / year predicate of a batch (rebert_gemm_topk_filtered): query u keeps local row r iff
+ *   (genre_any[u] == 0 || (genre_bits[r] & genre_any[u]) != 0) && year_lo[u] <= year[r] <= year_hi[u].
+ * Each test comes as a pair of the catalog's column and the per-query arrays: genre_bits + genre_any, year + year_lo /
+ * year_hi.  A NULL pair switches that test off for every query; half a pair is REBERT_ERR_INVALID.  A query with
+ * (0, 0, 65535) is unrestricted. */
+typedef struct {
+    const uint32_t* genre_bits;      /* [n] local, per row */
+    const uint16_t* year;            /* [n] local, per row */
+    const uint32_t* genre_any;       /* [b], device */
+    const uint16_t* year_lo;         /* [b], device */
+    const uint16_t* year_hi;         /* [b], device */
+} rebert_query_filter_t;
 
 /* How ONE RANK of a row-sharded catalog reaches its peers: NVLink peer memory, no NCCL on the request path.
  * Every rank owns a peer-mapped buffer of rebert_exchange_buffer_bytes(world, k_max, prof_len, channels) bytes,
@@ -303,6 +316,15 @@ REBERT_API int rebert_gemm_topk(const rebert_catalog_t* cat, const void* qbf16, 
                      size_t workspace_bytes,
                      int64_t* out_rows, double* out_scores, int32_t* out_count, int32_t* out_status,
                      rebert_stream stream);
+/* rebert_gemm_topk with a per-query predicate on top of the shared row_filter (query_filter NULL = rebert_gemm_topk).  The
+ * threshold sample leaves out the rows each query's test rejects, so its survivor count stays at the plan's figure; the
+ * filter GEMM's epilogue drops the rejected winners.  A query with fewer than sample_rank allowed sampled rows gets no
+ * threshold: every allowed row survives, and an overflowing candidate buffer sets its status. */
+REBERT_API int rebert_gemm_topk_filtered(const rebert_catalog_t* cat, const void* qbf16, const double* q64, const int64_t* excl_row_ptr,
+                                         const int32_t* excl_col, const rebert_filter_t* row_filter,
+                                         const rebert_query_filter_t* query_filter, const rebert_gemm_plan_t* plan, void* workspace,
+                                         size_t workspace_bytes, int64_t* out_rows, double* out_scores, int32_t* out_count,
+                                         int32_t* out_status, rebert_stream stream);
 /* ---- the same batched path with INT8 OPERANDS: the filter GEMM streams the prefilter shadow (rebert_catalog_quantize_i8)
  * with tcgen05 kind::i8 — half the bytes and twice the tensor rate of bf16 — and int8 queries; exact integer accumulation.
  * Only the FILTER is approximate: candidates are re-scored in fp64 from the catalog of record exactly as in
@@ -327,6 +349,12 @@ REBERT_API int rebert_gemm_topk_i8(const rebert_catalog_t* cat, const rebert_cat
                                    const rebert_filter_t* row_filter, const rebert_gemm_plan_t* plan, void* workspace,
                                    size_t workspace_bytes, int64_t* out_rows, double* out_scores, int32_t* out_count,
                                    int32_t* out_status, rebert_stream stream);
+/* rebert_gemm_topk_i8 with a per-query predicate, as rebert_gemm_topk_filtered (query_filter NULL = rebert_gemm_topk_i8). */
+REBERT_API int rebert_gemm_topk_i8_filtered(const rebert_catalog_t* cat, const rebert_catalog_t* shadow, const void* q8, const float* qscale,
+                                            const double* qeps, const double* q64, const int64_t* excl_row_ptr, const int32_t* excl_col,
+                                            const rebert_filter_t* row_filter, const rebert_query_filter_t* query_filter,
+                                            const rebert_gemm_plan_t* plan, void* workspace, size_t workspace_bytes, int64_t* out_rows,
+                                            double* out_scores, int32_t* out_count, int32_t* out_status, rebert_stream stream);
 /* out[u, j] = (sum_c q8[u, c] * shadow[j, c]) * factor[j] * qscale[u] for rows [row0, row0 + nrows), fp32 [b, nrows]. */
 REBERT_API int rebert_gemm_scores_i8(const rebert_catalog_t* shadow, const void* q8, const float* qscale, int32_t b, int64_t row0,
                                      int64_t nrows, float* out, rebert_stream stream);

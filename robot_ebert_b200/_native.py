@@ -12,7 +12,7 @@ F32, BF16 = 0, 1
 I8 = 2          # prefilter shadow only (rebert_catalog_quantize_i8)
 DTYPES = {"fp32": F32, "bf16": BF16, "i8": I8}
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_WORKSPACE, ERR_CUDA, ERR_DEVICE = 0, -1, -2, -3, -4, -5
 
 
@@ -32,6 +32,12 @@ class Filter(C.Structure):
     _fields_ = [("exclude_bitmap", C.c_void_p), ("exclude_rows", C.c_void_p), ("n_exclude", C.c_int32),
                 ("genre_any", C.c_uint32), ("genre_bits", C.c_void_p), ("year", C.c_void_p),
                 ("year_lo", C.c_uint16), ("year_hi", C.c_uint16), ("reserved", C.c_uint32)]
+
+
+class QueryFilter(C.Structure):
+    """rebert_query_filter_t: per-query genre / year tests of a batch (catalog columns [n] + per-query arrays [b])."""
+    _fields_ = [("genre_bits", C.c_void_p), ("year", C.c_void_p), ("genre_any", C.c_void_p), ("year_lo", C.c_void_p),
+                ("year_hi", C.c_void_p)]
 
 
 class Exchange(C.Structure):
@@ -96,6 +102,10 @@ _SIGS = {
     "rebert_query_quantize_i8": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, _P, _P, _P, _P]),
     "rebert_gemm_topk_i8": (C.c_int, [C.POINTER(Catalog), C.POINTER(Catalog), _P, _P, _P, _P, _P, _P, C.POINTER(Filter), C.POINTER(GemmPlan),
                                       _P, C.c_size_t, _P, _P, _P, _P, _P]),
+    "rebert_gemm_topk_filtered": (C.c_int, [C.POINTER(Catalog), _P, _P, _P, _P, C.POINTER(Filter), C.POINTER(QueryFilter),
+                                            C.POINTER(GemmPlan), _P, C.c_size_t, _P, _P, _P, _P, _P]),
+    "rebert_gemm_topk_i8_filtered": (C.c_int, [C.POINTER(Catalog), C.POINTER(Catalog), _P, _P, _P, _P, _P, _P, C.POINTER(Filter),
+                                               C.POINTER(QueryFilter), C.POINTER(GemmPlan), _P, C.c_size_t, _P, _P, _P, _P, _P]),
     "rebert_gemm_scores_i8": (C.c_int, [C.POINTER(Catalog), _P, _P, C.c_int32, C.c_int64, C.c_int64, _P, _P]),
     "rebert_synth_rows": (C.c_int, [C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
 }

@@ -34,6 +34,81 @@ class RowFilter:
         self.genre_any, self.year_lo, self.year_hi = int(genre_any), int(year_lo), int(year_hi)
         self.exclude_bitmap = exclude_bitmap
 
+    @property
+    def has_genre_or_year(self) -> bool:
+        return bool(self.genre_any) or (self.year_lo, self.year_hi) != (0, 65535)
+
+
+def _unsigned_column(x, name: str, dtype, hi: int) -> np.ndarray:
+    a = np.asarray(x)
+    if a.ndim != 1 or len(a) == 0:
+        raise ValueError(f"QueryFilters.{name} must be a non-empty 1-D array, got shape {a.shape}")
+    if not np.issubdtype(a.dtype, np.integer):
+        raise ValueError(f"QueryFilters.{name} must hold integers, got {a.dtype}")
+    if a.min() < 0 or a.max() > hi:
+        raise ValueError(f"QueryFilters.{name} out of range [0, {hi}]")
+    return a.astype(dtype)
+
+
+class QueryFilters:
+    """One genre / year predicate per user of a batch (recommend_batch(query_filters=...)).  User u keeps row r iff
+    (genre_any[u] == 0 or genre_bits[r] & genre_any[u] != 0) and year_lo[u] <= year[r] <= year_hi[u], on top of its
+    exclusion CSR and a shared exclude_bitmap.  (0, 0, 65535) leaves a user unrestricted; year_lo > year_hi allows no row.
+    year_lo / year_hi default to the whole range."""
+
+    def __init__(self, genre_any, year_lo=None, year_hi=None):
+        self.genre_any = _unsigned_column(genre_any, "genre_any", np.uint32, 0xFFFFFFFF)
+        b = len(self.genre_any)
+        self.year_lo = _unsigned_column(np.zeros(b, np.uint16) if year_lo is None else year_lo, "year_lo", np.uint16, 65535)
+        self.year_hi = _unsigned_column(np.full(b, 65535, np.uint16) if year_hi is None else year_hi, "year_hi", np.uint16, 65535)
+        if len(self.year_lo) != b or len(self.year_hi) != b:
+            raise ValueError(f"QueryFilters: genre_any, year_lo and year_hi must have one entry per user ({b}, {len(self.year_lo)}, "
+                             f"{len(self.year_hi)})")
+        self.has_genre = bool(self.genre_any.any())
+        self.has_year = bool((self.year_lo != 0).any() or (self.year_hi != 65535).any())
+        self._dev = {}
+
+    def __len__(self) -> int:
+        return len(self.genre_any)
+
+    def row_filter(self, u: int, exclude_bitmap: Optional[torch.Tensor] = None) -> RowFilter:
+        """User u's predicate as the RowFilter of a single request (the per-query route of a batch)."""
+        return RowFilter(int(self.genre_any[u]), int(self.year_lo[u]), int(self.year_hi[u]), exclude_bitmap)
+
+    def subset(self, users) -> "QueryFilters":
+        users = np.asarray(users, dtype=np.int64)
+        return QueryFilters(self.genre_any[users], self.year_lo[users], self.year_hi[users])
+
+    def validate(self, b: int, row_filter: Optional[RowFilter], genre_bits, year) -> None:
+        """ValueError unless these filters fit a batch of b users with `row_filter` shared and the catalog's metadata columns
+        genre_bits / year (None when set_metadata was not called).  A shared genre or year test is refused: the per-query
+        route takes one RowFilter, which cannot hold the AND of two genre masks.  A shared exclude_bitmap is fine."""
+        if len(self) != b:
+            raise ValueError(f"query_filters has {len(self)} users, the batch {b}")
+        if row_filter is not None and row_filter.has_genre_or_year:
+            raise ValueError("query_filters cannot be combined with a shared row_filter genre or year test "
+                             "(put the shared test into every user's filter instead)")
+        if self.has_genre and genre_bits is None:
+            raise ValueError("query_filters genre_any needs set_metadata()")
+        if self.has_year and year is None:
+            raise ValueError("query_filters year range needs set_metadata()")
+
+    def device_arrays(self, dev: torch.device):
+        """(genre_any, year_lo, year_hi) on `dev`, copied once per device and kept (int32 / int16 views of the unsigned data)."""
+        key = str(dev)
+        if key not in self._dev:
+            self._dev[key] = tuple(torch.from_numpy(a.view(np.int32 if a.dtype == np.uint32 else np.int16)).to(dev)
+                                   for a in (self.genre_any, self.year_lo, self.year_hi))
+        return self._dev[key]
+
+
+def user_row_filter(query_filters: Optional[QueryFilters], u: int, row_filter: Optional[RowFilter]) -> Optional[RowFilter]:
+    """The RowFilter the per-query route applies to user u of a batch: the shared row_filter, or with query_filters the
+    user's own test plus the shared exclude_bitmap."""
+    if query_filters is None:
+        return row_filter
+    return query_filters.row_filter(u, None if row_filter is None else row_filter.exclude_bitmap)
+
 
 class _Scratch:
     """Per-thread staging + device scratch so concurrent requests (FastAPI's threadpool) never share buffers."""
@@ -601,6 +676,19 @@ class CatalogStore:
             f.year, f.year_lo, f.year_hi = self.year.data_ptr(), row_filter.year_lo, row_filter.year_hi
         return f
 
+    def _query_filter_struct(self, query_filters: Optional[QueryFilters]):
+        """rebert_query_filter_t for the tests some user of the batch actually has (None when no user has one: the kernels
+        then run exactly as without query filters)."""
+        if query_filters is None or not (query_filters.has_genre or query_filters.has_year):
+            return None
+        genre_any, year_lo, year_hi = query_filters.device_arrays(self.device)
+        f = nat.QueryFilter()
+        if query_filters.has_genre:
+            f.genre_bits, f.genre_any = self.genre_bits.data_ptr(), genre_any.data_ptr()
+        if query_filters.has_year:
+            f.year, f.year_lo, f.year_hi = self.year.data_ptr(), year_lo.data_ptr(), year_hi.data_ptr()
+        return f
+
     def stage_inputs(self, query, liked_rows, weights, exclude_rows, k, kc, profile_partial_only: bool = False):
         """Pack the request into one pinned buffer, issue ONE H2D copy, and enqueue query normalisation or the
         profile build on the current stream.  Returns (device pointer of the exclusion list, its length)."""
@@ -784,31 +872,38 @@ class CatalogStore:
         return q8, qscale, qeps
 
     def enqueue_batch(self, plan, qbf16, q64, excl_ptr, excl_col, ws, out_rows, out_scores, out_count, out_status,
-                      row_filter: Optional[RowFilter] = None, shadow=None):
+                      row_filter: Optional[RowFilter] = None, shadow=None, query_filters: Optional[QueryFilters] = None):
         """Device-resident batched step (sample -> thresholds -> filtered GEMM -> select -> exact pass).
         shadow = (q8, qscale, qeps) from quantize_queries: the GEMMs run on int8 operands over the prefilter shadow (plan
-        from gemm_plan(shadow=True)); the exact pass reads the catalog of record either way."""
+        from gemm_plan(shadow=True)); the exact pass reads the catalog of record either way.
+        query_filters: one genre / year test per query (QueryFilters), applied inside the threshold sample and the GEMM epilogue."""
         lib = nat.load()
+        if query_filters is not None:
+            query_filters.validate(plan.b, row_filter, self.genre_bits, self.year)
         f = self._filter_struct(row_filter)
+        qf = self._query_filter_struct(query_filters)
+        fp, qfp = (None if f is None else C.byref(f)), (None if qf is None else C.byref(qf))
         st = torch.cuda.current_stream().cuda_stream
         if shadow is not None:
             q8, qscale, qeps = shadow
-            nat.check(lib.rebert_gemm_topk_i8(C.byref(self._c), C.byref(self._c8), q8.data_ptr(), qscale.data_ptr(), qeps.data_ptr(),
-                                              q64.data_ptr(), _ptr(excl_ptr), _ptr(excl_col), None if f is None else C.byref(f),
-                                              C.byref(plan), ws.data_ptr(), ws.numel(), out_rows.data_ptr(), out_scores.data_ptr(),
-                                              out_count.data_ptr(), out_status.data_ptr(), st))
+            nat.check(lib.rebert_gemm_topk_i8_filtered(C.byref(self._c), C.byref(self._c8), q8.data_ptr(), qscale.data_ptr(),
+                                                       qeps.data_ptr(), q64.data_ptr(), _ptr(excl_ptr), _ptr(excl_col), fp, qfp,
+                                                       C.byref(plan), ws.data_ptr(), ws.numel(), out_rows.data_ptr(), out_scores.data_ptr(),
+                                                       out_count.data_ptr(), out_status.data_ptr(), st))
             return
-        nat.check(lib.rebert_gemm_topk(C.byref(self._c), qbf16.data_ptr(), q64.data_ptr(), _ptr(excl_ptr), _ptr(excl_col),
-                                       None if f is None else C.byref(f),
-                                       C.byref(plan), ws.data_ptr(), ws.numel(), out_rows.data_ptr(), out_scores.data_ptr(),
-                                       out_count.data_ptr(), out_status.data_ptr(), st))
+        nat.check(lib.rebert_gemm_topk_filtered(C.byref(self._c), qbf16.data_ptr(), q64.data_ptr(), _ptr(excl_ptr), _ptr(excl_col), fp,
+                                                qfp, C.byref(plan), ws.data_ptr(), ws.numel(), out_rows.data_ptr(), out_scores.data_ptr(),
+                                                out_count.data_ptr(), out_status.data_ptr(), st))
 
     def recommend_batch(self, *, queries: Optional[np.ndarray] = None, liked_ptr: Optional[np.ndarray] = None,
                         liked_col: Optional[np.ndarray] = None, liked_w: Optional[np.ndarray] = None,
                         excl_ptr: Optional[np.ndarray] = None, excl_col: Optional[np.ndarray] = None, k: int = 10,
-                        row_filter: Optional[RowFilter] = None, return_info: bool = False, prefilter: Optional[bool] = None):
+                        row_filter: Optional[RowFilter] = None, return_info: bool = False, prefilter: Optional[bool] = None,
+                        query_filters: Optional[QueryFilters] = None):
         """Top-k for many users at once (lib.py:51-55 per user) on the tcgen05 path.
         row_filter: optional per-row predicate (genre / year / bitmap) shared by the whole batch.
+        query_filters: optional genre / year test per user (QueryFilters), applied in the same tensor-core pass.  It may be
+        combined with a shared exclude_bitmap, not with a shared genre or year test (ValueError).
         prefilter: None = int8 operands (twice the tensor rate) when enable_prefilter() has built a shadow the GEMM can use;
         True = require that; False = bf16 operands.  The result is the same either way.
 
@@ -825,6 +920,8 @@ class CatalogStore:
         with torch.cuda.device(dev):
             qn32, qn64, qbf = self.prepare_batch(queries, liked_ptr, liked_col, liked_w)
             b = qbf.shape[0]
+            if query_filters is not None:
+                query_filters.validate(b, row_filter, self.genre_bits, self.year)
             if prefilter and not self.batch_shadow_ok:
                 raise ValueError("prefilter=True needs enable_prefilter() and rows of whole 128-byte int8 k-blocks")
             use_shadow = self.batch_shadow_ok and prefilter is not False
@@ -836,7 +933,7 @@ class CatalogStore:
                     if e.code != nat.ERR_UNSUPPORTED:
                         raise    # ERR_UNSUPPORTED: catalog too small for the sampled-threshold scheme, plan stays None
             if plan is None:        # too small, or neither operand type fits the GEMM: one fused GEMV per user instead
-                return self._recommend_batch_loop(qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter)
+                return self._recommend_batch_loop(qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter, query_filters)
             ep = ec = None
             if excl_ptr is not None:
                 excl_ptr, excl_col = sorted_csr(excl_ptr, excl_col)
@@ -844,12 +941,13 @@ class CatalogStore:
                     raise ValueError("exclusion CSR must have one segment per query")
                 ep = torch.from_numpy(excl_ptr).to(dev)
                 ec = torch.from_numpy(excl_col).to(dev)
-            rows, scores, counts, status = self._run_batch(plan, qbf, qn64, qn32, ep, ec, row_filter, use_shadow)
+            rows, scores, counts, status = self._run_batch(plan, qbf, qn64, qn32, ep, ec, row_filter, use_shadow, query_filters)
             redo = np.nonzero(status)[0]
             if len(redo) and long_list:
-                redo = self._widened_retry(redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts)
+                redo = self._widened_retry(redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts,
+                                           query_filters)
             # proven single-query route for the ones the batch could not prove
-            self._rerun_prepared(redo, qn32, qn64, excl_ptr, ec, k, row_filter, rows, scores, counts)
+            self._rerun_prepared(redo, qn32, qn64, excl_ptr, ec, k, row_filter, rows, scores, counts, query_filters)
         if return_info:
             return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}, "int8_operands": use_shadow,
                                           "per_query": len(redo)}
@@ -858,7 +956,7 @@ class CatalogStore:
     # Largest k of the tensor-core path (rebert_gemm_plan); also the cap of the widened retry of long lists.
     BATCH_MAX_K = 2048
 
-    def _run_batch(self, plan, qbf, qn64, qn32, ep, ec, row_filter, use_shadow):
+    def _run_batch(self, plan, qbf, qn64, qn32, ep, ec, row_filter, use_shadow, query_filters=None):
         """One batched pass with freshly allocated workspace and outputs; returns host (rows, scores, counts, status)."""
         lib = nat.load()
         dev = self.device
@@ -869,10 +967,11 @@ class CatalogStore:
         out_count = torch.empty(b, dtype=torch.int32, device=dev)
         out_status = torch.empty(b, dtype=torch.int32, device=dev)
         self.enqueue_batch(plan, qbf, qn64, ep, ec, ws, out_rows, out_scores, out_count, out_status, row_filter,
-                           shadow=self.quantize_queries(qn32) if use_shadow else None)
+                           shadow=self.quantize_queries(qn32) if use_shadow else None, query_filters=query_filters)
         return out_rows.cpu().numpy(), out_scores.cpu().numpy(), out_count.cpu().numpy(), out_status.cpu().numpy()
 
-    def _widened_retry(self, redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts):
+    def _widened_retry(self, redo, k, use_shadow, qbf, qn64, qn32, excl_ptr, excl_col, row_filter, rows, scores, counts,
+                       query_filters=None):
         """Long lists: the queries the batched pass could not prove run once more, as a sub-batch at k' = min(2k, 2048) with
         its longer candidate list, and keep the first k results (a proven top-k' starts with the proven top-k).  Much cheaper
         than the per-query route when it works.  Fills rows / scores / counts in place; returns the queries still unproven."""
@@ -895,14 +994,14 @@ class CatalogStore:
             ep = torch.from_numpy(sub_ptr).to(dev)
             ec = torch.from_numpy(np.concatenate(segs) if sub_ptr[-1] else np.zeros(1, dtype=np.int32)).to(dev)
         r2, s2, c2, st2 = self._run_batch(plan, qbf[idx].contiguous(), qn64[idx].contiguous(), qn32[idx].contiguous(), ep, ec,
-                                          row_filter, use_shadow)
+                                          row_filter, use_shadow, None if query_filters is None else query_filters.subset(redo))
         ok = st2 == 0
         for i in np.nonzero(ok)[0]:
             u = redo[i]
             rows[u], scores[u], counts[u] = r2[i, :k], s2[i, :k], min(int(c2[i]), k)
         return redo[~ok]
 
-    def _recommend_batch_loop(self, qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter=None):
+    def _recommend_batch_loop(self, qn32, qn64, excl_ptr, excl_col, k, return_info, row_filter=None, query_filters=None):
         """Small catalogs, catalogs neither GEMM operand type takes, and k > 2048: the batch is served one prepared query at
         a time, by the single-query kernel for k <= 240 and by topk_prepared_large_k above."""
         b = qn32.shape[0]
@@ -913,15 +1012,15 @@ class CatalogStore:
         if excl_ptr is not None:
             ecp, ecol = sorted_csr(excl_ptr, excl_col)
             ec = torch.from_numpy(ecol).to(self.device)
-        self._rerun_prepared(range(b), qn32, qn64, ecp, ec, k, row_filter, rows, scores, counts)
+        self._rerun_prepared(range(b), qn32, qn64, ecp, ec, k, row_filter, rows, scores, counts, query_filters)
         if return_info:
             return rows, scores, counts, {"status": np.zeros(b, dtype=np.int32), "plan": None, "per_query": b}
         return rows, scores, counts
 
-    def _rerun_prepared(self, users, qn32, qn64, excl_ptr, excl_col_dev, k, row_filter, rows, scores, counts):
+    def _rerun_prepared(self, users, qn32, qn64, excl_ptr, excl_col_dev, k, row_filter, rows, scores, counts, query_filters=None):
         """Proven single-query route for `users` of a prepared batch (qn32 / qn64 [b, ld]): topk_prepared, or
         topk_prepared_large_k for k > 240, over the user's segment of the sorted exclusion CSR (host excl_ptr, device
-        excl_col_dev).  Overwrites those users' rows / scores / counts."""
+        excl_col_dev) and the user's own filter (user_row_filter).  Overwrites those users' rows / scores / counts."""
         large = nat.load().rebert_candidates_for_k(k) == 0
         s = self._scratch()
         for u in users:
@@ -930,7 +1029,7 @@ class CatalogStore:
             ptr, ne = None, 0
             if excl_ptr is not None and excl_ptr[u + 1] > excl_ptr[u]:
                 ptr, ne = excl_col_dev.data_ptr() + 4 * int(excl_ptr[u]), int(excl_ptr[u + 1] - excl_ptr[u])
-            r, sc = (self.topk_prepared_large_k if large else self.topk_prepared)(k, ptr, ne, row_filter)
+            r, sc = (self.topk_prepared_large_k if large else self.topk_prepared)(k, ptr, ne, user_row_filter(query_filters, u, row_filter))
             rows[u, :], scores[u, :] = -1, -np.inf
             rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
 

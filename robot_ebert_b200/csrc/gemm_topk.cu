@@ -50,11 +50,33 @@ constexpr int STAGE_SLOTS = 24;                                 // per-thread st
 constexpr int SMEM_STAGING = STAGE_SLOTS * 128 * 8;
 constexpr int SMEM_INV = 2 * BN * 4;
 constexpr int GEMM_SMEM = GEMM_STAGES * STAGE_BYTES + SMEM_STAGING + SMEM_INV + 256 + 1024;   // + alignment slack
+// per-query filters only: the tile's genre_bits [2][BN] and year [2][BN], behind the barriers (227,584 B of 232,448 B in all)
+constexpr int SMEM_QF = 2 * BN * 4 + 2 * BN * 2;
 constexpr uint32_t TMEM_COLS = 512;
 // k above kLargeK0 (the single-query kernel's limit) takes the long-list stages; kLargeKMax bounds kc at 4096 (int8 plans)
 constexpr int kLargeK0 = 240, kLargeKMax = 2048, kLargeRank = 64, kLargeKcMax = 4096;
 
 enum { MODE_STORE = 0, MODE_FILTER = 1 };
+
+// Per-query genre / year predicate of a batch (rebert_query_filter_t).  A null pair switches that test off for every query.
+struct QueryFilter {
+    const uint32_t* genre_bits;   // [n] local
+    const uint16_t* year;         // [n] local
+    const uint32_t* genre_any;    // [b]
+    const uint16_t* year_lo;      // [b]
+    const uint16_t* year_hi;      // [b]
+};
+// One query's test: keep a row iff (genre_any == 0 or genre_bits & genre_any) and year_lo <= year <= year_hi
+struct QueryTest { uint32_t genre_any, year_lo, year_hi; };
+__device__ __forceinline__ QueryTest load_query_test(const QueryFilter& f, int q) {
+    QueryTest t{0u, 0u, 0xFFFFu};
+    if (f.genre_any) t.genre_any = __ldg(f.genre_any + q);
+    if (f.year_lo) { t.year_lo = __ldg(f.year_lo + q); t.year_hi = __ldg(f.year_hi + q); }
+    return t;
+}
+__device__ __forceinline__ bool query_allows(const QueryTest& t, uint32_t genre_bits, uint32_t year) {
+    return (t.genre_any == 0u || (genre_bits & t.genre_any) != 0u) && year >= t.year_lo && year <= t.year_hi;
+}
 
 struct GemmParams {
     int b;                  // queries
@@ -77,6 +99,7 @@ struct GemmParams {
     unsigned* cand_count;   // [b]
     int cand_cap;
     int* status;            // [b]
+    QueryFilter qf;         // MODE_FILTER with the QF template flag: per-query genre / year tests
 };
 
 // ---------------------------------------------------------------- PTX wrappers ------------------------------
@@ -160,9 +183,12 @@ template <bool I8> __device__ __forceinline__ float acc_f32(uint32_t v) { return
 // onto the bit pattern of 1.5 * 2^23 plus an FADD, which run on the main pipes: 7.44 vs 7.21 ms at 4096 x 1M.  The kernel sits at the
 // board's power limit, where two instructions on the main pipes cost more than one on an idle pipe saves.  DESIGN.md 4.3.)
 
-template <int MODE, bool I8>
+// QF (per-query filters): the rare path drops each winner the query's own genre / year test rejects before it is staged or
+// counted; the tile's genre_bits / year sit in shared memory (gb_chunk / yr_chunk), so the test is two LDS per winner.
+template <int MODE, bool I8, bool QF>
 __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32_t* v, const float* inv_chunk, float tau, float qs, int q,
-                                               float* out_row, uint32_t row_chunk0, uint64_t* staging, int et, int& cnt) {
+                                               float* out_row, uint32_t row_chunk0, uint64_t* staging, int et, int& cnt,
+                                               const uint32_t* gb_chunk, const uint16_t* yr_chunk, const QueryTest& qt) {
     float s[32];
 #pragma unroll
     for (int c4 = 0; c4 < 8; ++c4) {
@@ -194,6 +220,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32
             while (mask) {
                 const int c = __ffs(mask) - 1;
                 mask &= mask - 1;
+                if (QF && !query_allows(qt, gb_chunk[c], yr_chunk[c])) continue;
                 float val = s[0];
 #pragma unroll
                 for (int j = 1; j < 32; ++j) val = (c == j) ? s[j] : val;       // register select, no local memory
@@ -205,9 +232,10 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32
     }
 }
 
-template <int MODE, bool I8>
+template <int MODE, bool I8, bool QF>
 __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t taddr, const float* inv, float tau, float qs, int q, int64_t row0,
-                                              int64_t rt, uint64_t* staging, int et, int& cnt) {
+                                              int64_t rt, uint64_t* staging, int et, int& cnt, const uint32_t* gb, const uint16_t* yr,
+                                              const QueryTest& qt) {
     float* out_row = nullptr;
     if (MODE == MODE_STORE) out_row = p.out + (int64_t)q * p.out_ld + rt * BN;
     uint32_t va[32], vb[32];
@@ -216,15 +244,31 @@ __device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tadd
 #pragma unroll
     for (int ch = 0; ch < BN / 32; ch += 2) {
         tc_ld32(taddr + (ch + 1) * 32, vb);                                     // in flight while chunk ch is processed
-        epilogue_chunk<MODE, I8>(p, va, inv + ch * 32, tau, qs, q, out_row + ch * 32, (uint32_t)(row0 + ch * 32), staging, et, cnt);
+        epilogue_chunk<MODE, I8, QF>(p, va, inv + ch * 32, tau, qs, q, out_row + ch * 32, (uint32_t)(row0 + ch * 32), staging, et, cnt,
+                                     gb + ch * 32, yr + ch * 32, qt);
         tc_wait_ld();
         if (ch + 2 < BN / 32) tc_ld32(taddr + (ch + 2) * 32, va);
-        epilogue_chunk<MODE, I8>(p, vb, inv + (ch + 1) * 32, tau, qs, q, out_row + (ch + 1) * 32, (uint32_t)(row0 + (ch + 1) * 32), staging, et, cnt);
+        epilogue_chunk<MODE, I8, QF>(p, vb, inv + (ch + 1) * 32, tau, qs, q, out_row + (ch + 1) * 32, (uint32_t)(row0 + (ch + 1) * 32), staging,
+                                     et, cnt, gb + (ch + 1) * 32, yr + (ch + 1) * 32, qt);
         if (ch + 2 < BN / 32) tc_wait_ld();
     }
 }
 
-template <int MODE, bool I8>
+// Shared by both kernels' epilogue warps: stage the tile's inv_norm (NaN marks rows beyond the shard and rows the batch
+// predicate filters out: they can never pass tau) and, with per-query filters, its genre_bits / year.
+template <bool QF>
+__device__ __forceinline__ void stage_tile_columns(const GemmParams& p, int64_t row0, int et, float* inv, uint32_t* gb, uint16_t* yr) {
+    for (int c = et; c < BN; c += 128) {
+        const int64_t r = row0 + c;
+        inv[c] = (r < p.n && (!p.has_pred || row_allowed(p.pred, (uint32_t)r))) ? __ldg(p.inv_norm + r) : __int_as_float(0x7FC00000);
+        if (QF) {
+            gb[c] = (r < p.n && p.qf.genre_bits) ? __ldg(p.qf.genre_bits + r) : 0u;
+            yr[c] = (r < p.n && p.qf.year) ? __ldg(p.qf.year + r) : (uint16_t)0;
+        }
+    }
+}
+
+template <int MODE, bool I8, bool QF = false>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_rows, const GemmParams p) {
     constexpr int BKE = I8 ? 2 * BK : BK;             // elements per 128-byte k-block
@@ -239,6 +283,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ C
     uint64_t* tfull_bar = bars + 2 * GEMM_STAGES;    // [2]
     uint64_t* tempty_bar = bars + 2 * GEMM_STAGES + 2;   // [2]
     uint32_t* tmem_slot = (uint32_t*)(bars + 2 * GEMM_STAGES + 4);
+    uint32_t* s_gb = (uint32_t*)((unsigned char*)bars + 256);                        // [2][BN]  QF only
+    uint16_t* s_yr = (uint16_t*)(s_gb + 2 * BN);                                       // [2][BN]  QF only
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t total_tiles = (int64_t)p.num_rt * p.num_qt;
@@ -320,20 +366,20 @@ gemm_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ C
             const int q = qt * BM + qrow;
             // inv_norm slice of this row tile -> smem (NaN marks rows beyond the shard so they never pass / are skipped)
             float* inv = s_inv + (tile_i & 1) * BN;
-            for (int c = et; c < BN; c += 128) {
-                const int64_t r = row0 + c;
-                // rows beyond the shard, and rows the batch predicate filters out, get NaN: they can never pass tau
-                inv[c] = (r < p.n && (!p.has_pred || row_allowed(p.pred, (uint32_t)r))) ? __ldg(p.inv_norm + r) : __int_as_float(0x7FC00000);
-            }
+            uint32_t* gb = s_gb + (tile_i & 1) * BN;
+            uint16_t* yr = s_yr + (tile_i & 1) * BN;
+            stage_tile_columns<QF>(p, row0, et, inv, gb, yr);
             float tau = INFINITY, qs = 1.f;
             if (I8 && q < p.b) qs = __ldg(p.qscale + q);
             if (MODE == MODE_FILTER && q < p.b) tau = I8 ? __ldg(p.tau + q) / qs : __ldg(p.tau + q);
+            QueryTest qtest{0u, 0u, 0xFFFFu};
+            if (QF && q < p.b) qtest = load_query_test(p.qf, q);
             asm volatile("bar.sync 1, 128;" ::: "memory");
             mbar_wait(&tfull_bar[acc], (tile_i >> 1) & 1u);
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN);
             int cnt = 0;
-            epilogue_tile<MODE, I8>(p, taddr, inv, tau, qs, q, row0, rt, staging, et, cnt);
+            epilogue_tile<MODE, I8, QF>(p, taddr, inv, tau, qs, q, row0, rt, staging, et, cnt, gb, yr, qtest);
             // accumulator drained: hand it back to the MMA warp before the (slow) global appends
             tc_fence_before();
             __syncwarp();
@@ -414,7 +460,7 @@ __device__ __forceinline__ void tc_mma_i8_2sm(uint32_t tmem_d, uint64_t desc_a, 
         : "memory");
 }
 
-template <int MODE, bool I8>
+template <int MODE, bool I8, bool QF = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 gemm2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_rows, const GemmParams p) {
     constexpr int BKE = I8 ? 2 * BK : BK;             // elements per 128-byte k-block
@@ -429,6 +475,8 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ 
     uint64_t* tfull_bar = bars + 2 * G2_STAGES;        // [2]          per CTA, arrived by the multicast commit
     uint64_t* tempty_bar = bars + 2 * G2_STAGES + 2;   // [2]          leader only: 2 x EPI_WARPS arrivals
     uint32_t* tmem_slot = (uint32_t*)(bars + 2 * G2_STAGES + 4);
+    uint32_t* s_gb = (uint32_t*)((unsigned char*)bars + 256);   // [2][BN]  QF only
+    uint16_t* s_yr = (uint16_t*)(s_gb + 2 * BN);                  // [2][BN]  QF only
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t cta_rank = cluster_ctarank();
@@ -516,20 +564,20 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ 
             const int acc = tile_i & 1;
             const int q = qt * 256 + (int)cta_rank * 128 + qrow;
             float* inv = s_inv + (tile_i & 1) * BN;
-            for (int c = et; c < BN; c += 128) {
-                const int64_t r = row0 + c;
-                // rows beyond the shard, and rows the batch predicate filters out, get NaN: they can never pass tau
-                inv[c] = (r < p.n && (!p.has_pred || row_allowed(p.pred, (uint32_t)r))) ? __ldg(p.inv_norm + r) : __int_as_float(0x7FC00000);
-            }
+            uint32_t* gb = s_gb + (tile_i & 1) * BN;
+            uint16_t* yr = s_yr + (tile_i & 1) * BN;
+            stage_tile_columns<QF>(p, row0, et, inv, gb, yr);
             float tau = INFINITY, qs = 1.f;
             if (I8 && q < p.b) qs = __ldg(p.qscale + q);
             if (MODE == MODE_FILTER && q < p.b) tau = I8 ? __ldg(p.tau + q) / qs : __ldg(p.tau + q);
+            QueryTest qtest{0u, 0u, 0xFFFFu};
+            if (QF && q < p.b) qtest = load_query_test(p.qf, q);
             asm volatile("bar.sync 1, 128;" ::: "memory");
             mbar_wait(&tfull_bar[acc], (tile_i >> 1) & 1u);
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * BN);
             int cnt = 0;
-            epilogue_tile<MODE, I8>(p, taddr, inv, tau, qs, q, row0, rt, staging, et, cnt);
+            epilogue_tile<MODE, I8, QF>(p, taddr, inv, tau, qs, q, row0, rt, staging, et, cnt, gb, yr, qtest);
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_remote(acc ? leader_tempty1 : leader_tempty0);
@@ -555,10 +603,13 @@ gemm2_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ 
 // ---------------------------------------------------------------------------------------------------------
 // Per query: r-th largest sample score after masking excluded rows (4-pass radix select on orderable keys).
 // Sample column j*256 + c is catalog row (tile0 + j*stride)*256 + c.
+// Per-query filters (has_qf): rows the query's own genre / year test rejects are masked like excluded rows, so the rank-th best
+// of the allowed sampled rows estimates the same quantile of the allowed population and the survivor count stays at the plan's
+// figure.  Fewer than `rank` allowed sampled rows give tau = -inf: every allowed row survives (an overflow sets status bit 2).
 // ---------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) select_threshold_kernel(float* sample, int keys_in_smem, int64_t s_cols, int64_t n,
                                                                int64_t row_base, int64_t tile0, int64_t tile_stride, int rank,
-                                                               DevFilter pred, int has_pred,
+                                                               DevFilter pred, int has_pred, QueryFilter qf, int has_qf,
                                                                const int64_t* __restrict__ excl_ptr,
                                                                const int32_t* __restrict__ excl_col, float* __restrict__ tau) {
     extern __shared__ uint32_t smem_keys[];        // [s_cols] when it fits, else the sample row is rewritten in place
@@ -570,10 +621,14 @@ __global__ void __launch_bounds__(256) select_threshold_kernel(float* sample, in
     const int32_t* ex = nullptr;
     int nex = 0;
     if (excl_ptr) { ex = excl_col + excl_ptr[q]; nex = (int)(excl_ptr[q + 1] - excl_ptr[q]); }
+    const QueryTest qt = has_qf ? load_query_test(qf, q) : QueryTest{0u, 0u, 0xFFFFu};
     for (int64_t j = threadIdx.x; j < s_cols; j += blockDim.x) {
         const int64_t row = (tile0 + (j / BN) * tile_stride) * BN + (j % BN);
         const float v = src[j];
-        keys[j] = (row < n && v == v && (!has_pred || row_allowed(pred, (uint32_t)row))) ? f32_orderable(v) : 0u;
+        bool keep = row < n && v == v && (!has_pred || row_allowed(pred, (uint32_t)row));
+        if (keep && has_qf)
+            keep = query_allows(qt, qf.genre_bits ? __ldg(qf.genre_bits + row) : 0u, qf.year ? (uint32_t)__ldg(qf.year + row) : 0u);
+        keys[j] = keep ? f32_orderable(v) : 0u;
     }
     __syncthreads();
     // knock out excluded rows that fall inside the sample: ~|excluded| scattered stores instead of a search per key
@@ -926,8 +981,10 @@ static void set_pred(GemmParams& p, const rebert_catalog_t* cat, const rebert_fi
 
 // `cat` is the operand catalog the tensor cores stream: the bf16 catalog of record, or its int8 shadow (then qmat is int8
 // [b, ld8] and p.qscale holds the queries' dequantisation steps).
-template <int MODE, bool I8>
+template <int MODE, bool I8, bool QF>
 static int launch_gemm_t(const rebert_catalog_t* cat, const void* qmat, GemmParams& p, cudaStream_t st) {
+    static_assert(!QF || MODE == MODE_FILTER, "per-query filters apply to the filter pass only");
+    constexpr int extra_smem = QF ? SMEM_QF : 0;
     const bool pair = p.b > BM;   // cta_group::2 needs >= 2 query tiles to pay off
     CUtensorMap map_q, map_rows;
     int rc = make_tmap(&map_q, qmat, p.b, cat->ld, BM, I8);
@@ -942,23 +999,23 @@ static int launch_gemm_t(const rebert_catalog_t* cat, const void* qmat, GemmPara
         const int64_t tiles = (int64_t)p.num_rt * ((p.b + 255) / 256);
         int grid = num_sms() & ~1;
         if (tiles * 2 < grid) grid = (int)(tiles * 2);
-        auto kern = gemm2_kernel<MODE, I8>;
+        auto kern = gemm2_kernel<MODE, I8, QF>;
         { int rc__ = raise_smem_limit(kern); if (rc__ != REBERT_OK) return rc__; }
-        kern<<<grid, GEMM_THREADS, G2_SMEM, st>>>(map_q, map_rows, p);
+        kern<<<grid, GEMM_THREADS, G2_SMEM + extra_smem, st>>>(map_q, map_rows, p);
     } else {
         const int64_t tiles = (int64_t)p.num_rt * p.num_qt;
         int grid = num_sms();
         if (tiles < grid) grid = (int)tiles;
-        auto kern = gemm_kernel<MODE, I8>;
+        auto kern = gemm_kernel<MODE, I8, QF>;
         { int rc__ = raise_smem_limit(kern); if (rc__ != REBERT_OK) return rc__; }
-        kern<<<grid, GEMM_THREADS, GEMM_SMEM, st>>>(map_q, map_rows, p);
+        kern<<<grid, GEMM_THREADS, GEMM_SMEM + extra_smem, st>>>(map_q, map_rows, p);
     }
     REBERT_CUDA(cudaGetLastError());
     return REBERT_OK;
 }
-template <int MODE>
+template <int MODE, bool QF = false>
 static int launch_gemm(const rebert_catalog_t* cat, const void* qmat, GemmParams& p, cudaStream_t st) {
-    return cat->dtype == REBERT_I8 ? launch_gemm_t<MODE, true>(cat, qmat, p, st) : launch_gemm_t<MODE, false>(cat, qmat, p, st);
+    return cat->dtype == REBERT_I8 ? launch_gemm_t<MODE, true, QF>(cat, qmat, p, st) : launch_gemm_t<MODE, false, QF>(cat, qmat, p, st);
 }
 
 // Queries for the int8 operand path: q8[u, c] = rint(qn32[u, c] / step_u), step_u = max|qn32[u, :]| / 127 (1 for an all-zero
@@ -1155,12 +1212,22 @@ REBERT_API int rebert_gemm_scores(const rebert_catalog_t* cat, const void* qbf16
 // from rebert_query_quantize_i8); the exact pass always reads `cat`.
 static int gemm_topk_impl(const rebert_catalog_t* cat, const rebert_catalog_t* op, const void* qbf16, const float* qscale,
                           const double* qeps, const double* q64, const int64_t* excl_row_ptr,
-                          const int32_t* excl_col, const rebert_filter_t* row_filter, const rebert_gemm_plan_t* plan,
-                          void* workspace, size_t workspace_bytes,
+                          const int32_t* excl_col, const rebert_filter_t* row_filter, const rebert_query_filter_t* query_filter,
+                          const rebert_gemm_plan_t* plan, void* workspace, size_t workspace_bytes,
                           int64_t* out_rows, double* out_scores, int32_t* out_count, int32_t* out_status,
                           rebert_stream stream) {
     int rc = check_gemm_catalog(op, "gemm_topk");
     if (rc != REBERT_OK) return rc;
+    QueryFilter qf;
+    memset(&qf, 0, sizeof(qf));
+    if (query_filter) {
+        qf = QueryFilter{query_filter->genre_bits, query_filter->year, query_filter->genre_any, query_filter->year_lo, query_filter->year_hi};
+        REBERT_REQUIRE((qf.genre_any == nullptr) == (qf.genre_bits == nullptr),
+                       "gemm_topk: a per-query genre test needs both genre_any [b] and the catalog's genre_bits [n]");
+        REBERT_REQUIRE((qf.year_lo == nullptr) == (qf.year_hi == nullptr) && (qf.year_lo == nullptr) == (qf.year == nullptr),
+                       "gemm_topk: a per-query year test needs year_lo and year_hi [b] and the catalog's year [n]");
+    }
+    const bool has_qf = qf.genre_any || qf.year_lo;
     REBERT_REQUIRE(cat && cat->rows && (cat->dtype == REBERT_BF16 || cat->dtype == REBERT_F32), "gemm_topk: the catalog of record must be fp32 or bf16");
     REBERT_REQUIRE(qbf16 && q64 && plan && workspace && out_rows && out_scores && out_count && out_status && cat->norm64,
                    "gemm_topk: null argument");
@@ -1203,7 +1270,8 @@ static int gemm_topk_impl(const rebert_catalog_t* cat, const rebert_catalog_t* o
     memset(&pf, 0, sizeof(pf));
     set_pred(pf, cat, row_filter);
     select_threshold_kernel<<<b, 256, tsmem, st>>>(w.sample, keys_in_smem, plan->sample_rows, cat->n, cat->row_base, 0, stride,
-                                                   plan->sample_rank, pf.pred, pf.has_pred, excl_row_ptr, excl_col, w.tau);
+                                                   plan->sample_rank, pf.pred, pf.has_pred, qf, has_qf ? 1 : 0, excl_row_ptr, excl_col,
+                                                   w.tau);
     REBERT_CUDA(cudaGetLastError());
     // 3. full pass with fused filter
     memset(&p, 0, sizeof(p));
@@ -1218,7 +1286,8 @@ static int gemm_topk_impl(const rebert_catalog_t* cat, const rebert_catalog_t* o
     p.status = out_status;
     p.qscale = qscale;
     set_pred(p, cat, row_filter);
-    rc = launch_gemm<MODE_FILTER>(op, qbf16, p, st);
+    p.qf = qf;
+    rc = has_qf ? launch_gemm<MODE_FILTER, true>(op, qbf16, p, st) : launch_gemm<MODE_FILTER>(op, qbf16, p, st);
     if (rc != REBERT_OK) return rc;
     // 4. per-query candidate selection
     if (large) {
@@ -1284,14 +1353,33 @@ REBERT_API int rebert_gemm_scores_i8(const rebert_catalog_t* shadow, const void*
     return launch_gemm<MODE_STORE>(shadow, q8, p, (cudaStream_t)stream);
 }
 
+REBERT_API int rebert_gemm_topk_filtered(const rebert_catalog_t* cat, const void* qbf16, const double* q64, const int64_t* excl_row_ptr,
+                                         const int32_t* excl_col, const rebert_filter_t* row_filter,
+                                         const rebert_query_filter_t* query_filter, const rebert_gemm_plan_t* plan, void* workspace,
+                                         size_t workspace_bytes, int64_t* out_rows, double* out_scores, int32_t* out_count,
+                                         int32_t* out_status, rebert_stream stream) {
+    REBERT_REQUIRE(cat && cat->dtype == REBERT_BF16, "gemm_topk: the bf16 tensor-core path needs a bf16 catalog");
+    return gemm_topk_impl(cat, cat, qbf16, nullptr, nullptr, q64, excl_row_ptr, excl_col, row_filter, query_filter, plan, workspace,
+                          workspace_bytes, out_rows, out_scores, out_count, out_status, stream);
+}
+
 REBERT_API int rebert_gemm_topk(const rebert_catalog_t* cat, const void* qbf16, const double* q64, const int64_t* excl_row_ptr,
                                 const int32_t* excl_col, const rebert_filter_t* row_filter, const rebert_gemm_plan_t* plan,
                                 void* workspace, size_t workspace_bytes,
                                 int64_t* out_rows, double* out_scores, int32_t* out_count, int32_t* out_status,
                                 rebert_stream stream) {
-    REBERT_REQUIRE(cat && cat->dtype == REBERT_BF16, "gemm_topk: the bf16 tensor-core path needs a bf16 catalog");
-    return gemm_topk_impl(cat, cat, qbf16, nullptr, nullptr, q64, excl_row_ptr, excl_col, row_filter, plan, workspace, workspace_bytes,
-                          out_rows, out_scores, out_count, out_status, stream);
+    return rebert_gemm_topk_filtered(cat, qbf16, q64, excl_row_ptr, excl_col, row_filter, nullptr, plan, workspace, workspace_bytes,
+                                     out_rows, out_scores, out_count, out_status, stream);
+}
+
+REBERT_API int rebert_gemm_topk_i8_filtered(const rebert_catalog_t* cat, const rebert_catalog_t* shadow, const void* q8, const float* qscale,
+                                            const double* qeps, const double* q64, const int64_t* excl_row_ptr, const int32_t* excl_col,
+                                            const rebert_filter_t* row_filter, const rebert_query_filter_t* query_filter,
+                                            const rebert_gemm_plan_t* plan, void* workspace, size_t workspace_bytes, int64_t* out_rows,
+                                            double* out_scores, int32_t* out_count, int32_t* out_status, rebert_stream stream) {
+    REBERT_REQUIRE(shadow && shadow->dtype == REBERT_I8, "gemm_topk_i8: shadow must be an int8 prefilter shadow");
+    return gemm_topk_impl(cat, shadow, q8, qscale, qeps, q64, excl_row_ptr, excl_col, row_filter, query_filter, plan, workspace,
+                          workspace_bytes, out_rows, out_scores, out_count, out_status, stream);
 }
 
 REBERT_API int rebert_gemm_topk_i8(const rebert_catalog_t* cat, const rebert_catalog_t* shadow, const void* q8, const float* qscale,
@@ -1299,9 +1387,8 @@ REBERT_API int rebert_gemm_topk_i8(const rebert_catalog_t* cat, const rebert_cat
                                    const rebert_filter_t* row_filter, const rebert_gemm_plan_t* plan, void* workspace,
                                    size_t workspace_bytes, int64_t* out_rows, double* out_scores, int32_t* out_count,
                                    int32_t* out_status, rebert_stream stream) {
-    REBERT_REQUIRE(shadow && shadow->dtype == REBERT_I8, "gemm_topk_i8: shadow must be an int8 prefilter shadow");
-    return gemm_topk_impl(cat, shadow, q8, qscale, qeps, q64, excl_row_ptr, excl_col, row_filter, plan, workspace, workspace_bytes,
-                          out_rows, out_scores, out_count, out_status, stream);
+    return rebert_gemm_topk_i8_filtered(cat, shadow, q8, qscale, qeps, q64, excl_row_ptr, excl_col, row_filter, nullptr, plan, workspace,
+                                        workspace_bytes, out_rows, out_scores, out_count, out_status, stream);
 }
 
 }  // extern "C"

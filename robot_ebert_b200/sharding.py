@@ -21,8 +21,8 @@ import torch
 import torch.distributed as dist
 
 from . import _native as nat
-from .catalog import (EMPTY_PROFILE, CatalogStore, RowFilter, close_proof, large_k_search, sorted_csr, unpack_result,
-                      validated_table, widen_until_proven)
+from .catalog import (EMPTY_PROFILE, CatalogStore, QueryFilters, RowFilter, close_proof, large_k_search, sorted_csr, unpack_result,
+                      user_row_filter, validated_table, widen_until_proven)
 
 log = logging.getLogger("robot_ebert_b200")
 
@@ -470,14 +470,18 @@ class ShardedCatalog:
         return rr, sc
 
     # ------------------------------------------------------------------ batched (tensor-core) path ----------
-    def batch_context(self, qbf: torch.Tensor, qn64: torch.Tensor, k: int, excl_ptr=None, excl_col=None, row_filter=None, qn32=None):
+    def batch_context(self, qbf: torch.Tensor, qn64: torch.Tensor, k: int, excl_ptr=None, excl_col=None, row_filter=None, qn32=None,
+                      query_filters: Optional[QueryFilters] = None):
         """Allocate everything a batched step needs (device tensors only) for prepared queries [b, ld].  With qn32 given and
-        an int8 shadow the GEMM can use (enable_prefilter), the step runs on int8 operands."""
+        an int8 shadow the GEMM can use (enable_prefilter), the step runs on int8 operands.  query_filters: one genre / year
+        test per query, tested against this rank's own metadata (set_metadata on backend.store)."""
         import ctypes as C
         store: CatalogStore = self.backend.store
         lib = nat.load()
         dev = store.device
         b = qbf.shape[0]
+        if query_filters is not None:
+            query_filters.validate(b, row_filter, store.genre_bits, store.year)
         shadow = store.quantize_queries(qn32) if (qn32 is not None and store.batch_shadow_ok) else None
         if shadow is None and not store.batch_gemm_ok:
             raise nat.NativeError(nat.ERR_UNSUPPORTED, f"batch_context: the tcgen05 GEMM takes neither this {store.dtype} shard "
@@ -490,7 +494,7 @@ class ShardedCatalog:
             ec = torch.from_numpy(excl_col).to(dev)
         hb = (b + 1) // 2
         words = 2 * b * k + 2 * hb                                       # rows | scores | counts | status
-        ctx = {"b": b, "k": k, "plan": plan, "row_filter": row_filter, "qbf": qbf, "qn64": qn64, "ep": ep, "ec": ec, "hb": hb, "words": words,
+        ctx = {"b": b, "k": k, "plan": plan, "row_filter": row_filter, "query_filters": query_filters, "qbf": qbf, "qn64": qn64, "ep": ep, "ec": ec, "hb": hb, "words": words,
                "shadow": shadow,
                "ws": torch.empty(lib.rebert_gemm_workspace_bytes(C.byref(store._c), C.byref(plan)), dtype=torch.uint8, device=dev),
                "local": torch.empty(words, dtype=torch.int64, device=dev),
@@ -509,7 +513,7 @@ class ShardedCatalog:
         o_count = local[2 * b * k:2 * b * k + hb].view(torch.int32)
         o_status = local[2 * b * k + hb:].view(torch.int32)
         store.enqueue_batch(ctx["plan"], ctx["qbf"], ctx["qn64"], ctx["ep"], ctx["ec"], ctx["ws"], o_rows, o_scores, o_count, o_status,
-                            ctx.get("row_filter"), shadow=ctx.get("shadow"))
+                            ctx.get("row_filter"), shadow=ctx.get("shadow"), query_filters=ctx.get("query_filters"))
         dist.all_gather_into_tensor(ctx["gathered"].view(-1), local, group=self.group)
         base = ctx["gathered"].data_ptr()
         nat.check(lib.rebert_merge_topk(base, base + 8 * b * k, base + 16 * b * k, words, words, 2 * words, self.world, b, k,
@@ -527,13 +531,13 @@ class ShardedCatalog:
         rows, scores = ctx["m_rows"].cpu().numpy(), ctx["m_scores"].cpu().numpy()
         counts, status = ctx["m_count"].cpu().numpy(), status.cpu().numpy()
         self._rerun(np.nonzero(status)[0], queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, ctx.get("row_filter"),
-                    prefilter, rows, scores, counts)
+                    prefilter, rows, scores, counts, ctx.get("query_filters"))
         return rows, scores, counts, status
 
     def _rerun(self, users, queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, prefilter,
-               rows, scores, counts):
+               rows, scores, counts, query_filters=None):
         """Sharded single-query route (recommend) for `users` of a batch of queries or of a liked CSR with optional weights,
-        each with its segment of the exclusion CSR.  `users` must be the same on every rank (the collectives stay aligned).
+        each with its segment of the exclusion CSR and its own filter (user_row_filter).  `users` must be the same on every rank (the collectives stay aligned).
         Overwrites those users' rows / scores / counts."""
         ecp = None if excl_ptr is None else np.asarray(excl_ptr, dtype=np.int64)
         eca = None if excl_col is None else np.asarray(excl_col)
@@ -542,17 +546,18 @@ class ShardedCatalog:
             lw = None if liked_w is None else np.asarray(liked_w)
         for u in users:
             ex = None if ecp is None else eca[ecp[u]:ecp[u + 1]]
+            rf = user_row_filter(query_filters, u, row_filter)
             if queries is not None:
-                r, sc = self.recommend(query=np.asarray(queries[u]), exclude_rows=ex, k=k, row_filter=row_filter, prefilter=prefilter)
+                r, sc = self.recommend(query=np.asarray(queries[u]), exclude_rows=ex, k=k, row_filter=rf, prefilter=prefilter)
             else:
                 seg = slice(lpn[u], lpn[u + 1])
                 r, sc = self.recommend(liked_rows=lcol[seg], weights=None if lw is None else lw[seg], exclude_rows=ex, k=k,
-                                       row_filter=row_filter, prefilter=prefilter)
+                                       row_filter=rf, prefilter=prefilter)
             rows[u, :], scores[u, :] = -1, -np.inf
             rows[u, :len(r)], scores[u, :len(r)], counts[u] = r, sc, len(r)
 
     def recommend_batch(self, *, queries=None, liked_ptr=None, liked_col=None, liked_w=None, excl_ptr=None, excl_col=None,
-                        k: int = 10, row_filter=None, return_info: bool = False):
+                        k: int = 10, row_filter=None, return_info: bool = False, query_filters: Optional[QueryFilters] = None):
         """Sharded form of CatalogStore.recommend_batch: every rank runs the tcgen05 pass over its rows, the per-rank
         [b, k] results are all-gathered in ONE packed buffer and merged on every rank.  CUDA backend only.
         k up to 2048 runs on the tensor cores when every shard is above the plan minimum (rebert_gemm_plan); the packed buffer
@@ -562,7 +567,7 @@ class ShardedCatalog:
             qn32, qn64, qbf = store.prepare_batch(queries, liked_ptr, liked_col, liked_w,
                                                   reduce_fn=lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM, group=self.group))
             try:
-                ctx = self.batch_context(qbf, qn64, k, excl_ptr, excl_col, row_filter, qn32=qn32)
+                ctx = self.batch_context(qbf, qn64, k, excl_ptr, excl_col, row_filter, qn32=qn32, query_filters=query_filters)
             except nat.NativeError as e:
                 if e.code != nat.ERR_UNSUPPORTED:
                     raise
@@ -570,7 +575,7 @@ class ShardedCatalog:
                                      # verdict on every rank: equal shard sizes, one dtype and width)
             if ctx is None:
                 return self._recommend_batch_loop(queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter,
-                                                  return_info)
+                                                  return_info, query_filters)
             self.batch_step(ctx)
             rows, scores, counts, status = self.batch_collect(ctx, queries, excl_ptr, excl_col, liked_ptr=liked_ptr,
                                                               liked_col=liked_col, liked_w=liked_w, prefilter=None)
@@ -579,13 +584,17 @@ class ShardedCatalog:
             return rows, scores, counts, {"status": status, "plan": {f: getattr(plan, f) for f, _ in plan._fields_}}
         return rows, scores, counts
 
-    def _recommend_batch_loop(self, queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, return_info):
+    def _recommend_batch_loop(self, queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, return_info,
+                              query_filters=None):
         """Small shards: every query of the batch goes through the sharded single-query path (identical on all ranks)."""
         b = len(queries) if queries is not None else len(liked_ptr) - 1
+        if query_filters is not None:
+            query_filters.validate(b, row_filter, self.backend.store.genre_bits, self.backend.store.year)
         rows = np.full((b, k), -1, dtype=np.int64)
         scores = np.full((b, k), -np.inf, dtype=np.float64)
         counts = np.zeros(b, dtype=np.int32)
-        self._rerun(range(b), queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, None, rows, scores, counts)
+        self._rerun(range(b), queries, liked_ptr, liked_col, liked_w, excl_ptr, excl_col, k, row_filter, None, rows, scores, counts,
+                    query_filters)
         if return_info:
             return rows, scores, counts, {"status": np.zeros(b, dtype=np.int32), "plan": None}
         return rows, scores, counts
