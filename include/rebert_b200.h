@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define REBERT_ABI_VERSION 4
+#define REBERT_ABI_VERSION 5
 
 #if defined(__GNUC__)
 #define REBERT_API __attribute__((visibility("default")))
@@ -62,7 +62,16 @@ typedef void* rebert_stream;      /* a cudaStream_t */
 
 /* One HBM-resident catalog shard (replaces the DataFrame at constants.py:55-56).
  * rows is row-major [n, ld]; ld >= d is the padded row stride from rebert_catalog_layout, padding
- * columns are zero.  inv_norm / norm64 follow sklearn's normalize(): zero-norm rows use 1. */
+ * columns are zero.  inv_norm / norm64 follow sklearn's normalize(): zero-norm rows use 1.
+ *
+ * Optional GATE (gate_rows != NULL; a zero-filled struct has none): the int8 rows and factors of
+ * rebert_catalog_quantize_i8 over THESE rows, and its *out_max_err as gate_err.  The single-query fast pass
+ * (rebert_gemv_topk, rebert_recommend_device, rebert_recommend_host) then streams the int8 rows and reads a bf16 / fp32
+ * row only when its int8 score can still reach the candidate list: shadow(r) >= L - delta, L a lower bound of the kc-th
+ * best fast score, delta the per-query bound of DESIGN.md §4.5.  The candidates, and so every result, margin and kc, are
+ * the ones the plain pass produces, bit for bit; only the bytes read change.  Taken for rows of more than 256 bytes in
+ * int8 and in the catalog's own dtype whose int8 layout has a streaming kernel (the others ignore the gate).  The gate
+ * must be rebuilt after ANY write to rows / inv_norm: a stale gate can hide rows. */
 typedef struct {
     const void*   rows;       /* [n, ld] of dtype */
     const float*  inv_norm;   /* [n] fp32 1 / ||row||2 */
@@ -73,6 +82,9 @@ typedef struct {
     int32_t       ld;         /* padded columns (elements) */
     int32_t       dtype;      /* rebert_dtype */
     int32_t       reserved;
+    const void*   gate_rows;  /* [n, ld8] int8 (128-byte aligned), or NULL = no gate */
+    const float*  gate_factor;/* [n] (16-byte aligned) */
+    double        gate_err;   /* max_r ||x_r - dequant(q8_r)|| / ||x_r|| of the gate rows */
 } rebert_catalog_t;
 
 /* Rows that may NOT be returned (lib.py:48,55 `unrated`), plus the optional C5 genre/year predicate.
@@ -193,6 +205,9 @@ REBERT_API size_t  rebert_gemv_workspace_bytes(int64_t n, int32_t kc);
 /* Zero the control words again after a launch that did not run to completion (a fault): they sit at a kc-independent
  * place at the start of the workspace, so one workspace serves every kc. */
 REBERT_API int     rebert_workspace_reset(void* workspace, size_t workspace_bytes, rebert_stream stream);
+/* Diagnostics: rows the gated fast pass has read from the catalog of record on this workspace since it was zero-filled
+ * or reset (a wrapping 32-bit count, summed over launches).  Synchronises the stream. */
+REBERT_API int     rebert_gate_fetches(const void* workspace, size_t workspace_bytes, uint32_t* out_count, rebert_stream stream);
 /* Fast pass.  score(r) = <qn32, row r> * inv_norm[r] in fp32; keeps the kc best allowed rows of the shard.
  * Output: cand_keys[kc] sorted best-first (packed (score, local row) keys; unused slots are 0). */
 REBERT_API int rebert_gemv_topk(const rebert_catalog_t* cat, const float* qn32, const rebert_filter_t* filter, int32_t kc,

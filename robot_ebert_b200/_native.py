@@ -12,7 +12,7 @@ F32, BF16 = 0, 1
 I8 = 2          # prefilter shadow only (rebert_catalog_quantize_i8)
 DTYPES = {"fp32": F32, "bf16": BF16, "i8": I8}
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_WORKSPACE, ERR_CUDA, ERR_DEVICE = 0, -1, -2, -3, -4, -5
 
 
@@ -25,7 +25,7 @@ class NativeError(RuntimeError):
 class Catalog(C.Structure):
     _fields_ = [("rows", C.c_void_p), ("inv_norm", C.c_void_p), ("norm64", C.c_void_p), ("n", C.c_int64),
                 ("row_base", C.c_int64), ("d", C.c_int32), ("ld", C.c_int32), ("dtype", C.c_int32),
-                ("reserved", C.c_int32)]
+                ("reserved", C.c_int32), ("gate_rows", C.c_void_p), ("gate_factor", C.c_void_p), ("gate_err", C.c_double)]
 
 
 class Filter(C.Structure):
@@ -87,6 +87,7 @@ _SIGS = {
     "rebert_recommend_device": (C.c_int, [C.POINTER(Catalog), C.POINTER(Catalog), _P, _P, C.POINTER(Filter), C.c_int32, C.c_int32, _P,
                                           C.c_size_t, _P, C.c_uint32, C.POINTER(Exchange), _P, _P]),
     "rebert_workspace_reset": (C.c_int, [_P, C.c_size_t, _P]),
+    "rebert_gate_fetches": (C.c_int, [_P, C.c_size_t, C.POINTER(C.c_uint32), _P]),
     "rebert_merge_topk": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "rebert_exchange_buffer_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     "rebert_exchange_merge": (C.c_int, [C.POINTER(Exchange), C.c_int32, _P, _P, _P, _P]),

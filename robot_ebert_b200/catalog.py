@@ -359,6 +359,122 @@ class CatalogStore:
         self._plain_proof = nat.Proof()      # read-only, shared by every request that does not try the shadow
         self._plain_proof.fast_eps, self._plain_proof.widen = self.fast_eps, 1
         self._kc_for_k = {}
+        self._gate = None          # (int8 rows, factors) the fast pass streams as its gate (build_gate)
+        self._q8_versions = None   # version counters of rows / inv_norm / norm64 when the int8 rows were last quantized
+        if self.n * self.ld * (esize - 1) >= self.GATE_MIN_SAVED_BYTES and self.build_gate() and not self._gate_pays():
+            self.drop_gate()
+
+    # ------------------------------------------------------------------ int8 gate ---------------
+    # When the gate pays (DESIGN.md §4.5, tools/bench_gate.py on a B200): its cost is the rows it fetches from the catalog of
+    # record, ~4 ns each in aggregate (one L2/HBM round trip of one warp), and ~50k of them before the pruning bounds
+    # settle whatever the size; its gain is the bytes it does not stream, at ~7 TB/s.  A catalog that saves fewer bytes
+    # than GATE_MIN_SAVED_BYTES cannot win; a larger one keeps its gate when a probe request fetches fewer rows than
+    # saved bytes / GATE_BYTES_PER_FETCH (half the break-even), so catalogs whose rows crowd together (text embeddings with
+    # a shared mean direction, where a quarter of the rows pass) keep the plain pass.
+    GATE_MIN_SAVED_BYTES = 2 << 30
+    GATE_BYTES_PER_FETCH = 56_000
+
+    @property
+    def gate_layout_ok(self) -> bool:
+        """True when the gated fast pass takes this catalog's rows: more than 256 bytes per row in int8 and in the catalog's
+        own dtype (32 lanes per row), and an int8 row length with a gated kernel (512 x 1, 2, 3, 4 or 6 bytes; mirrors
+        gate_applies in csrc/gemv_topk.cu)."""
+        ld8, _ = self.layout(max(self.n, 1), self.d, "i8")
+        return self.d > 256 and ld8 % 512 == 0 and ld8 // 512 in (1, 2, 3, 4, 6)
+
+    @property
+    def has_gate(self) -> bool:
+        return self._gate is not None
+
+    def build_gate(self) -> bool:
+        """Give the single-request fast pass an int8 gate of this shard (n x ld8 bytes + one fp32 factor per row): it then
+        streams the int8 rows and reads a row of record only where its int8 score can still reach the candidate list.
+        Results, margins and kc are those of the plain pass, bit for bit (DESIGN.md §4.5).  The constructor builds it when
+        it pays (GATE_MIN_SAVED_BYTES, _gate_pays).  Returns False, leaving the plain pass, when the layout has no gated kernel
+        or the memory is not there."""
+        if self._gate is not None:
+            return True
+        if not self.gate_layout_ok:
+            return False
+        try:
+            rows8, factor = self._int8_buffers()
+        except torch.cuda.OutOfMemoryError:
+            return False
+        self._gate = (rows8, factor)
+        self._c.gate_rows, self._c.gate_factor, self._c.gate_err = rows8.data_ptr(), factor.data_ptr(), self.q8_row_err
+        return True
+
+    def _gate_pays(self) -> bool:
+        """One probe request through the gated pass: a profile-like query (the mean of 64 rows spread over the catalog) with
+        k = 10; True when it fetched few enough rows (GATE_BYTES_PER_FETCH)."""
+        lib = nat.load()
+        with torch.cuda.device(self.device):
+            idx = torch.linspace(0, self.n - 1, 64, device=self.device).long()
+            q = self.rows[idx, :self.d].float().mean(0).cpu().numpy()
+            kc = lib.rebert_candidates_for_k(10)
+            s = self._scratch()
+            s.ensure_out(10, kc)
+            before = self.gate_fetches()
+            excl_ptr, ne = self.stage_inputs(q, None, None, None, 10, kc)
+            self.enqueue_fused(10, kc, excl_ptr, ne)
+            fetched = (self.gate_fetches() - before) & 0xFFFFFFFF
+        self.last_probe_fetches = fetched
+        return fetched * self.GATE_BYTES_PER_FETCH < self.n * self.ld * (self.rows.element_size() - 1)
+
+    def gate_fetches(self) -> int:
+        """Rows the gated pass has read from the catalog of record on this thread's scratch (a wrapping 32-bit count;
+        diagnostics: tools/bench_gate.py, tests)."""
+        s = self._scratch()
+        if not s.kc:
+            return 0
+        out = C.c_uint32(0)
+        nat.check(nat.load().rebert_gate_fetches(s.ws.data_ptr(), s.ws.numel(), C.byref(out), torch.cuda.current_stream().cuda_stream))
+        return out.value
+
+    def drop_gate(self) -> None:
+        """Back to the plain fast pass (the int8 rows stay allocated while the prefilter shadow uses them)."""
+        self._gate = None
+        self._c.gate_rows, self._c.gate_factor, self._c.gate_err = None, None, 0.0
+
+    def _int8_buffers(self):
+        """The int8 rows + factors of this shard: the gate's or the prefilter shadow's when one exists (one copy serves
+        both), else newly quantized."""
+        if self._gate is not None:
+            return self._gate
+        if self._c8 is not None:
+            return self._q8_rows, self._q8_factor
+        ld8, _ = self.layout(self.n, self.d, "i8")
+        rows8 = torch.empty((max(self.n, 1), ld8), dtype=torch.int8, device=self.device)
+        factor = torch.empty(_align(max(self.n, 1), 4), dtype=torch.float32, device=self.device)
+        self._quantize_into(rows8, factor)
+        return rows8, factor
+
+    def _row_versions(self):
+        return self.rows._version, self.inv_norm._version, self.norm64._version
+
+    def _quantize_into(self, rows8: torch.Tensor, factor: torch.Tensor) -> None:
+        lib = nat.load()
+        with torch.cuda.device(self.device):
+            max_err = torch.zeros(1, dtype=torch.float64, device=self.device)
+            nat.check(lib.rebert_catalog_quantize_i8(C.byref(self._c), rows8.data_ptr(), rows8.shape[1], factor.data_ptr(),
+                                                     max_err.data_ptr(), torch.cuda.current_stream().cuda_stream))
+            self.q8_row_err = float(max_err.item())
+        self._q8_versions = self._row_versions()
+
+    def _fresh_int8(self) -> None:
+        """Re-quantize the int8 rows (gate and prefilter shadow) if rows / inv_norm / norm64 were written since they were
+        built: a stale gate could hide a row that now belongs to the result.  About 24 ms at 10M x 1536."""
+        if self._q8_versions is None or self._q8_versions == self._row_versions():
+            return
+        if self._gate is None and self._c8 is None:     # both given up: nothing left to refresh
+            self._q8_versions = None
+            return
+        rows8, factor = self._gate if self._gate is not None else (self._q8_rows, self._q8_factor)
+        self._quantize_into(rows8, factor)
+        if self._gate is not None:
+            self._c.gate_err = self.q8_row_err
+        if self._c8 is not None:
+            self.q8_eps = self._shadow_eps(self.q8_row_err)
 
     # ------------------------------------------------------------------ construction -----------
     @staticmethod
@@ -434,24 +550,19 @@ class CatalogStore:
         int8 query planes.  A request whose proof margin does not clear that bound silently takes the standard path, so
         results never depend on the shadow.  The streaming kernel has no int8 variant for rows of 5 or 7-11 chunks per lane
         (d = 2049-2560 and 3073-5632, d = 4096 among them): there single requests always take the standard path, and the
-        shadow serves only the batched int8 GEMM."""
-        lib = nat.load()
-        ld8, _ = self.layout(self.n, self.d, "i8")
-        with torch.cuda.device(self.device):
-            rows8 = torch.empty((max(self.n, 1), ld8), dtype=torch.int8, device=self.device)
-            factor = torch.empty(_align(max(self.n, 1), 4), dtype=torch.float32, device=self.device)
-            max_err = torch.zeros(1, dtype=torch.float64, device=self.device)
-            nat.check(lib.rebert_catalog_quantize_i8(C.byref(self._c), rows8.data_ptr(), ld8, factor.data_ptr(), max_err.data_ptr(),
-                                                     torch.cuda.current_stream().cuda_stream))
-            row_err = float(max_err.item())
+        shadow serves only the batched int8 GEMM.  With a gate (build_gate) the shadow is the gate's int8 rows."""
+        self._fresh_int8()
+        rows8, factor = self._int8_buffers()
         self._q8_rows, self._q8_factor = rows8, factor
         self._c8 = nat.Catalog(rows=rows8.data_ptr(), inv_norm=factor.data_ptr(), norm64=self.norm64.data_ptr(), n=self.n,
-                               row_base=self.row_base, d=self.d, ld=ld8, dtype=nat.DTYPES["i8"], reserved=0)
+                               row_base=self.row_base, d=self.d, ld=rows8.shape[1], dtype=nat.DTYPES["i8"], reserved=0)
+        self.q8_eps = self._shadow_eps(self.q8_row_err)
+        return self.q8_eps
+
+    def _shadow_eps(self, row_err: float) -> float:
         # query planes: |q - (dh*hi + dl*lo)| <= dl/2 per element with dl = max|q| / (127*254) <= 1 / (127*254) for ||q|| <= 1
         query_err = float(np.sqrt(self.d)) / (127.0 * 254.0 * 2.0)
-        self.q8_row_err = row_err
-        self.q8_eps = row_err + 1.01 * (1.0 + row_err) * query_err + 4e-6      # + fp32 rounding of factor / int->float / final products
-        return self.q8_eps
+        return row_err + 1.01 * (1.0 + row_err) * query_err + 4e-6      # + fp32 rounding of factor / int->float / final products
 
     def set_metadata(self, genre_bits: np.ndarray, year: np.ndarray) -> None:
         """Per-row side columns for the genre/year predicate (local row order)."""
@@ -602,6 +713,7 @@ class CatalogStore:
         instead of the calling thread's own (the sharding layer pre-allocates one per exchange channel).
         Returns (rows, scores, info)."""
         lib = nat.load()
+        self._fresh_int8()
         d = self.d
         q = lk = w = ex = None
         nl = ne = 0
@@ -752,6 +864,7 @@ class CatalogStore:
         profile already sitting in this thread's scratch (qn32, qn64).  Result lands packed in scratch.d_out.
         Nothing is copied and nothing synchronises."""
         lib = nat.load()
+        self._fresh_int8()
         s = self._scratch()
         s.ensure_out(k, kc)
         st = torch.cuda.current_stream().cuda_stream
@@ -772,6 +885,7 @@ class CatalogStore:
         ranking in the tail of the same kernel (+ the NVLink exchange and merge when `exchange` is given), for the query /
         profile already sitting in this thread's scratch.  Result lands packed in scratch.d_out (or at out_ptr)."""
         lib = nat.load()
+        self._fresh_int8()
         s = self._scratch()
         s.ensure_out(k, kc)
         f = self._filter_struct(row_filter) or nat.Filter()
@@ -878,6 +992,8 @@ class CatalogStore:
         from gemm_plan(shadow=True)); the exact pass reads the catalog of record either way.
         query_filters: one genre / year test per query (QueryFilters), applied inside the threshold sample and the GEMM epilogue."""
         lib = nat.load()
+        if shadow is not None:
+            self._fresh_int8()
         if query_filters is not None:
             query_filters.validate(plan.b, row_filter, self.genre_bits, self.year)
         f = self._filter_struct(row_filter)

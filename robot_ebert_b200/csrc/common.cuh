@@ -72,6 +72,10 @@ __host__ __device__ __forceinline__ uint64_t make_key(float score, uint32_t row)
 __host__ __device__ __forceinline__ float key_score(uint64_t k) { return orderable_f32((uint32_t)(k >> 32)); }
 __host__ __device__ __forceinline__ uint32_t key_row(uint64_t k) { return 0xFFFFFFFFu - (uint32_t)k; }
 
+// Control word 3 of a streaming workspace: rows the gated fast pass fetched from the catalog of record, summed over
+// launches.  The merge that zeroes the other control words after every launch leaves it alone (rebert_gate_fetches).
+constexpr int kCtlGateFetches = 3;
+
 // ---------------------------------------------------------------- debug build ---------------
 // -DREBERT_DEBUG (robot_ebert_b200/build.py --debug -> librebert_b200_debug.so, loaded when REBERT_DEBUG=1) turns on
 // device-side bounds assertions at every computed index the kernels write through; compute-sanitizer is not available on

@@ -61,6 +61,11 @@ struct GemvParams {
     int64_t      static_rounds;  // every CTA takes tiles blockIdx.x + i * grid for i < static_rounds, the rest are claimed
     int          merge_cap; // keys the final merge may hold in shared memory (power of two)
     int          publish_only;  // request path: no ticket, no merge here — the cluster kernel behind this launch takes over
+    // gated kernel only (rows / inv_norm above are the int8 gate): the catalog of record a gated row is fetched from
+    const void*  xrows;     // [n, x_ld] bf16 / fp32
+    const float* xinv;      // [n] its inv_norm
+    int          x_ld, x_cpl;   // its padded row length and chunks per lane (32-lane layout)
+    double       gate_err;  // max relative row error of the int8 gate rows (rebert_catalog_quantize_i8)
 };
 
 template <typename T> struct Elem;
@@ -99,6 +104,72 @@ template <> struct Elem<int8_t> {
         hi = __dp4a((int)v.w, (int)q[3], hi); lo = __dp4a((int)v.w, (int)q[7], lo);
     }
 };
+
+// The fast score of one row, the same arithmetic wherever it is formed (the plain kernels and the gated kernel's fetch):
+// lane cl holds the row's chunks j * LANES + cl; chunk j accumulates into a0 (j even) or a1 (j odd) in element order
+// with fmaf; then a0 + a1, the xor-shuffle tree over the row's LANES lanes, and the caller's multiply by inv_norm.
+template <typename T>
+__device__ __forceinline__ void chunk_dot(const uint4& v, const float* q, int j, float& a0, float& a1) {
+    if (j & 1) Elem<T>::dot(v, q, a1);
+    else       Elem<T>::dot(v, q, a0);
+}
+template <int LANES>
+__device__ __forceinline__ float row_sum(float a0, float a1) {
+    float s = a0 + a1;
+#pragma unroll
+    for (int o = LANES / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    return s;
+}
+
+// Gated kernel: <q, row> of one row of record (32-lane layout, cpl chunks per lane) read straight from global memory,
+// the query from shared memory.  Every lane returns the full sum.  Up to 12 chunks per lane are in flight at once.
+template <typename TX>
+__device__ __forceinline__ float fetch_row_dot(const uint4* __restrict__ row, const float* q_smem, int cpl, int lane) {
+    constexpr int EPC = Elem<TX>::EPC;
+    constexpr int kBatch = 12;
+    float a0 = 0.f, a1 = 0.f;
+    for (int j0 = 0; j0 < cpl; j0 += kBatch) {
+        uint4 v[kBatch];
+#pragma unroll
+        for (int u = 0; u < kBatch; ++u)
+            if (j0 + u < cpl) v[u] = __ldg(row + (j0 + u) * 32 + lane);
+#pragma unroll
+        for (int u = 0; u < kBatch; ++u) {
+            if (j0 + u < cpl) {
+                const int j = j0 + u;
+                float qq[EPC];
+                const float4* qs = (const float4*)(q_smem + (j * 32 + lane) * EPC);
+#pragma unroll
+                for (int e = 0; e < EPC / 4; ++e) {
+                    const float4 f = qs[e];
+                    qq[e * 4 + 0] = f.x; qq[e * 4 + 1] = f.y; qq[e * 4 + 2] = f.z; qq[e * 4 + 3] = f.w;
+                }
+                chunk_dot<TX>(v[u], qq, j, a0, a1);
+            }
+        }
+    }
+    return row_sum<32>(a0, a1);
+}
+
+// One element of the int8 query planes: qv ~ dh * h + dl * l (the consumers' registers and the gate's delta use this).
+__device__ __forceinline__ void quant_planes(float qv, float dh, float dl, int& h, int& l) {
+    h = __float2int_rn(qv / dh);
+    h = max(-127, min(127, h));
+    l = __float2int_rn((qv - (float)h * dh) / dl);
+    l = max(-127, min(127, l));
+}
+
+// The gate's delta for the query actually passed (DESIGN.md §4.5), rounded up to fp32.  With S the int8 score, F the
+// fp32 fast score and T = <x, q> / ||x||:
+//   |S - T| <= row_err (||q|| + e_q) + e_q      (rows: Cauchy-Schwarz against the planes q~; query: e_q = ||q - q~||)
+//   |F - T| <= (elements per lane + 12) 2^-24 ||q||      (CatalogStore.fast_eps, scaled by ||q||)
+// plus 32 ulp of (||q|| + e_q)(1 + row_err) for S's own fp32 steps, and 1e-6 ||q|| for forming L - delta in fp32.
+__device__ __forceinline__ float gate_delta(double q2, double e2, double row_err, int x_epl) {
+    const double qn = sqrt(q2), eq = sqrt(e2);
+    const double shadow = row_err * (qn + eq) + eq + 32.0 * 0x1p-24 * (1.0 + row_err) * (qn + eq);
+    const double fast = (double)(x_epl + 12) * 0x1p-24 * qn;
+    return __double2float_ru((shadow + fast) * (1.0 + 1e-6) + 1e-6 * qn + 1e-30);
+}
 
 // Warp-distributed sorted list of M*32 keys: entry e = m*32 + lane, best first.
 template <int M>
@@ -149,12 +220,17 @@ __device__ __forceinline__ void publish_hints(uint64_t key0, float thr, int warp
     }
 }
 
-template <typename T, int CPL, int LANES, int M>
+// TX = void: the plain kernel (T = the streamed rows' type).  TX = bf16 / float: the GATED kernel — T = int8_t streams the
+// catalog's int8 gate, and a row whose int8 score reaches L - delta (L = the warp's pruning bound) is read from the bf16 /
+// fp32 catalog of record and scored with the plain kernel's arithmetic, so the keys are the plain kernel's (DESIGN §4.5).
+template <typename T, int CPL, int LANES, int M, typename TX = void>
 __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams p) {
     constexpr int EPC = Elem<T>::EPC;
     constexpr int RPW = 32 / LANES;              // rows a warp scores at once
     constexpr bool kRegQ = CPL > 0;              // query chunks live in registers
     constexpr bool kI8 = std::is_same<T, int8_t>::value;   // int8 prefilter shadow (register-query variants only)
+    constexpr bool kGate = !std::is_void<TX>::value;
+    static_assert(!kGate || (kI8 && kRegQ && LANES == 32), "the gated kernel streams 32-lane int8 rows");
     constexpr int QREGS = (kRegQ && !kI8) ? CPL * EPC : 1;
     constexpr int QIREGS = kI8 ? CPL * 8 : 1;    // per chunk: 4 words of the hi plane + 4 of the lo plane
     constexpr int kQuantLane = 4 * M - 1;        // list entry kc/8 - 1 lives in keys[0] of this lane (kc = 32 M)
@@ -167,8 +243,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     unsigned char* stage_base = smem;
     uint64_t* full_bar = (uint64_t*)(smem + (size_t)p.stages * stage_stride);
     uint64_t* empty_bar = full_bar + kStages;
-    float* q_smem = (float*)(empty_bar + kStages);               // generic kernel only: [ld]
-    int32_t* excl_smem = (int32_t*)(q_smem + (kRegQ ? 0 : p.ld));
+    float* q_smem = (float*)(empty_bar + kStages);               // generic kernel: [ld]; gated kernel: [x_ld]
+    int32_t* excl_smem = (int32_t*)(q_smem + (kGate ? p.x_ld : (kRegQ ? 0 : p.ld)));
     const bool excl_staged = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem;
     const int32_t* excl_s = excl_staged ? excl_smem : nullptr;
 
@@ -213,8 +289,9 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         }
     }
     pdl_wait();
-    if (!kRegQ) {
-        for (int c = threadIdx.x; c < p.ld; c += blockDim.x) q_smem[c] = p.q[c];
+    if (!kRegQ || kGate) {
+        const int qlen = kGate ? p.x_ld : p.ld;
+        for (int c = threadIdx.x; c < qlen; c += blockDim.x) q_smem[c] = p.q[c];
     }
     if (excl_staged) {
         for (int c = threadIdx.x; c < p.filter.n_exclude; c += blockDim.x) excl_smem[c] = __ldg(p.filter.exclude_rows + c);
@@ -239,6 +316,35 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     // It is recomputed only by a warp that has just inserted (the rare path); the per-tile cost stays one shared load.
     __shared__ unsigned s_hint;
     __shared__ unsigned s_wq[kConsumerWarps];   // orderable score of warp w's (kc/8)-th best key, 0 = not there yet
+    __shared__ float s_delta;
+    if constexpr (kGate) {
+        // delta from the query's own norm and the real error of its two int8 planes (the consumers form the same planes)
+        __shared__ double s_red[2][kConsumerWarps + 1];
+        __syncthreads();
+        float qmax = 0.f;
+#pragma unroll
+        for (int w = 0; w <= kConsumerWarps; ++w) qmax = fmaxf(qmax, s_qmax[w]);
+        const float gdh = qmax > 0.f ? qmax / 127.f : 1.f;
+        const float gdl = gdh / 254.f;
+        double e2 = 0.0, q2 = 0.0;
+        for (int c = threadIdx.x; c < p.d; c += blockDim.x) {
+            const float qv = __ldg(p.q + c);
+            int h, l;
+            quant_planes(qv, gdh, gdl, h, l);
+            const double r = (double)qv - ((double)gdh * h + (double)gdl * l);
+            e2 = fma(r, r, e2);
+            q2 = fma((double)qv, (double)qv, q2);
+        }
+        e2 = warp_sum(e2);
+        q2 = warp_sum(q2);
+        if (lane == 0) { s_red[0][warp] = e2; s_red[1][warp] = q2; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double se = 0.0, sq = 0.0;
+            for (int w = 0; w <= kConsumerWarps; ++w) { se += s_red[0][w]; sq += s_red[1][w]; }
+            s_delta = gate_delta(sq, se, p.gate_err, p.x_cpl * Elem<TX>::EPC);
+        }
+    }
     if (threadIdx.x == 0) s_hint = 0u;
     if (threadIdx.x < kConsumerWarps) s_wq[threadIdx.x] = 0u;
     __syncthreads();
@@ -309,10 +415,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                     for (int b = 0; b < 4; ++b) {
                         const int idx = (j * LANES + cl) * 16 + w * 4 + b;
                         const float qv = idx < p.d ? __ldg(p.q + idx) : 0.f;
-                        int h = __float2int_rn(qv / dh);
-                        h = max(-127, min(127, h));
-                        int l = __float2int_rn((qv - (float)h * dh) / dl);
-                        l = max(-127, min(127, l));
+                        int h, l;
+                        quant_planes(qv, dh, dl, h, l);
                         ph |= (uint32_t)(h & 0xFF) << (8 * b);
                         pl |= (uint32_t)(l & 0xFF) << (8 * b);
                     }
@@ -328,6 +432,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         }
         const int cpl = kRegQ ? CPL : p.cpl;
         const int row_chunks = cpl * LANES;
+        const float delta = kGate ? s_delta : 0.f;
+        unsigned fetched = 0;                    // gated kernel: rows read from the catalog of record (warp-uniform)
 
         for (int it = 0;; ++it) {
             const int s = it % p.stages;
@@ -387,6 +493,26 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                     for (int u = 0; u < 4; ++u) {          // u ascending = rows ascending, which WarpTopK::insert relies on
                         const float inv = vv[u] ? (rr[u] < nrows4 ? inv_s[rr[u]] : __ldg(p.inv_norm + row0 + rr[u])) : 0.f;
                         const float sc_lane = fmaf(dh, (float)hs[u], dl * (float)ls[u]) * inv;
+                        if constexpr (kGate) {
+                            // a row of the final list has F >= L, so S >= L - delta: rows below cannot get there
+                            unsigned mm = __ballot_sync(0xffffffffu, vv[u] && cl == 0 && sc_lane >= fmaxf(top.thr, hint) - delta);
+                            while (mm) {
+                                const int src = __ffs(mm) - 1;
+                                mm &= mm - 1;
+                                const float sv = __shfl_sync(0xffffffffu, sc_lane, src);
+                                const uint32_t lr = (uint32_t)(row0 + base + u * kConsumerWarps * RPW + src / LANES);
+                                if (sv >= fmaxf(top.thr, hint) - delta && row_allowed(p.filter, lr, excl_s)) {
+                                    ++fetched;
+                                    const uint4* xr = (const uint4*)((const TX*)p.xrows + (size_t)lr * p.x_ld);
+                                    const float sc = fetch_row_dot<TX>(xr, q_smem, p.x_cpl, lane) * __ldg(p.xinv + lr);
+                                    if (sc > top.thr && sc >= hint) {
+                                        top.insert(make_key(sc, lr), lane);
+                                        publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
+                                    }
+                                }
+                            }
+                            continue;
+                        }
                         unsigned mm = __ballot_sync(0xffffffffu, vv[u] && cl == 0 && sc_lane > top.thr && sc_lane >= hint);
                         while (mm) {
                             const int src = __ffs(mm) - 1;
@@ -417,8 +543,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                     for (int j = 0; j < (kRegQ ? CPL : 0); ++j) {
                         const uint4 va = pa[j * LANES];
                         const uint4 vb = pb[j * LANES];
-                        if (j & 1) { Elem<T>::dot(va, q + j * EPC, a1); Elem<T>::dot(vb, q + j * EPC, b1); }
-                        else       { Elem<T>::dot(va, q + j * EPC, a0); Elem<T>::dot(vb, q + j * EPC, b0); }
+                        chunk_dot<T>(va, q + j * EPC, j, a0, a1);
+                        chunk_dot<T>(vb, q + j * EPC, j, b0, b1);
                     }
                 } else {
                     for (int j = 0; j < cpl; ++j) {
@@ -431,16 +557,11 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                             float4 f = qs[e];
                             qq[e * 4 + 0] = f.x; qq[e * 4 + 1] = f.y; qq[e * 4 + 2] = f.z; qq[e * 4 + 3] = f.w;
                         }
-                        if (j & 1) { Elem<T>::dot(va, qq, a1); Elem<T>::dot(vb, qq, b1); }
-                        else       { Elem<T>::dot(va, qq, a0); Elem<T>::dot(vb, qq, b0); }
+                        chunk_dot<T>(va, qq, j, a0, a1);
+                        chunk_dot<T>(vb, qq, j, b0, b1);
                     }
                 }
-                float sa = a0 + a1, sb = b0 + b1;
-#pragma unroll
-                for (int o = LANES / 2; o > 0; o >>= 1) {
-                    sa += __shfl_xor_sync(0xffffffffu, sa, o);
-                    sb += __shfl_xor_sync(0xffffffffu, sb, o);
-                }
+                float sa = row_sum<LANES>(a0, a1), sb = row_sum<LANES>(b0, b1);
                 const float ia = vA ? (rA < nrows4 ? inv_s[rA] : __ldg(p.inv_norm + row0 + rA)) : 0.f;
                 const float ib = vB ? (rB < nrows4 ? inv_s[rB] : __ldg(p.inv_norm + row0 + rB)) : 0.f;
                 sa *= ia;
@@ -475,6 +596,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
             __syncwarp();
             if (lane == 0) mbar_arrive(&empty_bar[s]);
         }
+        if (kGate && lane == 0 && fetched) atomicAdd(p.counter + kCtlGateFetches, fetched);
     }
 
     // ===================== CTA merge: 8 sorted warp lists -> one sorted list of kc keys =====================
@@ -547,7 +669,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         select_winners<16>(pub, p.merge_cap, (uint64_t*)smem, p.cand_keys);
         __syncthreads();
     }
-    if (threadIdx.x < 32) p.counter[threadIdx.x] = 0u;       // ticket, hint, tile-claim counter, compaction cursors
+    if (threadIdx.x < 32 && threadIdx.x != kCtlGateFetches) p.counter[threadIdx.x] = 0u;   // ticket, hint, tile claims, cursors
 }
 
 // ---------------------------------------------------------------- host side ----------------------------------
@@ -558,7 +680,8 @@ struct GemvLaunch {
     size_t smem;
 };
 
-static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, bool generic, int n_exclude) {
+// q_floats: query elements staged in shared memory (generic kernel: ld; gated kernel: the catalog of record's ld)
+static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, int q_floats, int n_exclude) {
     GemvLaunch g;
     const int row_bytes = L.ld * L.esize;
     const int rpw = 32 / L.lanes;
@@ -575,7 +698,7 @@ static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, bool generic,
     const int tile_bytes = tr * row_bytes;
     const int stage_stride = tile_bytes + ((tr * 4 + 127) & ~127);
     const size_t excl_bytes = (n_exclude > 0 && n_exclude <= kMaxExclSmem) ? (size_t)n_exclude * 4 : 0;
-    const size_t fixed = 2 * kStages * sizeof(uint64_t) + (generic ? (size_t)L.ld * 4 : 0) + excl_bytes + 128;
+    const size_t fixed = 2 * kStages * sizeof(uint64_t) + (size_t)q_floats * 4 + excl_bytes + 128;
     int stages = kStages;
     while (stages > 1 && (size_t)stages * stage_stride + fixed > 220 * 1024) --stages;
     g.stages = stages;
@@ -597,11 +720,11 @@ static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, bool generic,
     return g;
 }
 
-template <typename T, int CPL, int LANES>
+template <typename T, int CPL, int LANES, typename TX = void>
 static int launch_gemv_m(const GemvParams& p, const GemvLaunch& g, int kc, cudaStream_t st) {
 #define REBERT_LAUNCH_M(MM)                                                                                      \
     {                                                                                                            \
-        auto kern = gemv_topk_kernel<T, CPL, LANES, MM>;                                                         \
+        auto kern = gemv_topk_kernel<T, CPL, LANES, MM, TX>;                                                         \
         { int rc__ = raise_smem_limit(kern); if (rc__ != REBERT_OK) return rc__; }       \
         REBERT_CUDA(launch_pdl(kern, dim3(g.grid), dim3(kThreads), g.smem, st, p));                             \
     }
@@ -674,6 +797,29 @@ static bool use_generic(const RowLayout& L) {
     return true;
 }
 
+// Gated kernels: the int8 gate streamed by its 32-lane register-query layout, rows of record fetched by 32 lanes.
+template <typename TX>
+static int launch_gemv_gated(const RowLayout& L8, const GemvParams& p, const GemvLaunch& g, int kc, cudaStream_t st) {
+    switch (L8.cpl) {
+        case 1: return launch_gemv_m<int8_t, 1, 32, TX>(p, g, kc, st);
+        case 2: return launch_gemv_m<int8_t, 2, 32, TX>(p, g, kc, st);
+        case 3: return launch_gemv_m<int8_t, 3, 32, TX>(p, g, kc, st);
+        case 4: return launch_gemv_m<int8_t, 4, 32, TX>(p, g, kc, st);
+        case 6: return launch_gemv_m<int8_t, 6, 32, TX>(p, g, kc, st);
+    }
+    set_error("gemv_topk: no gated kernel for int8 rows of %d chunks per lane", L8.cpl);
+    return REBERT_ERR_UNSUPPORTED;
+}
+
+// The catalog's gate is taken when both its int8 rows and its rows of record are 32-lane layouts and the int8 rows have a
+// register-query kernel of at most 6 chunks per lane (d <= 3072; at 12 the gated kernel spills); any other catalog streams
+// its own rows (the gate changes which rows are read, never the result).
+static bool gate_applies(const rebert_catalog_t* cat) {
+    if (cat->dtype == REBERT_I8 || !cat->gate_rows || !cat->gate_factor) return false;
+    const RowLayout L8 = row_layout(cat->d, REBERT_I8), L = row_layout(cat->d, cat->dtype);
+    return L8.lanes == 32 && L.lanes == 32 && !use_generic(L8) && L8.cpl <= 6;
+}
+
 // The int8 shadow has register-query kernels only (launch_gemv_i8): rows of 5 or 7-11 chunks per lane (d = 2049-2560,
 // 3073-5632) have none, and such a shadow serves only the batched int8 GEMM.
 bool gemv_streams(const rebert_catalog_t* cat) {
@@ -715,6 +861,14 @@ REBERT_API int rebert_workspace_reset(void* workspace, size_t workspace_bytes, r
     return REBERT_OK;
 }
 
+REBERT_API int rebert_gate_fetches(const void* workspace, size_t workspace_bytes, uint32_t* out_count, rebert_stream stream) {
+    REBERT_REQUIRE(workspace && out_count && workspace_bytes >= 128 + kWsCtl, "gate_fetches: bad arguments");
+    const unsigned* ctl = (const unsigned*)(((uintptr_t)workspace + 127) & ~(uintptr_t)127);
+    REBERT_CUDA(cudaMemcpyAsync(out_count, ctl + kCtlGateFetches, sizeof(uint32_t), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    REBERT_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
+    return REBERT_OK;
+}
+
 }  // extern "C"
 
 namespace rebert {
@@ -752,18 +906,29 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
         }
         // an empty shard still has to answer (and, on a row shard, to take part in the exchange): run one empty tile
     }
-    const bool generic = use_generic(L);
+    const bool gated = gate_applies(cat);
+    const RowLayout LS = gated ? row_layout(cat->d, REBERT_I8) : L;     // layout of the rows the kernel streams
+    if (gated)
+        REBERT_REQUIRE(((uintptr_t)cat->gate_rows & 127) == 0 && ((uintptr_t)cat->gate_factor & 15) == 0,
+                       "gemv_topk: gate rows must be 128-byte and gate factors 16-byte aligned");
     const int n_excl = (filter && filter->exclude_rows && filter->n_exclude > 0) ? filter->n_exclude : 0;
-    GemvLaunch g = plan_gemv(L, cat->n, kc, generic, n_excl);
+    GemvLaunch g = plan_gemv(LS, cat->n, kc, gated ? L.ld : (use_generic(L) ? L.ld : 0), n_excl);
     GemvParams p;
     memset(&p, 0, sizeof(p));
-    p.rows = cat->rows;
-    p.inv_norm = cat->inv_norm;
+    p.rows = gated ? cat->gate_rows : cat->rows;
+    p.inv_norm = gated ? cat->gate_factor : cat->inv_norm;
     p.q = qn32;
     p.n = cat->n;
-    p.ld = L.ld;
+    p.ld = LS.ld;
     p.d = cat->d;
-    p.cpl = L.cpl;
+    p.cpl = LS.cpl;
+    if (gated) {
+        p.xrows = cat->rows;
+        p.xinv = cat->inv_norm;
+        p.x_ld = L.ld;
+        p.x_cpl = L.cpl;
+        p.gate_err = cat->gate_err;
+    }
     p.tile_rows = g.tile_rows;
     p.num_tiles = (cat->n + g.tile_rows - 1) / g.tile_rows;
     p.stages = g.stages;
@@ -795,6 +960,7 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
 
     int rc;
     if (cat->dtype == REBERT_I8) rc = launch_gemv_i8(L, p, g, st);
+    else if (gated) rc = cat->dtype == REBERT_F32 ? launch_gemv_gated<float>(LS, p, g, kc, st) : launch_gemv_gated<__nv_bfloat16>(LS, p, g, kc, st);
     else rc = cat->dtype == REBERT_F32 ? launch_gemv<float>(L, p, g, kc, st) : launch_gemv<__nv_bfloat16>(L, p, g, kc, st);
     if (rc != REBERT_OK || !fused) return rc;
     // request path: the cluster kernel that selects the winners, runs the exact pass, ranks, writes the result (and exchanges)
