@@ -365,9 +365,9 @@ class CatalogStore:
             self.drop_gate()
 
     # ------------------------------------------------------------------ int8 gate ---------------
-    # When the gate pays (DESIGN.md §4.5, tools/bench_gate.py on a B200): its cost is the rows it fetches from the catalog of
-    # record, ~4 ns each in aggregate (one L2/HBM round trip of one warp), and ~50k of them before the pruning bounds
-    # settle whatever the size; its gain is the bytes it does not stream, at ~7 TB/s.  A catalog that saves fewer bytes
+    # When the gate pays (DESIGN.md §4.5, tools/bench_gate.py on a B200 at 1000 W): its cost is the rows it fetches from the
+    # catalog of record, ~2 ns each in aggregate (one L2/HBM round trip of one warp; 8k per request at 10M synthetic rows
+    # once the seed kernel has set the bound, 87k without it); its gain is the bytes it does not stream, at ~7 TB/s.  A catalog that saves fewer bytes
     # than GATE_MIN_SAVED_BYTES cannot win; a larger one keeps its gate when a probe request fetches fewer rows than
     # saved bytes / GATE_BYTES_PER_FETCH (half the break-even), so catalogs whose rows crowd together (text embeddings with
     # a shared mean direction, where a quarter of the rows pass) keep the plain pass.

@@ -75,6 +75,11 @@ __host__ __device__ __forceinline__ uint32_t key_row(uint64_t k) { return 0xFFFF
 // Control word 3 of a streaming workspace: rows the gated fast pass fetched from the catalog of record, summed over
 // launches.  The merge that zeroes the other control words after every launch leaves it alone (rebert_gate_fetches).
 constexpr int kCtlGateFetches = 3;
+// Control words 20 and 21: the ticket of the gate's seed kernel (its last CTA resets it), and the bound that kernel wrote
+// into the grid-wide hint at the last gated launch (orderable fp32 bits, 0 = none).  The merges leave word 21 alone too, so
+// it can be read after the request (tests/test_gpu_gate_seed.py).
+constexpr int kCtlSeedTicket = 20, kCtlSeedBound = 21;
+__host__ __device__ __forceinline__ bool ctl_survives_merge(int w) { return w == kCtlGateFetches || w == kCtlSeedBound; }
 
 // ---------------------------------------------------------------- debug build ---------------
 // -DREBERT_DEBUG (robot_ebert_b200/build.py --debug -> librebert_b200_debug.so, loaded when REBERT_DEBUG=1) turns on

@@ -296,7 +296,7 @@ __global__ void __launch_bounds__(kFinalClusterThreads, 2) finalize_published_ke
         exchange_results(p.xchg, k, s_block, p.out_packed, s_all);
         pdl_trigger();
     }
-    if (threadIdx.x < 32 && threadIdx.x != kCtlGateFetches) p.pub.ctl[threadIdx.x] = 0u;   // ticket, hint, tile claims, cursors
+    if (threadIdx.x < 32 && !ctl_survives_merge(threadIdx.x)) p.pub.ctl[threadIdx.x] = 0u;   // ticket, hint, tile claims, cursors
     if (p.done_flag) {
         __syncthreads();                                     // every thread's result stores are ordered before the flag
         if (threadIdx.x == 0) {

@@ -66,6 +66,10 @@ struct GemvParams {
     const float* xinv;      // [n] its inv_norm
     int          x_ld, x_cpl;   // its padded row length and chunks per lane (32-lane layout)
     double       gate_err;  // max relative row error of the int8 gate rows (rebert_catalog_quantize_i8)
+    // gate_seed_kernel only: rows i * seed_stride (i < seed_m) are sampled; every CTA publishes its seed_P best into seed_keys
+    int64_t      seed_m, seed_stride;
+    int          seed_P;
+    uint64_t*    seed_keys; // [grid * seed_P]
 };
 
 template <typename T> struct Elem;
@@ -157,6 +161,60 @@ __device__ __forceinline__ void quant_planes(float qv, float dh, float dl, int& 
     h = max(-127, min(127, h));
     l = __float2int_rn((qv - (float)h * dh) / dl);
     l = max(-127, min(127, l));
+}
+
+// The int8 arithmetic, one definition for the streaming kernel and the gate's seed (gate_seed_kernel).
+// Plane steps from max |q|: dh = max|q| / 127, dl = dh / 254.
+__device__ __forceinline__ void i8_steps(float qmax, float& dh, float& dl) {
+    dh = qmax > 0.f ? qmax / 127.f : 1.f;
+    dl = dh / 254.f;
+}
+// Lane cl's query registers: per chunk j (elements (j * LANES + cl) * 16 ...), 4 words of the hi plane, then 4 of the lo plane.
+template <int CPL, int LANES>
+__device__ __forceinline__ void i8_query_regs(const float* __restrict__ q, int d, int cl, float dh, float dl, uint32_t* qi) {
+#pragma unroll
+    for (int j = 0; j < CPL; ++j) {
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {
+            uint32_t ph = 0, pl = 0;
+#pragma unroll
+            for (int b = 0; b < 4; ++b) {
+                const int idx = (j * LANES + cl) * 16 + w * 4 + b;
+                const float qv = idx < d ? __ldg(q + idx) : 0.f;
+                int h, l;
+                quant_planes(qv, dh, dl, h, l);
+                ph |= (uint32_t)(h & 0xFF) << (8 * b);
+                pl |= (uint32_t)(l & 0xFF) << (8 * b);
+            }
+            qi[j * 8 + w] = ph;
+            qi[j * 8 + 4 + w] = pl;
+        }
+    }
+}
+// Four rows at once (8 independent dp4a chains, 8 shuffle reductions in flight): pr[u] points at row u's first chunk of this
+// lane; on return every lane of the row holds its exact int32 sums against both planes.
+template <int CPL, int LANES>
+__device__ __forceinline__ void i8_dot4(const uint4* const (&pr)[4], const uint32_t* qi, int (&hs)[4], int (&ls)[4]) {
+#pragma unroll
+    for (int j = 0; j < CPL; ++j) {
+        uint4 x[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) x[u] = pr[u][j * LANES];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) Elem<int8_t>::dot2(x[u], qi + j * 8, hs[u], ls[u]);
+    }
+#pragma unroll
+    for (int o = LANES / 2; o > 0; o >>= 1) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            hs[u] += __shfl_xor_sync(0xffffffffu, hs[u], o);
+            ls[u] += __shfl_xor_sync(0xffffffffu, ls[u], o);
+        }
+    }
+}
+// The int8 score S of a row from its sums and its factor (gate_factor / the shadow's inv_norm).
+__device__ __forceinline__ float i8_score(float dh, float dl, int hs, int ls, float factor) {
+    return fmaf(dh, (float)hs, dl * (float)ls) * factor;
 }
 
 // The gate's delta for the query actually passed (DESIGN.md §4.5), rounded up to fp32.  With S the int8 score, F the
@@ -404,26 +462,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
             float qmax = 0.f;
 #pragma unroll
             for (int w = 0; w <= kConsumerWarps; ++w) qmax = fmaxf(qmax, s_qmax[w]);
-            dh = qmax > 0.f ? qmax / 127.f : 1.f;
-            dl = dh / 254.f;
-#pragma unroll
-            for (int j = 0; j < (kI8 ? CPL : 0); ++j) {
-#pragma unroll
-                for (int w = 0; w < 4; ++w) {
-                    uint32_t ph = 0, pl = 0;
-#pragma unroll
-                    for (int b = 0; b < 4; ++b) {
-                        const int idx = (j * LANES + cl) * 16 + w * 4 + b;
-                        const float qv = idx < p.d ? __ldg(p.q + idx) : 0.f;
-                        int h, l;
-                        quant_planes(qv, dh, dl, h, l);
-                        ph |= (uint32_t)(h & 0xFF) << (8 * b);
-                        pl |= (uint32_t)(l & 0xFF) << (8 * b);
-                    }
-                    qi[j * 8 + w] = ph;
-                    qi[j * 8 + 4 + w] = pl;
-                }
-            }
+            i8_steps(qmax, dh, dl);
+            i8_query_regs<CPL, LANES>(p.q, p.d, cl, dh, dl, qi);
         } else if (kRegQ) {
 #pragma unroll
             for (int j = 0; j < (kRegQ ? CPL : 0); ++j)
@@ -473,26 +513,11 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                         vv[u] = rr[u] < nrows;
                         pr[u] = tile + (size_t)(vv[u] ? rr[u] : 0) * row_chunks + cl;
                     }
-#pragma unroll
-                    for (int j = 0; j < (kI8 ? CPL : 0); ++j) {
-                        uint4 x[4];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) x[u] = pr[u][j * LANES];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) Elem<int8_t>::dot2(x[u], qi + j * 8, hs[u], ls[u]);
-                    }
-#pragma unroll
-                    for (int o = LANES / 2; o > 0; o >>= 1) {
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            hs[u] += __shfl_xor_sync(0xffffffffu, hs[u], o);
-                            ls[u] += __shfl_xor_sync(0xffffffffu, ls[u], o);
-                        }
-                    }
+                    i8_dot4<CPL, LANES>(pr, qi, hs, ls);
 #pragma unroll
                     for (int u = 0; u < 4; ++u) {          // u ascending = rows ascending, which WarpTopK::insert relies on
                         const float inv = vv[u] ? (rr[u] < nrows4 ? inv_s[rr[u]] : __ldg(p.inv_norm + row0 + rr[u])) : 0.f;
-                        const float sc_lane = fmaf(dh, (float)hs[u], dl * (float)ls[u]) * inv;
+                        const float sc_lane = i8_score(dh, dl, hs[u], ls[u], inv);
                         if constexpr (kGate) {
                             // a row of the final list has F >= L, so S >= L - delta: rows below cannot get there
                             unsigned mm = __ballot_sync(0xffffffffu, vv[u] && cl == 0 && sc_lane >= fmaxf(top.thr, hint) - delta);
@@ -669,7 +694,140 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         select_winners<16>(pub, p.merge_cap, (uint64_t*)smem, p.cand_keys);
         __syncthreads();
     }
-    if (threadIdx.x < 32 && threadIdx.x != kCtlGateFetches) p.counter[threadIdx.x] = 0u;   // ticket, hint, tile claims, cursors
+    if (threadIdx.x < 32 && !ctl_survives_merge(threadIdx.x)) p.counter[threadIdx.x] = 0u;   // ticket, hint, tile claims, cursors
+}
+
+// Seed of the gated kernel's grid-wide bound (DESIGN §4.5).  Until a warp's list is full its threshold is -inf, and until
+// the CTA's warps hold kc/8 keys each its hint is too, so the gated kernel used to read the row of record of almost every
+// row it met first (~38k rows at kc = 32 on 148 SMs) and later only the kc-th best of the rows ONE CTA had seen.  This
+// kernel runs between the query staging and the gated kernel:
+//   1. it scores a strided sample of seed_m int8 rows with the streaming kernel's arithmetic (i8_dot4 / i8_score);
+//   2. each warp keeps its seed_P best allowed rows by S (the request's whole filter), each CTA the seed_P best of its warps;
+//   3. the last CTA (ticket) takes the kc best of those, reads their rows of record, scores them exactly as the gated kernel
+//      does (fetch_row_dot, xinv) and writes L0 = the smallest of these kc fast scores into the grid-wide hint.
+// kc distinct allowed rows have F >= L0, so L0 is a lower bound of the final kc-th best fast score: the meaning the hint
+// already has.  Nothing is inserted into any list, so the candidates stay the plain kernel's.  Fewer than kc published keys:
+// no bound.  seed_P = 2 ceil(kc / grid) per CTA loses a row of the sample's best kc only where one CTA holds more than that.
+constexpr int kSeedWarps = 8;
+
+template <int CPL, typename TX>
+__global__ void __launch_bounds__(kSeedWarps * 32, 1) gate_seed_kernel(const GemvParams p) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    float* q_smem = (float*)smem;                                  // [x_ld] the query, last CTA
+    uint64_t* buf = (uint64_t*)(smem + (((size_t)p.x_ld * 4 + 15) & ~(size_t)15));   // [grid * seed_P] published keys, last CTA
+    int32_t* excl_smem = (int32_t*)(buf + (size_t)gridDim.x * p.seed_P);
+    const bool excl_staged = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem;
+    const int32_t* excl_s = excl_staged ? excl_smem : nullptr;   // a filter test is a chain of dependent loads: keep it on chip
+    __shared__ float s_qmax[kSeedWarps];
+    __shared__ uint64_t s_keys[kSeedWarps * 32];                   // each warp's seed_P best, then the kc selected keys
+    __shared__ uint64_t s_best[32];
+    __shared__ int s_last, s_cnt;
+    __shared__ unsigned s_min;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int P = p.seed_P, kc = p.kc;
+    pdl_trigger();                   // the gated kernel may place its CTAs and start its early TMA as these retire
+    pdl_wait();
+    if (excl_staged) {
+        for (int c = threadIdx.x; c < p.filter.n_exclude; c += blockDim.x) excl_smem[c] = __ldg(p.filter.exclude_rows + c);
+    }
+
+    float m = 0.f;
+    for (int c = threadIdx.x; c < p.d; c += blockDim.x) m = fmaxf(m, fabsf(__ldg(p.q + c)));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if (lane == 0) s_qmax[warp] = m;
+    if (threadIdx.x < 32) s_best[threadIdx.x] = 0;
+    __syncthreads();
+    float qmax = 0.f, dh, dl;
+#pragma unroll
+    for (int w = 0; w < kSeedWarps; ++w) qmax = fmaxf(qmax, s_qmax[w]);
+    i8_steps(qmax, dh, dl);
+    uint32_t qi[CPL * 8];
+    i8_query_regs<CPL, 32>(p.q, p.d, lane, dh, dl, qi);
+
+    WarpTopK<1> top;
+    top.init();
+    uint64_t pth = 0;                                              // this warp's seed_P-th best key (0 while it has fewer)
+    const int64_t W = (int64_t)gridDim.x * kSeedWarps;
+    for (int64_t i0 = (int64_t)blockIdx.x * kSeedWarps + warp; i0 < p.seed_m; i0 += 4 * W) {
+        int64_t rr[4];
+        bool vv[4];
+        const uint4* pr[4];
+        float fac[4];
+        int hs[4] = {0, 0, 0, 0}, ls[4] = {0, 0, 0, 0};
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int64_t i = i0 + u * W;
+            vv[u] = i < p.seed_m;
+            rr[u] = vv[u] ? i * p.seed_stride : 0;
+            pr[u] = (const uint4*)p.rows + (size_t)rr[u] * (CPL * 32) + lane;
+            fac[u] = __ldg(p.inv_norm + rr[u]);
+        }
+        i8_dot4<CPL, 32>(pr, qi, hs, ls);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {                              // warp-uniform: every lane holds the row's sums
+            if (!vv[u]) continue;
+            const float s = i8_score(dh, dl, hs[u], ls[u], fac[u]);
+            const uint64_t key = make_key(s, (uint32_t)rr[u]);
+            if (key > pth && row_allowed(p.filter, (uint32_t)rr[u], excl_s)) {
+                top.insert(key, lane);
+                pth = __shfl_sync(0xffffffffu, top.keys[0], P - 1);
+            }
+        }
+    }
+    if (lane < P) s_keys[warp * P + lane] = top.keys[0];
+    __syncthreads();
+    // the CTA's seed_P best of its warps' keys (distinct: every sampled row belongs to one warp), by rank counting
+    for (int i = threadIdx.x; i < kSeedWarps * P; i += blockDim.x) {
+        const uint64_t key = s_keys[i];
+        if (!key) continue;
+        int rank = 0;
+        for (int j = 0; j < kSeedWarps * P; ++j) rank += s_keys[j] > key;
+        if (rank < P) s_best[rank] = key;
+    }
+    __syncthreads();
+    if (threadIdx.x < P) p.seed_keys[(size_t)blockIdx.x * P + threadIdx.x] = s_best[threadIdx.x];
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = (atomicAdd(p.counter + kCtlSeedTicket, 1u) == gridDim.x - 1);
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+
+    // ---- last CTA: the kc best published keys, their fast scores, the bound
+    const int total = (int)gridDim.x * P;
+    for (int i = threadIdx.x; i < total; i += blockDim.x) buf[i] = ldcg_u64(p.seed_keys + i);
+    for (int c = threadIdx.x; c < p.x_ld; c += blockDim.x) q_smem[c] = p.q[c];
+    if (threadIdx.x == 0) { s_cnt = 0; s_min = ~0u; }
+    __syncthreads();
+    uint64_t* sel = s_keys;                                        // [kc <= 256]
+    for (int i = threadIdx.x; i < total; i += blockDim.x) {
+        const uint64_t key = buf[i];
+        if (!key) continue;
+        int rank = 0;
+        for (int j = 0; j < total; ++j) rank += buf[j] > key;
+        if (rank < kc) { sel[rank] = key; atomicAdd(&s_cnt, 1); }
+    }
+    __syncthreads();
+    unsigned bound = 0;
+    if (s_cnt == kc) {
+        for (int j = warp; j < kc; j += kSeedWarps) {
+            const uint32_t lr = key_row(sel[j]);
+            const uint4* xr = (const uint4*)((const TX*)p.xrows + (size_t)lr * p.x_ld);
+            const float sc = fetch_row_dot<TX>(xr, q_smem, p.x_cpl, lane) * __ldg(p.xinv + lr);
+            if (lane == 0) atomicMin(&s_min, f32_orderable(sc));
+        }
+        __syncthreads();
+        bound = s_min;
+    }
+    if (threadIdx.x == 0) {
+        if (bound) {
+            atomicMax(p.ghint, bound);
+            atomicAdd(p.counter + kCtlGateFetches, (unsigned)kc);
+        }
+        p.counter[kCtlSeedBound] = bound;
+        p.counter[kCtlSeedTicket] = 0u;
+    }
 }
 
 // ---------------------------------------------------------------- host side ----------------------------------
@@ -808,6 +966,37 @@ static int launch_gemv_gated(const RowLayout& L8, const GemvParams& p, const Gem
         case 6: return launch_gemv_m<int8_t, 6, 32, TX>(p, g, kc, st);
     }
     set_error("gemv_topk: no gated kernel for int8 rows of %d chunks per lane", L8.cpl);
+    return REBERT_ERR_UNSUPPORTED;
+}
+
+// Rows the gate's seed samples: 1/64 of the catalog, at least 16k and at most 128k (measured on the B200, DESIGN §4.5).
+constexpr int64_t kSeedRowsMin = 16384, kSeedRowsMax = 131072, kSeedShare = 64;
+static int64_t seed_rows(int64_t n) {
+    int64_t m = n / kSeedShare;
+    m = m < kSeedRowsMin ? kSeedRowsMin : (m > kSeedRowsMax ? kSeedRowsMax : m);
+    return m < n ? m : n;
+}
+
+template <int CPL, typename TX>
+static int launch_gate_seed_one(const GemvParams& p, cudaStream_t st) {
+    auto kern = gate_seed_kernel<CPL, TX>;
+    const int n_excl = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem ? p.filter.n_exclude : 0;
+    const size_t smem = (((size_t)p.x_ld * 4 + 15) & ~(size_t)15) + (size_t)num_sms() * p.seed_P * sizeof(uint64_t) + (size_t)n_excl * 4;
+    { int rc = raise_smem_limit(kern); if (rc != REBERT_OK) return rc; }
+    REBERT_CUDA(launch_pdl(kern, dim3(num_sms()), dim3(kSeedWarps * 32), smem, st, p));
+    REBERT_CUDA(cudaGetLastError());
+    return REBERT_OK;
+}
+template <typename TX>
+static int launch_gate_seed(const RowLayout& L8, const GemvParams& p, cudaStream_t st) {
+    switch (L8.cpl) {
+        case 1: return launch_gate_seed_one<1, TX>(p, st);
+        case 2: return launch_gate_seed_one<2, TX>(p, st);
+        case 3: return launch_gate_seed_one<3, TX>(p, st);
+        case 4: return launch_gate_seed_one<4, TX>(p, st);
+        case 6: return launch_gate_seed_one<6, TX>(p, st);
+    }
+    set_error("gemv_topk: no gate seed kernel for int8 rows of %d chunks per lane", L8.cpl);
     return REBERT_ERR_UNSUPPORTED;
 }
 
@@ -959,6 +1148,15 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
     p.publish_only = fused ? 1 : 0;
 
     int rc;
+    if (gated && cat->n > 0) {                       // the seed's bound, in the grid-wide hint before the gated kernel starts
+        p.seed_m = seed_rows(cat->n);
+        p.seed_stride = cat->n / p.seed_m;
+        const int per = (kc + num_sms() - 1) / num_sms();
+        p.seed_P = 2 * per < 32 ? 2 * per : 32;
+        p.seed_keys = p.pub_keys;                    // free until the gated kernel publishes, which waits for the seed
+        rc = cat->dtype == REBERT_F32 ? launch_gate_seed<float>(LS, p, st) : launch_gate_seed<__nv_bfloat16>(LS, p, st);
+        if (rc != REBERT_OK) return rc;
+    }
     if (cat->dtype == REBERT_I8) rc = launch_gemv_i8(L, p, g, st);
     else if (gated) rc = cat->dtype == REBERT_F32 ? launch_gemv_gated<float>(LS, p, g, kc, st) : launch_gemv_gated<__nv_bfloat16>(LS, p, g, kc, st);
     else rc = cat->dtype == REBERT_F32 ? launch_gemv<float>(L, p, g, kc, st) : launch_gemv<__nv_bfloat16>(L, p, g, kc, st);
