@@ -66,10 +66,11 @@ struct GemvParams {
     const float* xinv;      // [n] its inv_norm
     int          x_ld, x_cpl;   // its padded row length and chunks per lane (32-lane layout)
     double       gate_err;  // max relative row error of the int8 gate rows (rebert_catalog_quantize_i8)
-    // gate_seed_kernel only: rows i * seed_stride (i < seed_m) are sampled; every CTA publishes its seed_P best into seed_keys
+    // the gate's seed: rows i * seed_stride (i < seed_m) are sampled; every CTA publishes its seed_P best into seed_keys
     int64_t      seed_m, seed_stride;
     int          seed_P;
     uint64_t*    seed_keys; // [grid * seed_P]
+    int          seed_fold; // gated kernel: run the seed as its prologue (else gate_seed_kernel ran ahead of it)
 };
 
 template <typename T> struct Elem;
@@ -191,10 +192,10 @@ __device__ __forceinline__ void i8_query_regs(const float* __restrict__ q, int d
         }
     }
 }
-// Four rows at once (8 independent dp4a chains, 8 shuffle reductions in flight): pr[u] points at row u's first chunk of this
-// lane; on return every lane of the row holds its exact int32 sums against both planes.
+// Four rows at once (8 independent dp4a chains): pr[u] points at row u's first chunk of this lane; on return this lane's
+// partial int32 sums against both planes.
 template <int CPL, int LANES>
-__device__ __forceinline__ void i8_dot4(const uint4* const (&pr)[4], const uint32_t* qi, int (&hs)[4], int (&ls)[4]) {
+__device__ __forceinline__ void i8_partial4(const uint4* const (&pr)[4], const uint32_t* qi, int (&hs)[4], int (&ls)[4]) {
 #pragma unroll
     for (int j = 0; j < CPL; ++j) {
         uint4 x[4];
@@ -203,6 +204,11 @@ __device__ __forceinline__ void i8_dot4(const uint4* const (&pr)[4], const uint3
 #pragma unroll
         for (int u = 0; u < 4; ++u) Elem<int8_t>::dot2(x[u], qi + j * 8, hs[u], ls[u]);
     }
+}
+// Rows narrower than 32 lanes: 8 shuffle reductions over the row's LANES lanes; every lane of the row holds its exact sums.
+template <int CPL, int LANES>
+__device__ __forceinline__ void i8_dot4(const uint4* const (&pr)[4], const uint32_t* qi, int (&hs)[4], int (&ls)[4]) {
+    i8_partial4<CPL, LANES>(pr, qi, hs, ls);
 #pragma unroll
     for (int o = LANES / 2; o > 0; o >>= 1) {
 #pragma unroll
@@ -211,6 +217,30 @@ __device__ __forceinline__ void i8_dot4(const uint4* const (&pr)[4], const uint3
             ls[u] += __shfl_xor_sync(0xffffffffu, ls[u], o);
         }
     }
+}
+// 32-lane rows: the 8 partial sums are reduced by a transposing butterfly instead of 8 separate 5-level trees (10 shuffles
+// instead of 40).  At each of the first three levels a lane keeps half of its sums and adds its partner's copy of them, so
+// afterwards lane L holds sum 4 b4 + 2 b3 + b2 (its lane bits) over the 8 lanes that share those bits; two more levels
+// complete it over the warp, and one swap across lane bit 4 pairs each row's hi sum with its lo sum.  On return lane L holds
+// the exact sums (hs, ls) of row i8_row(L).  Integer sums are exact, so they equal the trees' bit for bit.
+__device__ __forceinline__ int i8_row(int lane) { return (lane >> 2) & 3; }
+template <int CPL>
+__device__ __forceinline__ void i8_dot4_32(const uint4* const (&pr)[4], const uint32_t* qi, int lane, int& hs, int& ls) {
+    int h[4] = {0, 0, 0, 0}, l[4] = {0, 0, 0, 0};
+    i8_partial4<CPL, 32>(pr, qi, h, l);
+    const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4;
+    int w[4];                                            // sums j + 4 b4: hi plane (b4 = 0) or lo plane (b4 = 1) of row j
+#pragma unroll
+    for (int j = 0; j < 4; ++j) w[j] = (b4 ? l[j] : h[j]) + __shfl_xor_sync(0xffffffffu, b4 ? h[j] : l[j], 16);
+    int x[2];                                            // rows 2 b3 + j
+#pragma unroll
+    for (int j = 0; j < 2; ++j) x[j] = (b3 ? w[j + 2] : w[j]) + __shfl_xor_sync(0xffffffffu, b3 ? w[j] : w[j + 2], 8);
+    int y = (b2 ? x[1] : x[0]) + __shfl_xor_sync(0xffffffffu, b2 ? x[0] : x[1], 4);   // row 2 b3 + b2
+    y += __shfl_xor_sync(0xffffffffu, y, 2);
+    y += __shfl_xor_sync(0xffffffffu, y, 1);
+    const int other = __shfl_xor_sync(0xffffffffu, y, 16);
+    hs = b4 ? other : y;
+    ls = b4 ? y : other;
 }
 // The int8 score S of a row from its sums and its factor (gate_factor / the shadow's inv_norm).
 __device__ __forceinline__ float i8_score(float dh, float dl, int hs, int ls, float factor) {
@@ -278,6 +308,151 @@ __device__ __forceinline__ void publish_hints(uint64_t key0, float thr, int warp
     }
 }
 
+// Seed of the gated kernel's grid-wide bound (DESIGN §4.5).  Until a warp's list is full its threshold is -inf, and until
+// the CTA's warps hold kc/8 keys each its hint is too, so without a seed the gated kernel reads the row of record of almost
+// every row it meets first (~38k rows at kc = 32 on 148 SMs) and later only the kc-th best of the rows ONE CTA has seen.
+// The seed runs on 8 warps of every CTA of a grid of one CTA per SM: as the prologue of the gated kernel's consumer warps
+// (seed_fold), or as gate_seed_kernel ahead of a gated grid of another size.
+//   1. seed_sample: it scores a strided sample of seed_m int8 rows with the streaming kernel's arithmetic (i8_dot4_32 /
+//      i8_score); warp w of CTA c takes samples c * 8 + w + t * 8 * grid;
+//   2. each warp keeps its seed_P best allowed rows by S (the request's whole filter), each CTA the seed_P best of its warps;
+//   3. seed_bound, in the last CTA (ticket): it takes the kc best of those, reads their rows of record, scores them exactly as
+//      the gated kernel does (fetch_row_dot, xinv) and writes L0 = the smallest of these kc fast scores into the grid-wide
+//      hint and control word 21, then resets the ticket, which tells the other CTAs that the seed is done (seed_wait).
+// kc distinct allowed rows have F >= L0, so L0 is a lower bound of the final kc-th best fast score: the meaning the hint
+// already has.  Nothing is inserted into any list, so the candidates stay the plain kernel's.  Fewer than kc published keys:
+// no bound.  seed_P = 2 ceil(kc / grid) per CTA loses a row of the sample's best kc only where one CTA holds more than that.
+constexpr int kSeedWarps = kConsumerWarps;
+// The fold is compiled for int8 rows of up to 4 chunks per lane (d <= 2048): at 6 the prologue would make the gated kernel
+// spill, so those rows keep gate_seed_kernel.
+constexpr int kSeedFoldMaxCpl = 4;
+constexpr int kSeedThreads = kSeedWarps * 32;
+// shared memory of the seed: [kSeedWarps * 32] each warp's seed_P best (then the kc selected keys), [32] the CTA's seed_P best
+constexpr int kSeedSmemKeys = kSeedWarps * 32 + 32;
+// barrier of the 8 seed warps alone (the gated kernel's producer warp keeps issuing its first tiles meanwhile)
+__device__ __forceinline__ void seed_sync() { asm volatile("bar.sync 1, %0;" ::"n"(kSeedThreads) : "memory"); }
+
+// Steps 1 and 2, then the ticket: true in the last CTA to publish.  Threads 0 .. kSeedThreads - 1; qi / dh / dl are the
+// streaming kernel's query planes.
+template <int CPL>
+__device__ __forceinline__ bool seed_sample(const GemvParams& p, const uint32_t* qi, float dh, float dl, const int32_t* excl_s,
+                                            uint64_t* s_keys, int* s_last) {
+    uint64_t* s_best = s_keys + kSeedWarps * 32;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int P = p.seed_P;
+    if (threadIdx.x < 32) s_best[threadIdx.x] = 0;
+    WarpTopK<1> top;
+    top.init();
+    uint64_t pth = 0;                                              // this warp's seed_P-th best key (0 while it has fewer)
+    const int64_t W = (int64_t)gridDim.x * kSeedWarps;
+    const int ul = i8_row(lane);
+    for (int64_t i0 = (int64_t)blockIdx.x * kSeedWarps + warp; i0 < p.seed_m; i0 += 4 * W) {
+        int64_t rr[4];
+        const uint4* pr[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int64_t i = i0 + u * W;
+            rr[u] = i < p.seed_m ? i * p.seed_stride : -1;
+            pr[u] = (const uint4*)p.rows + (size_t)(rr[u] < 0 ? 0 : rr[u]) * (CPL * 32) + lane;
+        }
+        const int64_t rl = i0 + ul * W < p.seed_m ? (i0 + ul * W) * p.seed_stride : 0;   // this lane's row
+        const float fac = __ldg(p.inv_norm + rl);
+        int hs, ls;
+        i8_dot4_32<CPL>(pr, qi, lane, hs, ls);
+        const float s_lane = i8_score(dh, dl, hs, ls, fac);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {                              // warp-uniform
+            if (rr[u] < 0) continue;
+            const float s = __shfl_sync(0xffffffffu, s_lane, 4 * u);
+            const uint64_t key = make_key(s, (uint32_t)rr[u]);
+            if (key > pth && row_allowed(p.filter, (uint32_t)rr[u], excl_s)) {
+                top.insert(key, lane);
+                pth = __shfl_sync(0xffffffffu, top.keys[0], P - 1);
+            }
+        }
+    }
+    if (lane < P) s_keys[warp * P + lane] = top.keys[0];
+    seed_sync();
+    // the CTA's seed_P best of its warps' keys (distinct: every sampled row belongs to one warp), by rank counting
+    for (int i = threadIdx.x; i < kSeedWarps * P; i += kSeedThreads) {
+        const uint64_t key = s_keys[i];
+        if (!key) continue;
+        int rank = 0;
+        for (int j = 0; j < kSeedWarps * P; ++j) rank += s_keys[j] > key;
+        if (rank < P) s_best[rank] = key;
+    }
+    seed_sync();
+    if (threadIdx.x < P) p.seed_keys[(size_t)blockIdx.x * P + threadIdx.x] = s_best[threadIdx.x];
+    __threadfence();
+    seed_sync();
+    if (threadIdx.x == 0) *s_last = (atomicAdd(p.counter + kCtlSeedTicket, 1u) == gridDim.x - 1);
+    seed_sync();
+    return *s_last != 0;
+}
+
+// Step 3, in the last CTA: q_smem holds the query [x_ld], buf has room for grid * seed_P keys.
+template <typename TX>
+__device__ __forceinline__ void seed_bound(const GemvParams& p, const float* q_smem, uint64_t* s_keys, uint64_t* buf, int* s_cnt,
+                                           unsigned* s_min) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int kc = p.kc;
+    __threadfence();
+    const int total = (int)gridDim.x * p.seed_P;
+    for (int i = threadIdx.x; i < total; i += kSeedThreads) buf[i] = ldcg_u64(p.seed_keys + i);
+    if (threadIdx.x == 0) { *s_cnt = 0; *s_min = ~0u; }
+    seed_sync();
+    uint64_t* sel = s_keys;                                        // [kc <= 256]
+    for (int i = threadIdx.x; i < total; i += kSeedThreads) {
+        const uint64_t key = buf[i];
+        if (!key) continue;
+        int rank = 0;
+        for (int j = 0; j < total; ++j) rank += buf[j] > key;
+        if (rank < kc) { sel[rank] = key; atomicAdd(s_cnt, 1); }
+    }
+    seed_sync();
+    unsigned bound = 0;
+    if (*s_cnt == kc) {
+        for (int j = warp; j < kc; j += kSeedWarps) {
+            const uint32_t lr = key_row(sel[j]);
+            const uint4* xr = (const uint4*)((const TX*)p.xrows + (size_t)lr * p.x_ld);
+            const float sc = fetch_row_dot<TX>(xr, q_smem, p.x_cpl, lane) * __ldg(p.xinv + lr);
+            if (lane == 0) atomicMin(s_min, f32_orderable(sc));
+        }
+        seed_sync();
+        bound = *s_min;
+    }
+    if (threadIdx.x == 0) {
+        if (bound) {
+            atomicMax(p.ghint, bound);
+            atomicAdd(p.counter + kCtlGateFetches, (unsigned)kc);
+        }
+        p.counter[kCtlSeedBound] = bound;
+        __threadfence();                                           // the bound is visible before the ticket says "done"
+        *(volatile unsigned*)(p.counter + kCtlSeedTicket) = 0u;
+    }
+}
+
+// The other CTAs of a folded seed wait (each warp on its own) until the last CTA has reset the ticket; their own increment
+// came first, so a zero ticket cannot be the state before the seed.  The wait is bounded: a CTA that is not co-resident
+// with the rest of its grid (another stream's kernel holds SMs) streams on after kSeedWaitNs without the bound, which is
+// only slower; a bound that lands later reaches it through the grid-wide hint.
+constexpr unsigned long long kSeedWaitNs = 200000;
+__device__ __forceinline__ void seed_wait(const GemvParams& p) {
+    if ((threadIdx.x & 31) == 0) {
+        unsigned long long t0, t;
+        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
+        for (;;) {
+            unsigned v;
+            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p.counter + kCtlSeedTicket) : "memory");
+            if (v == 0u) break;
+            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+            if (t - t0 > kSeedWaitNs) break;
+            __nanosleep(256);
+        }
+    }
+    __syncwarp();
+}
+
 // TX = void: the plain kernel (T = the streamed rows' type).  TX = bf16 / float: the GATED kernel — T = int8_t streams the
 // catalog's int8 gate, and a row whose int8 score reaches L - delta (L = the warp's pruning bound) is read from the bf16 /
 // fp32 catalog of record and scored with the plain kernel's arithmetic, so the keys are the plain kernel's (DESIGN §4.5).
@@ -305,6 +480,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     int32_t* excl_smem = (int32_t*)(q_smem + (kGate ? p.x_ld : (kRegQ ? 0 : p.ld)));
     const bool excl_staged = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem;
     const int32_t* excl_s = excl_staged ? excl_smem : nullptr;
+    // seed_fold: the seed's keys after the staged exclusion list (seed_smem_bytes)
+    uint64_t* seed_smem = (uint64_t*)(((uintptr_t)(excl_smem + (excl_staged ? p.filter.n_exclude : 0)) + 7) & ~(uintptr_t)7);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
@@ -474,6 +651,18 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
         const int row_chunks = cpl * LANES;
         const float delta = kGate ? s_delta : 0.f;
         unsigned fetched = 0;                    // gated kernel: rows read from the catalog of record (warp-uniform)
+        if constexpr (kGate && CPL <= kSeedFoldMaxCpl) {
+            if (p.seed_fold) {
+                // the seed, while the producer's first tiles are in flight; the last CTA forms the bound, the others wait
+                // for it (bounded) and every CTA then streams with it from its first tile
+                __shared__ int s_last, s_cnt;
+                __shared__ unsigned s_min;
+                if (seed_sample<CPL>(p, qi, dh, dl, excl_s, seed_smem, &s_last))
+                    seed_bound<TX>(p, q_smem, seed_smem, seed_smem + kSeedSmemKeys, &s_cnt, &s_min);
+                else
+                    seed_wait(p);
+            }
+        }
 
         for (int it = 0;; ++it) {
             const int s = it % p.stages;
@@ -499,9 +688,63 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
             const int nrows = left < p.tile_rows ? (int)left : p.tile_rows;
             const int nrows4 = nrows & ~3;
 
-            if constexpr (kI8) {
-                // int8 shadow: rows are half as long, so a warp has to turn rows around twice as fast to keep up with HBM;
-                // FOUR rows per step (8 independent dp4a chains, 8 shuffle reductions in flight) hide the per-step latency.
+            if constexpr (kI8 && LANES == 32) {
+                // int8 rows are half as long, so a warp has to turn rows around twice as fast to keep up with HBM: FOUR rows
+                // per step (8 independent dp4a chains, one butterfly reduction) hide the per-step latency.  Lane L scores
+                // row i8_row(L); lanes 0, 4, 8, 12 vote for rows 0..3 in one ballot, whose bits ascend with the rows (which
+                // WarpTopK::insert relies on).  Each candidate is re-tested against the list as it stands when its turn comes.
+                const int ul = i8_row(lane);
+                for (int base = warp; base < nrows; base += 4 * kConsumerWarps) {
+                    const uint4* pr[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int r = base + u * kConsumerWarps;
+                        pr[u] = tile + (size_t)(r < nrows ? r : 0) * row_chunks + lane;
+                    }
+                    const int rl = base + ul * kConsumerWarps;     // this lane's row
+                    const bool vl = rl < nrows;
+                    const float inv = vl ? (rl < nrows4 ? inv_s[rl] : __ldg(p.inv_norm + row0 + rl)) : 0.f;
+                    int hs, ls;
+                    i8_dot4_32<CPL>(pr, qi, lane, hs, ls);
+                    const float sc_lane = i8_score(dh, dl, hs, ls, inv);
+                    const bool voter = vl && (lane & 19) == 0;
+                    if constexpr (kGate) {
+                        // a row of the final list has F >= L, so S >= L - delta: rows below cannot get there
+                        unsigned mm = __ballot_sync(0xffffffffu, voter && sc_lane >= fmaxf(top.thr, hint) - delta);
+                        while (mm) {
+                            const int src = __ffs(mm) - 1;
+                            mm &= mm - 1;
+                            const float sv = __shfl_sync(0xffffffffu, sc_lane, src);
+                            const uint32_t lr = (uint32_t)(row0 + base + i8_row(src) * kConsumerWarps);
+                            if (sv >= fmaxf(top.thr, hint) - delta && row_allowed(p.filter, lr, excl_s)) {
+                                ++fetched;
+                                const uint4* xr = (const uint4*)((const TX*)p.xrows + (size_t)lr * p.x_ld);
+                                const float sc = fetch_row_dot<TX>(xr, q_smem, p.x_cpl, lane) * __ldg(p.xinv + lr);
+                                if (sc > top.thr && sc >= hint) {
+                                    top.insert(make_key(sc, lr), lane);
+                                    publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
+                                }
+                            }
+                        }
+                    } else {
+                        unsigned mm = __ballot_sync(0xffffffffu, voter && sc_lane > top.thr && sc_lane >= hint);
+                        while (mm) {
+                            const int src = __ffs(mm) - 1;
+                            mm &= mm - 1;
+                            const float sc = __shfl_sync(0xffffffffu, sc_lane, src);
+                            const uint32_t lr = (uint32_t)(row0 + base + i8_row(src) * kConsumerWarps);
+                            if (sc > top.thr && row_allowed(p.filter, lr, excl_s)) {
+                                top.insert(make_key(sc, lr), lane);
+                                publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
+                            }
+                        }
+                    }
+                }
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&empty_bar[s]);
+                continue;
+            } else if constexpr (kI8) {
+                // int8 shadow rows narrower than 32 lanes: RPW rows per lane group, four groups per step
                 for (int base = warp * RPW; base < nrows; base += 4 * kConsumerWarps * RPW) {
                     int rr[4];
                     bool vv[4];
@@ -518,26 +761,6 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
                     for (int u = 0; u < 4; ++u) {          // u ascending = rows ascending, which WarpTopK::insert relies on
                         const float inv = vv[u] ? (rr[u] < nrows4 ? inv_s[rr[u]] : __ldg(p.inv_norm + row0 + rr[u])) : 0.f;
                         const float sc_lane = i8_score(dh, dl, hs[u], ls[u], inv);
-                        if constexpr (kGate) {
-                            // a row of the final list has F >= L, so S >= L - delta: rows below cannot get there
-                            unsigned mm = __ballot_sync(0xffffffffu, vv[u] && cl == 0 && sc_lane >= fmaxf(top.thr, hint) - delta);
-                            while (mm) {
-                                const int src = __ffs(mm) - 1;
-                                mm &= mm - 1;
-                                const float sv = __shfl_sync(0xffffffffu, sc_lane, src);
-                                const uint32_t lr = (uint32_t)(row0 + base + u * kConsumerWarps * RPW + src / LANES);
-                                if (sv >= fmaxf(top.thr, hint) - delta && row_allowed(p.filter, lr, excl_s)) {
-                                    ++fetched;
-                                    const uint4* xr = (const uint4*)((const TX*)p.xrows + (size_t)lr * p.x_ld);
-                                    const float sc = fetch_row_dot<TX>(xr, q_smem, p.x_cpl, lane) * __ldg(p.xinv + lr);
-                                    if (sc > top.thr && sc >= hint) {
-                                        top.insert(make_key(sc, lr), lane);
-                                        publish_hints<kQuantLane>(top.keys[0], top.thr, warp, lane, &s_hint, s_wq);
-                                    }
-                                }
-                            }
-                            continue;
-                        }
                         unsigned mm = __ballot_sync(0xffffffffu, vv[u] && cl == 0 && sc_lane > top.thr && sc_lane >= hint);
                         while (mm) {
                             const int src = __ffs(mm) - 1;
@@ -697,21 +920,10 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_topk_kernel(const GemvParams
     if (threadIdx.x < 32 && !ctl_survives_merge(threadIdx.x)) p.counter[threadIdx.x] = 0u;   // ticket, hint, tile claims, cursors
 }
 
-// Seed of the gated kernel's grid-wide bound (DESIGN §4.5).  Until a warp's list is full its threshold is -inf, and until
-// the CTA's warps hold kc/8 keys each its hint is too, so the gated kernel used to read the row of record of almost every
-// row it met first (~38k rows at kc = 32 on 148 SMs) and later only the kc-th best of the rows ONE CTA had seen.  This
-// kernel runs between the query staging and the gated kernel:
-//   1. it scores a strided sample of seed_m int8 rows with the streaming kernel's arithmetic (i8_dot4 / i8_score);
-//   2. each warp keeps its seed_P best allowed rows by S (the request's whole filter), each CTA the seed_P best of its warps;
-//   3. the last CTA (ticket) takes the kc best of those, reads their rows of record, scores them exactly as the gated kernel
-//      does (fetch_row_dot, xinv) and writes L0 = the smallest of these kc fast scores into the grid-wide hint.
-// kc distinct allowed rows have F >= L0, so L0 is a lower bound of the final kc-th best fast score: the meaning the hint
-// already has.  Nothing is inserted into any list, so the candidates stay the plain kernel's.  Fewer than kc published keys:
-// no bound.  seed_P = 2 ceil(kc / grid) per CTA loses a row of the sample's best kc only where one CTA holds more than that.
-constexpr int kSeedWarps = 8;
-
+// The seed ahead of a gated grid that is not one CTA per SM (small catalogs), or whose seed keys do not fit beside the
+// pipeline: one CTA per SM, 8 warps, the same seed functions.
 template <int CPL, typename TX>
-__global__ void __launch_bounds__(kSeedWarps * 32, 1) gate_seed_kernel(const GemvParams p) {
+__global__ void __launch_bounds__(kSeedThreads, 1) gate_seed_kernel(const GemvParams p) {
     extern __shared__ __align__(128) unsigned char smem[];
     float* q_smem = (float*)smem;                                  // [x_ld] the query, last CTA
     uint64_t* buf = (uint64_t*)(smem + (((size_t)p.x_ld * 4 + 15) & ~(size_t)15));   // [grid * seed_P] published keys, last CTA
@@ -719,12 +931,10 @@ __global__ void __launch_bounds__(kSeedWarps * 32, 1) gate_seed_kernel(const Gem
     const bool excl_staged = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem;
     const int32_t* excl_s = excl_staged ? excl_smem : nullptr;   // a filter test is a chain of dependent loads: keep it on chip
     __shared__ float s_qmax[kSeedWarps];
-    __shared__ uint64_t s_keys[kSeedWarps * 32];                   // each warp's seed_P best, then the kc selected keys
-    __shared__ uint64_t s_best[32];
+    __shared__ uint64_t s_keys[kSeedSmemKeys];
     __shared__ int s_last, s_cnt;
     __shared__ unsigned s_min;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int P = p.seed_P, kc = p.kc;
     pdl_trigger();                   // the gated kernel may place its CTAs and start its early TMA as these retire
     pdl_wait();
     if (excl_staged) {
@@ -736,7 +946,6 @@ __global__ void __launch_bounds__(kSeedWarps * 32, 1) gate_seed_kernel(const Gem
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
     if (lane == 0) s_qmax[warp] = m;
-    if (threadIdx.x < 32) s_best[threadIdx.x] = 0;
     __syncthreads();
     float qmax = 0.f, dh, dl;
 #pragma unroll
@@ -744,90 +953,9 @@ __global__ void __launch_bounds__(kSeedWarps * 32, 1) gate_seed_kernel(const Gem
     i8_steps(qmax, dh, dl);
     uint32_t qi[CPL * 8];
     i8_query_regs<CPL, 32>(p.q, p.d, lane, dh, dl, qi);
-
-    WarpTopK<1> top;
-    top.init();
-    uint64_t pth = 0;                                              // this warp's seed_P-th best key (0 while it has fewer)
-    const int64_t W = (int64_t)gridDim.x * kSeedWarps;
-    for (int64_t i0 = (int64_t)blockIdx.x * kSeedWarps + warp; i0 < p.seed_m; i0 += 4 * W) {
-        int64_t rr[4];
-        bool vv[4];
-        const uint4* pr[4];
-        float fac[4];
-        int hs[4] = {0, 0, 0, 0}, ls[4] = {0, 0, 0, 0};
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int64_t i = i0 + u * W;
-            vv[u] = i < p.seed_m;
-            rr[u] = vv[u] ? i * p.seed_stride : 0;
-            pr[u] = (const uint4*)p.rows + (size_t)rr[u] * (CPL * 32) + lane;
-            fac[u] = __ldg(p.inv_norm + rr[u]);
-        }
-        i8_dot4<CPL, 32>(pr, qi, hs, ls);
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {                              // warp-uniform: every lane holds the row's sums
-            if (!vv[u]) continue;
-            const float s = i8_score(dh, dl, hs[u], ls[u], fac[u]);
-            const uint64_t key = make_key(s, (uint32_t)rr[u]);
-            if (key > pth && row_allowed(p.filter, (uint32_t)rr[u], excl_s)) {
-                top.insert(key, lane);
-                pth = __shfl_sync(0xffffffffu, top.keys[0], P - 1);
-            }
-        }
-    }
-    if (lane < P) s_keys[warp * P + lane] = top.keys[0];
-    __syncthreads();
-    // the CTA's seed_P best of its warps' keys (distinct: every sampled row belongs to one warp), by rank counting
-    for (int i = threadIdx.x; i < kSeedWarps * P; i += blockDim.x) {
-        const uint64_t key = s_keys[i];
-        if (!key) continue;
-        int rank = 0;
-        for (int j = 0; j < kSeedWarps * P; ++j) rank += s_keys[j] > key;
-        if (rank < P) s_best[rank] = key;
-    }
-    __syncthreads();
-    if (threadIdx.x < P) p.seed_keys[(size_t)blockIdx.x * P + threadIdx.x] = s_best[threadIdx.x];
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) s_last = (atomicAdd(p.counter + kCtlSeedTicket, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-
-    // ---- last CTA: the kc best published keys, their fast scores, the bound
-    const int total = (int)gridDim.x * P;
-    for (int i = threadIdx.x; i < total; i += blockDim.x) buf[i] = ldcg_u64(p.seed_keys + i);
+    if (!seed_sample<CPL>(p, qi, dh, dl, excl_s, s_keys, &s_last)) return;
     for (int c = threadIdx.x; c < p.x_ld; c += blockDim.x) q_smem[c] = p.q[c];
-    if (threadIdx.x == 0) { s_cnt = 0; s_min = ~0u; }
-    __syncthreads();
-    uint64_t* sel = s_keys;                                        // [kc <= 256]
-    for (int i = threadIdx.x; i < total; i += blockDim.x) {
-        const uint64_t key = buf[i];
-        if (!key) continue;
-        int rank = 0;
-        for (int j = 0; j < total; ++j) rank += buf[j] > key;
-        if (rank < kc) { sel[rank] = key; atomicAdd(&s_cnt, 1); }
-    }
-    __syncthreads();
-    unsigned bound = 0;
-    if (s_cnt == kc) {
-        for (int j = warp; j < kc; j += kSeedWarps) {
-            const uint32_t lr = key_row(sel[j]);
-            const uint4* xr = (const uint4*)((const TX*)p.xrows + (size_t)lr * p.x_ld);
-            const float sc = fetch_row_dot<TX>(xr, q_smem, p.x_cpl, lane) * __ldg(p.xinv + lr);
-            if (lane == 0) atomicMin(&s_min, f32_orderable(sc));
-        }
-        __syncthreads();
-        bound = s_min;
-    }
-    if (threadIdx.x == 0) {
-        if (bound) {
-            atomicMax(p.ghint, bound);
-            atomicAdd(p.counter + kCtlGateFetches, (unsigned)kc);
-        }
-        p.counter[kCtlSeedBound] = bound;
-        p.counter[kCtlSeedTicket] = 0u;
-    }
+    seed_bound<TX>(p, q_smem, s_keys, buf, &s_cnt, &s_min);
 }
 
 // ---------------------------------------------------------------- host side ----------------------------------
@@ -838,8 +966,9 @@ struct GemvLaunch {
     size_t smem;
 };
 
-// q_floats: query elements staged in shared memory (generic kernel: ld; gated kernel: the catalog of record's ld)
-static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, int q_floats, int n_exclude) {
+// q_floats: query elements staged in shared memory (generic kernel: ld; gated kernel: the catalog of record's ld);
+// seed_bytes: the folded seed's keys (seed_smem_bytes), 0 without
+static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, int q_floats, int n_exclude, size_t seed_bytes = 0) {
     GemvLaunch g;
     const int row_bytes = L.ld * L.esize;
     const int rpw = 32 / L.lanes;
@@ -856,7 +985,7 @@ static GemvLaunch plan_gemv(const RowLayout& L, int64_t n, int kc, int q_floats,
     const int tile_bytes = tr * row_bytes;
     const int stage_stride = tile_bytes + ((tr * 4 + 127) & ~127);
     const size_t excl_bytes = (n_exclude > 0 && n_exclude <= kMaxExclSmem) ? (size_t)n_exclude * 4 : 0;
-    const size_t fixed = 2 * kStages * sizeof(uint64_t) + (size_t)q_floats * 4 + excl_bytes + 128;
+    const size_t fixed = 2 * kStages * sizeof(uint64_t) + (size_t)q_floats * 4 + excl_bytes + 128 + seed_bytes;
     int stages = kStages;
     while (stages > 1 && (size_t)stages * stage_stride + fixed > 220 * 1024) --stages;
     g.stages = stages;
@@ -976,6 +1105,14 @@ static int64_t seed_rows(int64_t n) {
     m = m < kSeedRowsMin ? kSeedRowsMin : (m > kSeedRowsMax ? kSeedRowsMax : m);
     return m < n ? m : n;
 }
+// Keys each seed CTA publishes: twice its share of kc, at most 32.
+static int seed_P_for(int kc) {
+    const int per = (kc + num_sms() - 1) / num_sms();
+    return 2 * per < 32 ? 2 * per : 32;
+}
+// Shared memory of the folded seed (gemv_topk_kernel's seed_smem): its warps' and CTA's keys, the last CTA's copy of all
+// CTAs' keys, 8 bytes of alignment.
+static size_t seed_smem_bytes(int kc) { return ((size_t)kSeedSmemKeys + (size_t)num_sms() * seed_P_for(kc)) * sizeof(uint64_t) + 8; }
 
 template <int CPL, typename TX>
 static int launch_gate_seed_one(const GemvParams& p, cudaStream_t st) {
@@ -983,7 +1120,7 @@ static int launch_gate_seed_one(const GemvParams& p, cudaStream_t st) {
     const int n_excl = p.filter.n_exclude > 0 && p.filter.n_exclude <= kMaxExclSmem ? p.filter.n_exclude : 0;
     const size_t smem = (((size_t)p.x_ld * 4 + 15) & ~(size_t)15) + (size_t)num_sms() * p.seed_P * sizeof(uint64_t) + (size_t)n_excl * 4;
     { int rc = raise_smem_limit(kern); if (rc != REBERT_OK) return rc; }
-    REBERT_CUDA(launch_pdl(kern, dim3(num_sms()), dim3(kSeedWarps * 32), smem, st, p));
+    REBERT_CUDA(launch_pdl(kern, dim3(num_sms()), dim3(kSeedThreads), smem, st, p));
     REBERT_CUDA(cudaGetLastError());
     return REBERT_OK;
 }
@@ -1035,13 +1172,16 @@ REBERT_API int32_t rebert_candidates_for_k(int32_t k) {
 //   [0, 128)       32 control words: ticket counter, grid-wide hint, tile-claim counter, -, 16 compaction cursors  (zero
 //                  before a launch; whoever merges — the last CTA, or the cluster kernel of the request path — zeroes them)
 //   [128, 2176)    tail key of every CTA list (u64 x 256)
-//   [2176, ...)    kept keys of all CTAs [16 regions][region_cap] u64; then the list heads [kc + 256] u64
+//   [2176, ...)    kept keys of all CTAs [16 regions][region_cap] u64; then the list heads [kc + 256] u64; then the keys the
+//                  gate's seed CTAs publish [SMs * 32] u64 (their own region: with a folded seed, a CTA may publish its list
+//                  while the last seed CTA still reads them)
 constexpr size_t kWsCtl = 128, kWsTails = 8 * 256;
 static inline int region_cap_for(int kc) { return ((num_sms() + kPubRegions - 1) / kPubRegions) * kc; }
+static inline size_t ws_pub_keys(int kc) { return (size_t)kPubRegions * region_cap_for(kc) + (size_t)kc + 256; }
 
 REBERT_API size_t rebert_gemv_workspace_bytes(int64_t n, int32_t kc) {
     (void)n;
-    return 128 + kWsCtl + kWsTails + ((size_t)kPubRegions * region_cap_for(kc) + (size_t)kc + 256) * sizeof(uint64_t) + 256;
+    return 128 + kWsCtl + kWsTails + (ws_pub_keys(kc) + (size_t)num_sms() * 32) * sizeof(uint64_t) + 256;
 }
 
 REBERT_API int rebert_workspace_reset(void* workspace, size_t workspace_bytes, rebert_stream stream) {
@@ -1102,6 +1242,14 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
                        "gemv_topk: gate rows must be 128-byte and gate factors 16-byte aligned");
     const int n_excl = (filter && filter->exclude_rows && filter->n_exclude > 0) ? filter->n_exclude : 0;
     GemvLaunch g = plan_gemv(LS, cat->n, kc, gated ? L.ld : (use_generic(L) ? L.ld : 0), n_excl);
+    // The seed runs as the gated kernel's prologue when the gated grid is one CTA per SM (the seed's sample-to-CTA mapping),
+    // the kernel has the prologue (kSeedFoldMaxCpl) and its keys fit beside the pipeline without a shallower ring; else
+    // gate_seed_kernel runs ahead of the gated kernel.
+    bool fold = false;
+    if (gated && cat->n > 0 && g.grid == num_sms() && LS.cpl <= kSeedFoldMaxCpl) {
+        const GemvLaunch gf = plan_gemv(LS, cat->n, kc, L.ld, n_excl, seed_smem_bytes(kc));
+        if (gf.stages == g.stages) { g = gf; fold = true; }
+    }
     GemvParams p;
     memset(&p, 0, sizeof(p));
     p.rows = gated ? cat->gate_rows : cat->rows;
@@ -1148,14 +1296,16 @@ int gemv_launch(const rebert_catalog_t* cat, const float* qn32, const rebert_fil
     p.publish_only = fused ? 1 : 0;
 
     int rc;
-    if (gated && cat->n > 0) {                       // the seed's bound, in the grid-wide hint before the gated kernel starts
+    if (gated && cat->n > 0) {                       // the seed's bound in the grid-wide hint
         p.seed_m = seed_rows(cat->n);
         p.seed_stride = cat->n / p.seed_m;
-        const int per = (kc + num_sms() - 1) / num_sms();
-        p.seed_P = 2 * per < 32 ? 2 * per : 32;
-        p.seed_keys = p.pub_keys;                    // free until the gated kernel publishes, which waits for the seed
-        rc = cat->dtype == REBERT_F32 ? launch_gate_seed<float>(LS, p, st) : launch_gate_seed<__nv_bfloat16>(LS, p, st);
-        if (rc != REBERT_OK) return rc;
+        p.seed_P = seed_P_for(kc);
+        p.seed_keys = p.pub_keys + ws_pub_keys(kc);
+        p.seed_fold = fold ? 1 : 0;
+        if (!fold) {
+            rc = cat->dtype == REBERT_F32 ? launch_gate_seed<float>(LS, p, st) : launch_gate_seed<__nv_bfloat16>(LS, p, st);
+            if (rc != REBERT_OK) return rc;
+        }
     }
     if (cat->dtype == REBERT_I8) rc = launch_gemv_i8(L, p, g, st);
     else if (gated) rc = cat->dtype == REBERT_F32 ? launch_gemv_gated<float>(LS, p, g, kc, st) : launch_gemv_gated<__nv_bfloat16>(LS, p, g, kc, st);
