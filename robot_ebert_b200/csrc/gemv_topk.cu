@@ -157,10 +157,12 @@ __device__ __forceinline__ float fetch_row_dot(const uint4* __restrict__ row, co
 }
 
 // One element of the int8 query planes: qv ~ dh * h + dl * l (the consumers' registers and the gate's delta use this).
+// The residual qv - h * dh is rounded once (fmaf), so the planes do not depend on whether the compiler contracts it; the
+// tests' exact model of S (tests/int8_score_model.py) rounds it the same way.
 __device__ __forceinline__ void quant_planes(float qv, float dh, float dl, int& h, int& l) {
     h = __float2int_rn(qv / dh);
     h = max(-127, min(127, h));
-    l = __float2int_rn((qv - (float)h * dh) / dl);
+    l = __float2int_rn(fmaf(-dh, (float)h, qv) / dl);
     l = max(-127, min(127, l));
 }
 

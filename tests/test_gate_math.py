@@ -3,7 +3,8 @@
 The gated fast pass skips a row when its int8 score S falls below L - delta, L a lower bound of the kc-th best fp32 fast
 score F.  That is sound only if S >= F - delta for every row and every query the kernel may be passed (also non-unit
 ones).  Here the int8 rows, the two query planes, S and F are formed the way the kernels form them (rebert_catalog_quantize_i8,
-the consumers' planes, the per-lane fmaf chains and the xor-shuffle tree of the plain kernel), and the inequality is checked
+S bit for bit from tests/int8_score_model.py, the per-lane fmaf chains and the xor-shuffle tree of the plain kernel, delta
+rounded up as gate_delta rounds it), and the inequality is checked
 for every row over gaussian, scaled, spiky, one-hot and non-unit queries and catalogs with a dominant column.
 """
 import zlib
@@ -11,8 +12,7 @@ import zlib
 import numpy as np
 import pytest
 
-U = 2.0 ** -24
-
+from tests import int8_score_model as model
 
 def quantize_rows(x):
     """rebert_catalog_quantize_i8: int8 rows, fp32 factor, max relative row error (fp64)."""
@@ -27,29 +27,14 @@ def quantize_rows(x):
 
 
 def query_planes(q):
-    """The consumers' planes: q ~ dh * h + dl * l (gemv_topk.cu quant_planes)."""
-    qmax = np.float32(np.abs(q).max())
-    dh = np.float32(qmax / np.float32(127)) if qmax > 0 else np.float32(1)
-    dl = np.float32(dh / np.float32(254))
-    h = np.clip(np.rint(q / dh), -127, 127).astype(np.int32)
-    l = np.clip(np.rint((q - h.astype(np.float32) * dh) / dl), -127, 127).astype(np.int32)
-    return dh, dl, h, l
-
-
-def gate_delta(q, dh, dl, h, l, row_err, epl):
-    r = q.astype(np.float64) - (np.float64(dh) * h + np.float64(dl) * l)
-    qn, eq = np.sqrt((q.astype(np.float64) ** 2).sum()), np.sqrt((r ** 2).sum())
-    shadow = row_err * (qn + eq) + eq + 32.0 * U * (1.0 + row_err) * (qn + eq)
-    fast = (epl + 12) * U * qn
-    return float(np.float32(np.nextafter((shadow + fast) * (1.0 + 1e-6) + 1e-6 * qn + 1e-30, np.inf)))
+    """The consumers' planes: q ~ dh * h + dl * l (gemv_topk.cu quant_planes, residual rounded once)."""
+    return model.query_planes(q)
 
 
 def shadow_scores(q8, factor, dh, dl, h, l):
-    hs = (q8.astype(np.int64) @ h).astype(np.float32)
-    ls = (q8.astype(np.int64) @ l).astype(np.float32)
-    lo = (np.float32(dl) * ls).astype(np.float32)
-    s = (np.float64(dh) * hs.astype(np.float64) + lo).astype(np.float32)        # fmaf
-    return (s * factor).astype(np.float32)
+    """S bit for bit (tests/int8_score_model.py)."""
+    hs, ls = model.plane_sums(q8, h, l)
+    return model.score_from_sums(dh, dl, hs, ls, factor)
 
 
 def fast_scores(x, q, inv, epc):
@@ -62,7 +47,7 @@ def fast_scores(x, q, inv, epc):
     acc = np.zeros((2, n, 32), dtype=np.float32)
     for j in range(cpl):
         for e in range(epc):
-            acc[j & 1] = (acc[j & 1].astype(np.float64) + xv[:, j, :, e].astype(np.float64) * qv[j, :, e]).astype(np.float32)
+            acc[j & 1] = model.fmaf32(xv[:, j, :, e], qv[j, :, e], acc[j & 1])
     s = (acc[0] + acc[1]).astype(np.float32)
     o = 16
     while o:
@@ -121,7 +106,7 @@ def test_shadow_never_falls_below_fast_minus_delta(dtype, d, rows, qkind):
     q[:d] = query(qkind, rng, d)
     q8, factor, row_err, inv = quantize_rows(x[:, :d])
     dh, dl, h, l = query_planes(q[:d])
-    delta = gate_delta(q[:d], dh, dl, h, l, row_err, (ld // 32 // epc) * epc)
+    delta = float(model.gate_delta(q, d, row_err, (ld // 32 // epc) * epc))
     S = shadow_scores(q8, factor, dh, dl, h, l).astype(np.float64)
     F = fast_scores(x, q, inv, epc).astype(np.float64)
     gap = F - S

@@ -60,8 +60,15 @@ def num_sms():
     return torch.cuda.get_device_properties(DEV).multi_processor_count
 
 
-def plan_gemv(d, dtype, n, kc, n_excl=0):
-    """csrc/gemv_topk.cu plan_gemv and gemv_launch's static / dynamic split."""
+def seed_smem_bytes(kc):
+    """csrc/gemv_topk.cu seed_smem_bytes: the folded seed's keys beside the gated kernel's pipeline."""
+    p = min(2 * -(-kc // num_sms()), 32)
+    return (8 * 32 + 32 + num_sms() * p) * 8 + 8
+
+
+def plan_gemv(d, dtype, n, kc, n_excl=0, q_floats=None, seed_bytes=0):
+    """csrc/gemv_topk.cu plan_gemv and gemv_launch's static / dynamic split.  q_floats: query floats staged in shared memory
+    (default: ld for the generic kernel, else none; the gated kernel stages the record's ld); seed_bytes: seed_smem_bytes."""
     sms = num_sms()
     lanes, cpl, ld = row_layout(d, dtype)
     row_bytes = ld * ESIZE[dtype]
@@ -77,8 +84,9 @@ def plan_gemv(d, dtype, n, kc, n_excl=0):
     while tr >= 2 * unit and (n + tr - 1) // tr < sms and ((tr // 2) & 3) == 0:
         tr //= 2
     stage_stride = tr * row_bytes + ((tr * 4 + 127) & ~127)
-    generic = kernel_class(d, dtype) == ("generic",)
-    fixed = 2 * 4 * 8 + (ld * 4 if generic else 0) + (4 * n_excl if 0 < n_excl <= 4096 else 0) + 128
+    if q_floats is None:
+        q_floats = ld if kernel_class(d, dtype) == ("generic",) else 0
+    fixed = 2 * 4 * 8 + q_floats * 4 + (4 * n_excl if 0 < n_excl <= 4096 else 0) + 128 + seed_bytes
     stages = 4
     while stages > 1 and stages * stage_stride + fixed > 220 * 1024:
         stages -= 1
@@ -95,7 +103,18 @@ def plan_gemv(d, dtype, n, kc, n_excl=0):
     if rounds - sr < 8:
         sr = rounds
     sr = max(sr, 1)
-    return dict(tile_rows=tr, grid=grid, static_rounds=sr, rounds=rounds, tiles=tiles, merge_cap=cap, rpw=rpw)
+    return dict(tile_rows=tr, grid=grid, static_rounds=sr, rounds=rounds, tiles=tiles, merge_cap=cap, rpw=rpw, stages=stages)
+
+
+def gated_seed_mode(d, dtype, n, kc, n_excl=0):
+    """gemv_launch's choice for a gated request: "fold" (the seed as the gated kernel's prologue: grid of one CTA per SM,
+    int8 rows of at most 4 chunks per lane, and the seed's keys fit without a shallower ring) or "kernel" (gate_seed_kernel
+    ahead of it).  Also returns the gated grid."""
+    x_ld = row_layout(d, dtype)[2]
+    g = plan_gemv(d, "i8", n, kc, n_excl, q_floats=x_ld)
+    fold = n > 0 and g["grid"] == num_sms() and row_layout(d, "i8")[1] <= 4 and \
+        plan_gemv(d, "i8", n, kc, n_excl, q_floats=x_ld, seed_bytes=seed_smem_bytes(kc))["stages"] == g["stages"]
+    return ("fold" if fold else "kernel"), g["grid"]
 
 
 # ------------------------------------------------------------------ exact integer catalogs ----------------------------

@@ -68,13 +68,17 @@ def key_rows(keys):
     return (0xFFFFFFFF - (keys.astype(np.uint64) & np.uint64(0xFFFFFFFF))).astype(np.int64)
 
 
-def run(store, k, query=None, liked=None, excl=None, row_filter=None, q_scale=None):
-    """(packed request result, candidate keys, seed word of each launch) for one request."""
+def run(store, k, query=None, liked=None, excl=None, row_filter=None, q_scale=None, q_raw=None):
+    """(packed request result, candidate keys, seed word of each launch) for one request.  q_raw: the fast pass gets this
+    fp32 query as it is (not normalised; the exact pass keeps the normalised one)."""
     kc = nat.load().rebert_candidates_for_k(k)
     excl_ptr, ne = store.stage_inputs(query, liked, None, excl, k, kc)
     s = store._scratch()
     if q_scale is not None:
         s.qn32.mul_(q_scale)
+    if q_raw is not None:
+        s.qn32.zero_()
+        s.qn32[:len(q_raw)] = torch.from_numpy(np.asarray(q_raw, dtype=np.float32)).to(s.qn32.device)
     packed = store.enqueue_fused(k, kc, excl_ptr, ne, row_filter).cpu().numpy().copy()
     w_fused = seed_word(s.ws)
     store.enqueue_topk(k, kc, excl_ptr, ne, row_filter)

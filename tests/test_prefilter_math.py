@@ -1,8 +1,10 @@
-"""CPU check of the int8 prefilter's error bound (the arithmetic of quantize_i8_kernel and of the int8 query planes in
-gemv_topk_kernel, restated in numpy): |shadow score - true cosine| never exceeds the bound CatalogStore.enable_prefilter
-adds to the proof margin."""
+"""CPU check of the int8 prefilter's error bound (the arithmetic of quantize_i8_kernel restated in numpy, the shadow score S
+bit for bit from tests/int8_score_model.py): |S - true cosine| never exceeds the bound CatalogStore.enable_prefilter adds to
+the proof margin."""
 import numpy as np
 import pytest
+
+from tests import int8_score_model as model
 
 
 def _quantize_rows(x, nrm=None):
@@ -16,15 +18,6 @@ def _quantize_rows(x, nrm=None):
     err = np.linalg.norm(x.astype(np.float64) - q8 * scale[:, None].astype(np.float64), axis=1) / nrm
     factor = (scale.astype(np.float64) / nrm).astype(np.float32)
     return q8, factor, err.max()
-
-
-def _query_planes(q):
-    qmax = np.float32(np.abs(q).max())
-    dh = qmax / np.float32(127) if qmax > 0 else np.float32(1)
-    dl = np.float32(dh / np.float32(254))
-    hi = np.clip(np.rint(q / dh), -127, 127).astype(np.int32)
-    lo = np.clip(np.rint((q - hi.astype(np.float32) * dh) / dl), -127, 127).astype(np.int32)
-    return hi, lo, dh, dl
 
 
 @pytest.mark.parametrize("d", [1, 7, 32, 50, 768, 1536])
@@ -44,8 +37,8 @@ def test_shadow_score_error_is_within_the_proven_bound(d, kind):
         q[rng.integers(0, d)] = 1.0
     qn = (q / np.linalg.norm(q)).astype(np.float32)              # what query_normalize hands the kernel
     q8, factor, row_err = _quantize_rows(x)
-    hi, lo, dh, dl = _query_planes(qn)
-    shadow = (np.float32(dh) * (q8 @ hi).astype(np.float32) + np.float32(dl) * (q8 @ lo).astype(np.float32)) * factor
+    dh, dl, hi, lo = model.query_planes(qn)
+    shadow = model.int8_scores(q8, factor, qn)                    # S bit for bit, as the kernel forms it
     nrm = np.linalg.norm(x.astype(np.float64), axis=1)
     nrm[nrm == 0] = 1.0
     true = (x.astype(np.float64) @ qn.astype(np.float64)) / nrm
